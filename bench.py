@@ -202,7 +202,10 @@ class CpuReference:
     def __init__(self, blobs, pixels):
         self.cores = os.cpu_count() or 1
         self.kind = "reference" if reference_binary() else "port"
-        base = "/dev/shm" if os.path.isdir("/dev/shm") and os.access("/dev/shm", os.W_OK) else None
+        # what ran, for the JSON lines: the reference CLI runs 2 threads per process, the restatement one
+        self.program = "the reference CLI (oracle/_ref/decoder)" if self.kind == "reference" else "the C restatement (oracle/librestate.so)"
+        self.threads = " x 2 threads" if self.kind == "reference" else ""
+        base ="/dev/shm" if os.path.isdir("/dev/shm") and os.access("/dev/shm", os.W_OK) else None
         self.dir = tempfile.mkdtemp(prefix="bjref_", dir=base)
         self.files = []
         for i, b in enumerate(blobs):
@@ -234,6 +237,40 @@ def pixels_of(specs):
     return sum(s[0] * s[1] for s in specs)
 
 
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+
+DUMP_IMAGES = 16           # images of the batch whose outputs are written (a fixed, seeded choice)
+DUMP_VALUES = 15 << 20     # float32 values in all: 60 MiB, below the 64 MB the dump may take
+
+
+def dump_selection(n):
+    """Indices of the images --dump-outputs writes: the same for the same batch size on every run."""
+    rng = np.random.default_rng(0)
+    return sorted(int(i) for i in rng.choice(n, size=min(n, DUMP_IMAGES), replace=False))
+
+
+def download_selected(batch, first, wanted):
+    """{index in the whole batch: BMP bytes} of the wanted images that lie in `batch` (images first .. first + n - 1)."""
+    mine = [i - first for i in wanted if first <= i < first + batch.n]
+    if not mine:
+        return {}
+    views = batch.download(only=mine)
+    return {first + j: views[j].copy() for j in mine}
+
+
+def write_dump(dirname, arrays):
+    """arrays: {name: integer array} -> dirname/<name>.npy as float32 (exact for int16 / uint8 values).  An array larger
+    than its share of DUMP_VALUES is written as a seeded sample: its values at sorted random positions, which depend only
+    on its size, so that two builds of the project write comparable samples."""
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_VALUES // max(1, len(arrays))
+    for name, a in arrays.items():
+        if a.size > share:
+            pos = np.sort(np.random.default_rng(a.size).choice(a.size, size=share, replace=False))
+            a = a.reshape(-1)[pos]
+        np.save(os.path.join(dirname, name + ".npy"), a.astype(np.float32))
+
+
 def run_reference(args, rank, world):
     if rank != 0:
         return
@@ -245,11 +282,14 @@ def run_reference(args, rank, world):
         for _ in range(args.warmup):
             ref.step()
         times = [ref.step() for _ in range(args.steps)]
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, {f"bmp_{i:05d}": np.fromfile(ref.files[i][:-4] + ".bmp", dtype=np.uint8)
+                                           for i in dump_selection(len(ref.files))})
     finally:
         ref.close()
     total = sum(times)
     mpx = ref.pixels * args.steps / total / 1e6
-    sample = f"{n} images of the workload per step ({desc}), {min(ref.cores, n)} processes x 2 threads, files on tmpfs, BMP written"
+    sample = f"{n} images of the workload per step ({desc}), {min(ref.cores, n)} processes{ref.threads} of {ref.program}, files on tmpfs, BMP written"
     line = {"impl": "reference", "metric": METRIC, "value": mpx, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": 1e3 * total / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int32/int16",
             "data": "synthetic", "images_per_s": n * args.steps / total,
@@ -368,10 +408,12 @@ def run_compat(args, rank, local_rank, world):
     t0 = time.perf_counter()
     kern_ms = 0.0
     for _ in range(args.steps):
-        dec.exec_mcus(md, pre)
+        got = dec.exec_mcus(md, pre)
         kern_ms += dec.stat("exec_ms")
     wall = time.perf_counter() - t0
     dec.close()
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, {"mcus": got})
     cpu = None
     if ol.ref_available():
         t0 = time.perf_counter()
@@ -397,7 +439,10 @@ def run_compat(args, rank, local_rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of every decode pass that reports a value: device-resident (one and several streams), one-call "
+                         "(unless --e2e-steps), compat, reference.  Baselines run a fixed length: the CPU arm beside the GPU run (up to 12 "
+                         "passes or 10 s), the CLI leg (3 runs) and, with several ranks, rank 0's one-call pass alone (2 passes)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="config2")
@@ -410,7 +455,7 @@ def main():
     ap.add_argument("--sync-phased", type=int, default=-1, help="1/0: Huffman synchronisation pass with / without early stop of re-decodes (-1 = library default)")
     ap.add_argument("--sync-preroll", type=int, default=-1, help="bits of pre-roll of the Huffman synchronisation pass' first guess (-1 = library default)")
     ap.add_argument("--streams", type=int, default=2, help="device-resident value: decode the batch as this many independent parts on as many CUDA streams (1: one stream; the per-stage times always come from a one-stream pass)")
-    ap.add_argument("--e2e-steps", type=int, default=0)
+    ap.add_argument("--e2e-steps", type=int, default=0, help="timed steps of the one-call path (0 = --steps)")
     ap.add_argument("--sub-batch-mb", type=int, default=0, help="compressed MB per sub-batch of the one-call path (0 = library default)")
     ap.add_argument("--host-threads", type=int, default=0, help="host worker threads of the one-call path (0 = library default)")
     ap.add_argument("--no-ramp", action="store_true", help="one-call path: all sub-batches the same size")
@@ -421,7 +466,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cli", action="store_true", help="skip the CLI-to-CLI leg (decoder_b200 vs the reference CLI on the same tmpfs files)")
     ap.add_argument("--clock-sample-ms", type=int, default=100, help="nvidia-smi polling interval while the timed regions run (0 = no sampling: for A/B only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed (rank 0) to DIR/<name>.npy as float32: the BMP bytes of "
+                         f"a fixed, seeded choice of {DUMP_IMAGES} images (bmp_<index in the batch>; --workload compat: the mcus buffers), "
+                         "larger ones as a seeded sample of their bytes, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -524,7 +575,12 @@ def main():
     launches = 0
     ms_total = 0.0
     first_hash = None
-    steps = args.steps if not stream else 1                  # a stream is decoded once (it is 16x to 64x the default batch)
+    steps = args.steps
+    # the reported value comes from the multi-stream pass (1b) when there is one, else from this pass: --dump-outputs
+    # writes the outputs of that pass' last step
+    nstreams = 1 if stream else max(1, min(args.streams, len(blobs)))
+    dump_idx = dump_selection(len(blobs)) if args.dump_outputs and rank == 0 else []
+    dumped = {}
     barrier()
     t_wall0 = time.perf_counter()
     for ci, (c0, c1) in enumerate(chunks):
@@ -557,6 +613,8 @@ def main():
             import hashlib
             first = batch.download(only=[0])[0]
             first_hash = hashlib.sha256(first.tobytes()).hexdigest()
+        if nstreams == 1:
+            dumped.update(download_selected(batch, c0, dump_idx))
         batch.destroy()
     barrier()
     windows.append((t_wall0, time.perf_counter()))
@@ -567,7 +625,6 @@ def main():
     # kernels of different parts overlap on the GPU - the Huffman kernels are latency bound, the IDCT kernel issue bound,
     # so they fill each other's gaps.  This is the whole-job device-resident throughput; the per-stage times above come
     # from the one-stream pass, where a kernel has the GPU to itself.
-    nstreams = 1 if stream else max(1, min(args.streams, len(blobs)))
     if nstreams > 1:
         streams = [torch.cuda.Stream() for _ in range(nstreams)]
         cut = [len(blobs) * i // nstreams for i in range(nstreams + 1)]
@@ -604,7 +661,8 @@ def main():
             import hashlib
             assert hashlib.sha256(parts[0].download(only=[0])[0].tobytes()).hexdigest() == first_hash, "multi-stream and one-stream decodes disagree"
         launches = sum(bpart.info().launches for bpart in parts) * steps
-        for bpart in parts:
+        for p, bpart in enumerate(parts):
+            dumped.update(download_selected(bpart, cut[p], dump_idx))
             bpart.destroy()
         ms_max = allmax(ms_par)
 
@@ -653,7 +711,7 @@ def main():
                 st_all.append(dec.decode_packed(pin_in.array, in_off[a:b], in_len[a:b], pin_out.array, offs, bj.BJ_OUT_BMP))
             return st_all
 
-        k2 = args.e2e_steps or (1 if stream else max(2, min(args.steps, 5)))
+        k2 = args.e2e_steps or steps
         e2e_single = None
         if world > 1:                                         # rank 0 alone first: the denominator of the e2e scaling efficiency
             if rank == 0:
@@ -663,7 +721,7 @@ def main():
                     one_pass()
                 e2e_single = px * 2 / (time.perf_counter() - t0) / 1e6
             barrier()
-        if stream:                                            # a stream is decoded once; its first call twice (buffers reach their size)
+        if stream:                                            # a stream's warm-up is its first call (buffers reach their size)
             a, b, offs = calls[0]
             dec.decode_packed(pin_in.array, in_off[a:b], in_len[a:b], pin_out.array, offs, bj.BJ_OUT_BMP)
         for _ in range(max(1, min(args.warmup, 2)) if not stream else 0):
@@ -725,7 +783,7 @@ def main():
                 t += ref.step()
                 passes += 1
             cpu = {"value": ref.pixels * passes / t / 1e6, "unit": UNIT, "cores": ref.cores, "kind": ref.kind, "images_per_s": n * passes / t,
-                   "sample": f"first {n} images of the batch, {passes} passes, {min(ref.cores, n)} processes x 2 threads of the reference CLI on tmpfs (BMP written), {t:.2f} s"}
+                   "sample": f"first {n} images of the batch, {passes} passes, {min(ref.cores, n)} processes{ref.threads} of {ref.program} on tmpfs (BMP written), {t:.2f} s"}
             # ---- parity against what the reference just wrote
             if pin_out is not None:
                 want = {}
@@ -745,7 +803,7 @@ def main():
                 a0, b0, offs0 = calls[0]
                 nchk = min(n, b0 - a0)
                 mism = [i for i in range(nchk) if hashlib.sha256(pin_out.array[int(offs0[i]):int(offs0[i]) + sizes[i]].tobytes()).hexdigest() != want[i]]
-                parity = {"checked": nchk, "mismatches": len(mism), "against": "the BMP files the reference CLI (oracle/_ref/decoder) wrote in this run", "rule": rule}
+                parity = {"checked": nchk, "mismatches": len(mism), "against": f"the BMP files {ref.program} wrote in this run", "rule": rule}
             # ---- CLI to CLI on the same tmpfs files: decoder_b200 (file -> BMP file, one process, every visible GPU)
             cli_bin = os.path.join(ROOT, "pim_jpeg_decoder_b200", "host", "_build", "decoder_b200")
             if not args.no_cli and os.path.exists(cli_bin) and ref.kind == "reference":
@@ -778,6 +836,8 @@ def main():
     sampler.stop()
     if dec is not None:
         dec.close()
+    if dumped:
+        write_dump(args.dump_outputs, {f"bmp_{i:05d}": b for i, b in sorted(dumped.items())})
 
     if rank != 0:
         if world > 1:

@@ -79,6 +79,24 @@ def ref_available():
     return os.path.exists(os.path.join(ORACLE, "_ref", "libref.so"))
 
 
+REFERENCE_VECTORS = os.path.join(ROOT, "tests", "golden", "reference_vectors.json")
+
+
+def reference_vectors():
+    """What the reference computed on the seeded inputs of the exec and damaged-header tests (make_reference_vectors.py)."""
+    import json
+    with open(REFERENCE_VECTORS) as f:
+        return json.load(f)
+
+
+def sha256(*arrays):
+    import hashlib
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
 def ref():
     global _ref
     if _ref is None:

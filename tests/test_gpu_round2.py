@@ -379,7 +379,12 @@ def test_ref_mcus_output_and_descriptor_input(dec, golden, golden_dir, tmp_path)
     o_bmp, st_bmp = dec.decode_desc(descs, [p[1] for p in pairs], None, fmt=bj.BJ_OUT_BMP)
     for n, o in zip(names, o_bmp):
         assert sha(o) == golden[golden[n]["expect"]]["bmp_sha256"], n
-    # (3) the reference's own write_BMP on our buffers
+    # (3) the reference's own write_BMP on our buffers: its inputs - metadata and post-exec buffer - are the ones it
+    # turned into the golden BMP (golden.json holds the reference's hashes of both; for a restart-parity twin, the
+    # twin's); where oracle/_ref/libref.so is built, write_BMP itself runs on them too
+    for n, o, r in zip(names, o_raw, rs):
+        e = golden[golden[n]["expect"]]
+        assert sha(o) == e["mcus_post_sha256"] and sha(r.metadata[0]) == e["metadata_sha256"], n
     if ol.ref_available() and hasattr(ol.ref(), "ref_write_bmp"):
         for n, o, r in list(zip(names, o_raw, rs))[::3]:
             path = str(tmp_path / (n + ".bmp"))

@@ -2,7 +2,8 @@
 
 Two anchors: (1) tests/golden/golden.json - SHA-256 of the BMP, the post-Huffman buffer and the post-exec buffer
 that the REAL reference code produced for every fixture (made by tests/golden/make_golden.py);
-(2) when oracle/_ref/libref.so is present, the real reference code itself, run live on random inputs.
+(2) tests/golden/reference_vectors.json - what the reference's DPU program computed on seeded random buffers, and,
+when oracle/_ref/libref.so is present, the real reference code itself, run live on the same buffers.
 """
 import hashlib
 import os
@@ -82,33 +83,31 @@ def _random_exec_case(rng, vs, hs, ncomp, nchunk, full_range):
     return md, mcus
 
 
-@pytest.mark.skipif(not ol.ref_available(), reason="oracle/_ref/libref.so not built")
-@pytest.mark.parametrize("vs,hs,ncomp", [(1, 1, 3), (2, 1, 3), (1, 2, 3), (2, 2, 3), (1, 1, 1), (2, 2, 1), (0, 0, 0)])
-@pytest.mark.parametrize("full_range", [False, True])
-def test_exec_restatement_vs_live_reference(vs, hs, ncomp, full_range):
-    """The DPU program (dequant, IDCT, colour) on random buffers, incl. values that wrap 16 and 32 bits."""
+EXEC_SHAPES = [(1, 1, 3), (2, 1, 3), (1, 2, 3), (2, 2, 3), (1, 1, 1), (2, 2, 1), (0, 0, 0)]
+
+
+def exec_case(vs, hs, ncomp, full_range):
+    """-> (key in reference_vectors.json, metadata, mcus): three chunks of seeded random input for the DPU program."""
     rng = np.random.default_rng(vs * 100 + hs * 10 + ncomp + (1000 if full_range else 0))
     md, mcus = _random_exec_case(rng, vs, hs, ncomp, 3, full_range)
     if ncomp == 0:
         md[:] = 0  # idle DPU: nothing runs, buffer unchanged
-        md_ref = md
+    return f"{vs},{hs},{ncomp},{int(full_range)}", md, mcus
+
+
+@pytest.mark.parametrize("vs,hs,ncomp", EXEC_SHAPES)
+@pytest.mark.parametrize("full_range", [False, True])
+def test_exec_restatement_vs_live_reference(vs, hs, ncomp, full_range):
+    """The DPU program (dequant, IDCT, colour) on random buffers, incl. values that wrap 16 and 32 bits: the
+    restatement against what the reference's program computed on the same buffers (tests/golden/reference_vectors.json),
+    and against the reference itself where oracle/_ref/libref.so is built."""
+    key, md, mcus = exec_case(vs, hs, ncomp, full_range)
+    want = ol.reference_vectors()["exec_mcus"][key]
+    assert ol.sha256(md, mcus) == want["input_sha256"], "the seeded inputs are not the ones the reference was run on"
     got = ol.restate_exec_mcus(md, mcus)
-    want = ol.ref_exec_mcus(md, mcus)
-    assert np.array_equal(got, want)
-
-
-@pytest.mark.skipif(not ol.ref_available(), reason="oracle/_ref/libref.so not built")
-def test_live_reference_matches_golden_json(golden, golden_dir, tmp_path):
-    """golden.json really is what the reference code computes (guards against a stale json)."""
-    import shutil
-    for name in ("ilsvrc_444", "p420_50x37", "enc_440_zz48_52"):
-        e = golden[name]
-        p = str(tmp_path / e["file"])
-        shutil.copy(os.path.join(golden_dir, e["file"]), p)
-        r = ol.RefDecoded(p, str(tmp_path / (name + ".bmp")))
-        assert sha(r.mcus_pre) == e["mcus_pre_sha256"]
-        assert sha(r.mcus_post) == e["mcus_post_sha256"]
-        assert sha(np.fromfile(str(tmp_path / (name + ".bmp")), dtype=np.uint8)) == e["bmp_sha256"]
+    assert ol.sha256(got) == want["output_sha256"]
+    if ol.ref_available():
+        assert np.array_equal(got, ol.ref_exec_mcus(md, mcus))
 
 
 def test_idct_dc_only():
