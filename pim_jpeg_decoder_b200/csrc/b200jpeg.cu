@@ -58,20 +58,9 @@ extern "C" int bj_create(bj_ctx **out, int device) {
     cudaDeviceProp prop;
     if (rc == BJ_OK) rc = c->check(cudaGetDeviceProperties(&prop, device));
     if (rc == BJ_OK) c->sm_count = prop.multiProcessorCount;
-    c->ri_split_threads = 0;       // measured (profiles/r2_latency_experiments.md): cutting restart segments finer is slower even for one 4K image
-    if (const char *e = getenv("B200JPEG_RI_SPLIT")) c->ri_split_threads = atoi(e);          // (experiments)
-    if (const char *e = getenv("B200JPEG_IDCT_TMA")) c->idct_tma = atoi(e) != 0;
-    if (const char *e = getenv("B200JPEG_MIN_SUB")) c->min_sub_bytes = std::max(16, atoi(e));
     if (rc == BJ_OK) rc = c->check(cudaFuncSetAttribute(k_idct_color<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctColor));
     if (rc == BJ_OK) rc = c->check(cudaFuncSetAttribute(k_idct_color<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctColor));
     if (rc == BJ_OK) rc = batch_kernels_init(c);
-    if (rc == BJ_OK) rc = c->check(cudaFuncSetAttribute(k_idct_color_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctTma));
-    if (rc == BJ_OK) {
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess) c->encode_tiled = (bj_ctx::EncodeTiledFn)fn;
-        else cudaGetLastError();
-    }
     for (int i = 0; i < kSlots && rc == BJ_OK; i++) rc = c->check(cudaStreamCreateWithFlags(&c->streams[i], cudaStreamNonBlocking));
     for (int i = 0; i < 2 && rc == BJ_OK; i++) rc = c->check(cudaEventCreate(&c->ev_exec[i]));
     if (rc != BJ_OK) { bj_destroy(c); return BJ_ERR_CUDA; }                   // (releases whatever was created)
@@ -183,7 +172,8 @@ extern "C" int bj_set_option(bj_ctx *c, const char *name, long value) {
     }
     if (!strcmp(name, "subseq_bits")) { if (value != 0 && (value < 128 || value % 32 || value > (1 << 18))) return BJ_ERR_ARG; c->subseq_bits = (int)value; return BJ_OK; }
     if (!strcmp(name, "sub_batch_ramp")) { c->sub_batch_ramp = value != 0; return BJ_OK; }
-    if (!strcmp(name, "sync_phased")) { c->sync_phased = value != 0; return BJ_OK; }
+    // the synchronisation pass with early stop of re-decodes is the only one; the option stays for bench.py --sync-phased
+    if (!strcmp(name, "sync_phased")) return value == 1 ? BJ_OK : BJ_ERR_ARG;
     if (!strcmp(name, "slices")) { if (value != 0 && value != 1 && value != 2 && value != 4 && value != 8) return BJ_ERR_ARG; c->slices = (int)value; return BJ_OK; }
     if (!strcmp(name, "sub_batch_bytes")) { if (value < (1 << 16)) return BJ_ERR_ARG; c->sub_batch_bytes = (size_t)value; return BJ_OK; }
     if (!strcmp(name, "packed_outputs")) { c->packed_outputs = value != 0; return BJ_OK; }
@@ -193,7 +183,6 @@ extern "C" int bj_set_option(bj_ctx *c, const char *name, long value) {
     if (!strcmp(name, "max_image_pixels")) { if (value < 1) return BJ_ERR_ARG; c->max_image_pixels = (size_t)value; return BJ_OK; }
     if (!strcmp(name, "sub_batch_out_bytes")) { if (value < (1 << 16)) return BJ_ERR_ARG; c->sub_batch_out_bytes = (size_t)value; return BJ_OK; }
     if (!strcmp(name, "host_threads")) { if (value < 1 || value > 256) return BJ_ERR_ARG; c->host_pool.resize((int)value); return BJ_OK; }
-    if (!strcmp(name, "idct_tma")) { c->idct_tma = value != 0; return BJ_OK; }
     if (!strcmp(name, "debug_sync_iters")) { if (value < 0) return BJ_ERR_ARG; c->debug_sync_iters = (int)value; return BJ_OK; }
     if (!strcmp(name, "sync_preroll_bits")) { if (value < 0 || value > (1 << 16) || value % 32) return BJ_ERR_ARG; c->sync_preroll_bits = (int)value; return BJ_OK; }
     if (!strcmp(name, "sync_rounds")) { if (value < 0 || value > kMaxRounds) return BJ_ERR_ARG; c->sync_rounds = (int)value; return BJ_OK; }

@@ -41,17 +41,12 @@ constexpr int kSmemHuffSyncMax = kSmemLutMax;
 
 inline int batch_kernels_init(bj_ctx *c) {
     if (c->check(cudaFuncSetAttribute(k_huff_write, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffWriteMax)) != BJ_OK) return BJ_ERR_CUDA;
-    if (c->check(cudaFuncSetAttribute(k_huff_sync<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
-    if (c->check(cudaFuncSetAttribute(k_huff_sync<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
+    if (c->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
 #ifndef BJ_SYNC_CARVEOUT
 #define BJ_SYNC_CARVEOUT 72            // % of 228 KB: 164 KB of shared memory for 5 CTAs, the rest is L1 (kernels_huff.cuh: BJ_SYNC_CTAS)
 #endif
 #if BJ_SYNC_CARVEOUT > 0
-    if (c->check(cudaFuncSetAttribute(k_huff_sync<true>, cudaFuncAttributePreferredSharedMemoryCarveout, BJ_SYNC_CARVEOUT)) != BJ_OK) return BJ_ERR_CUDA;
-    if (c->check(cudaFuncSetAttribute(k_huff_sync<false>, cudaFuncAttributePreferredSharedMemoryCarveout, BJ_SYNC_CARVEOUT)) != BJ_OK) return BJ_ERR_CUDA;
-#endif
-#ifdef BJ_WRITE_CARVEOUT
-    if (c->check(cudaFuncSetAttribute(k_huff_write, cudaFuncAttributePreferredSharedMemoryCarveout, BJ_WRITE_CARVEOUT)) != BJ_OK) return BJ_ERR_CUDA;
+    if (c->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributePreferredSharedMemoryCarveout, BJ_SYNC_CARVEOUT)) != BJ_OK) return BJ_ERR_CUDA;
 #endif
     return BJ_OK;
 }
@@ -79,9 +74,6 @@ struct bj_batch {
     size_t o_himg = 0, o_idev = 0, o_qtab = 0, o_lutdc = 0, o_lutac = 0, o_lutacs = 0;
     // offsets inside the map buffer (written on the device by k_expand_maps)
     size_t m_tiles = 0, m_blk = 0, m_wblk = 0, m_utile = 0, m_dcc = 0, maps_bytes = 0;
-    uint32_t rgb_max = 0;               // bytes of the widest pixel tile of this batch
-    CUtensorMap tmap;                   // the coefficient buffer as a 2-D tensor of 128-byte rows (k_idct_color_tma)
-    bool use_tma = false;
     uint32_t idct_smem = 0;             // dynamic shared memory of k_idct_color: sized for the widest pixel tile of this batch
     uint32_t n_wblk = 0;                // CTAs of the Huffman write pass
     size_t n_slice_slots = 0;
@@ -97,7 +89,6 @@ struct bj_batch {
     cudaEvent_t ev_done = nullptr;       // one-call path: recorded behind the copy-out, created for a sleeping wait
     cudaStream_t last_stream = nullptr;
     bool uploaded = false, decoded = false, synced = false;
-    bool phased = true;                  // which variant of the synchronisation kernel this batch was laid out for
     bool multi_blk = false;              // some image's sub-sequences span more than one CTA of the synchronisation pass
     bool redone = false;                 // batch_sync had to run extra fix-up rounds: everything after them was computed again
     uint32_t launches = 0, sync_rounds = 0;
@@ -206,27 +197,22 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
     // fill whole CTAs (a nearly empty second CTA costs a cross-CTA fix-up round); the write pass works on whole
     // sub-sequences (1 slice).  An image with restart markers gets sub-sequences that hold a typical restart segment
     // in one piece - segment heads need no speculation at all - and the write pass cuts them into 4 slices (8 when
-    // the batch is small), whose entry states the single synchronisation decode records.
+    // the batch is small), whose entry states the synchronisation pass records.
     const uint32_t fixed_sub = c->subseq_bits ? (uint32_t)c->subseq_bits / 8u : 0u;
     uint32_t fixed_rl = c->slices == 2 ? 1u : c->slices == 4 ? 2u : c->slices == 8 ? 3u : 0u;
     if (fixed_sub) while (fixed_rl && fixed_sub % (1u << fixed_rl)) fixed_rl--;
+    constexpr uint64_t kMinSubBytes = 128;              // shortest sub-sequence the automatic layout picks (small batches)
     uint32_t nominal_sub = 512;
-    uint64_t total_scan = 0, total_ri_segs = 0;
-    for (int i = 0; i < n; i++) if (b->parse_status[i] == BJ_OK) {
-        total_scan += b->desc[i].scan_len;
-        if (b->desc[i].restart_interval) total_ri_segs += (geo[i].nmcu + b->desc[i].restart_interval - 1) / b->desc[i].restart_interval;
-    }
-    if (!fixed_sub) nominal_sub = (uint32_t)std::min<uint64_t>(512u, std::max<uint64_t>((uint64_t)c->min_sub_bytes, total_scan / ((uint64_t)c->sm_count * 3072u)));
-    // whole restart segments as sub-sequences need no speculation, but a batch with few of them (a single 4K image with
-    // a restart interval of 8 MCUs: 4 050) would leave most of the GPU idle: then segments are cut like any other stream
-    const bool ri_whole = total_ri_segs >= (uint64_t)c->ri_split_threads;
+    uint64_t total_scan = 0;
+    for (int i = 0; i < n; i++) if (b->parse_status[i] == BJ_OK) total_scan += b->desc[i].scan_len;
+    if (!fixed_sub) nominal_sub = (uint32_t)std::min<uint64_t>(512u, std::max<uint64_t>(kMinSubBytes, total_scan / ((uint64_t)c->sm_count * 3072u)));
     auto round_sub = [&](uint32_t len, uint32_t rl) { const uint32_t q = 4u << rl; return (std::max(len, 64u) + q - 1u) / q * q; };
     auto sub_layout_of = [&](uint32_t raw_len, uint32_t nseg, uint32_t *rl) -> uint32_t {
         *rl = c->slices ? fixed_rl : 0u;
         if (fixed_sub) return fixed_sub;
         if (nseg > 1) {
             const uint32_t avg = raw_len / nseg;
-            if (avg <= 1024 && (ri_whole || nominal_sub >= avg)) {
+            if (avg <= 1024) {
                 if (!c->slices) *rl = total_scan < ((uint64_t)16 << 20) ? 3u : 2u;
                 return round_sub(std::max(2 * avg, nominal_sub), *rl);
             }
@@ -249,7 +235,7 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
     size_t fbytes = 0, clean_words = 0, out_bytes = 0, coef_units = 0;
     uint32_t seg_entries = 0, nblk = 0, n_utile = 0, n_wblk = 0, n_dcc = 0, n_tiles = 0;
     int prev = -1;                                  // last valid image: its table slots are reused when the tables match
-    b->pixels = 0; b->scan_bytes_max = 0; b->ref_blocks_max = 0; b->nseg_max = 0; b->lut_smem = 0; b->multi_blk = false; b->phased = c->sync_phased != 0;
+    b->pixels = 0; b->scan_bytes_max = 0; b->ref_blocks_max = 0; b->nseg_max = 0; b->lut_smem = 0; b->multi_blk = false;
     uint32_t rgb_max = 0;
     auto same_tables = [](const bj_image_desc &a, const bj_image_desc &q) {
         if (a.ncomp != q.ncomp || memcmp(a.dc_id, q.dc_id, 3) || memcmp(a.ac_id, q.ac_id, 3)) return false;
@@ -375,7 +361,6 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
         if (coef_units > 0xFFFFFFF0ull || clean_words > 0xFFFFFFF0ull || slice_slots > 0xFFFFFFF0ull) return BJ_ERR_ARG;   // split the batch
     }
     b->idct_smem = kSmemDu + kSmemQ + kRgbFront + std::min<uint32_t>(rgb_max, kRgbMax) + 64;
-    b->rgb_max = rgb_max;
     b->files_bytes = b->direct_src ? (size_t)(span_hi - span_lo) : fbytes + 64; b->clean_words = clean_words + 96; b->coef_units = coef_units; b->out_bytes = out_bytes;   // (96 words of slack: a damaged unit is read to its end, up to 63 symbols of 27 bits past the data)
     b->n_wblk = n_wblk; b->n_slice_slots = slice_slots;
     b->n_idct_tiles = n_tiles; b->n_blk = nblk; b->n_utile = n_utile;
@@ -399,7 +384,7 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
     b->m_dcc = o;   o = align_up(o + (size_t)n_dcc * 4, 256);
     b->maps_bytes = o;
     if (b->h_meta.reserve(b->meta_bytes) || (!b->direct_src && b->h_files.reserve(b->files_bytes)) ||
-        b->h_res.reserve(align_up((size_t)n * sizeof(HuffImgState), 64) + kMaxRounds * 4 + 16 + 64)) return BJ_ERR_NOMEM;
+        b->h_res.reserve(align_up((size_t)n * sizeof(HuffImgState), 64) + kMaxRounds * 4 + 64)) return BJ_ERR_NOMEM;
     if (n) { memcpy(b->hmeta<HuffImg>(b->o_himg), himg.data(), (size_t)n * sizeof(HuffImg)); memcpy(b->hmeta<ImgDev>(b->o_idev), idev.data(), (size_t)n * sizeof(ImgDev)); }
     if (!qtabs.empty()) memcpy(b->hmeta<QTab>(b->o_qtab), qtabs.data(), qtabs.size() * sizeof(QTab));
     if (!luts_dc.empty()) memcpy(b->hmeta<uint32_t>(b->o_lutdc), luts_dc.data(), luts_dc.size() * 4);
@@ -422,20 +407,11 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
         b->d_seg.reserve((size_t)(seg_entries + 2) * 4 * 2) || b->d_subseg.reserve((size_t)b->n_sub_slots * 4 + 16) ||
         b->d_stin.reserve((size_t)b->n_sub_slots * 8 + 16) || b->d_stout.reserve((size_t)b->n_sub_slots * 8 + 16) ||
         b->d_tot.reserve((size_t)b->n_sub_slots * 4 + 16) || b->d_pre.reserve((size_t)b->n_sub_slots * 8 + 16) ||
-        b->d_slice.reserve(b->n_slice_slots * 16 + 16) || (b->phased && b->d_quarter.reserve((size_t)b->n_sub_slots * 8 * 16 + 16)) ||
+        b->d_slice.reserve(b->n_slice_slots * 16 + 16) || b->d_quarter.reserve((size_t)b->n_sub_slots * 8 * 16 + 16) ||
         b->d_dc.reserve(coef_units * 2 + 64) || b->d_dcagg.reserve((size_t)b->n_dcc * sizeof(DcAgg) + 16) ||
         b->d_blkagg.reserve((size_t)nblk * sizeof(BlkAgg) + 16) ||
         b->d_state.reserve((size_t)n * sizeof(HuffImgState) + 16) || b->d_flags.reserve(kMaxRounds * 4 + 16) ||
         b->d_coef.reserve(coef_units * 128 + 16) || b->d_out.reserve(out_bytes + 64)) return BJ_ERR_NOMEM;
-    // the coefficient buffer as a tensor of 128-byte rows for the TMA variant of the K2/K3 kernel
-    b->use_tma = false;
-    if (c->idct_tma && c->encode_tiled && format != BJ_OUT_REF_MCUS && coef_units > 0) {
-        const cuuint64_t dims[2] = {64, (cuuint64_t)coef_units}, strides[1] = {128};
-        const cuuint32_t box[2] = {64, (cuuint32_t)kTmaRows}, estr[2] = {1, 1};
-        const CUresult r = c->encode_tiled(&b->tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, b->d_coef.p, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        b->use_tma = r == CUDA_SUCCESS;
-    }
     return BJ_OK;
 }
 
@@ -488,7 +464,7 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
             cudaMemsetAsync(b->d_out.p, 0xA5, b->out_bytes, s);
             cudaMemsetAsync(b->d_clean.p, 0xA5, b->clean_words * 4, s);
         }
-        cudaMemsetAsync(flags, 0, kMaxRounds * 4 + 16, s);
+        cudaMemsetAsync(flags, 0, kMaxRounds * 4, s);
         cudaMemsetAsync(st, 0, (size_t)n * sizeof(HuffImgState), s);                  // (rejected files keep an all-zero state)
         b->launches = 0;
         if (b->n_utile) {
@@ -509,10 +485,7 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
     }
     if (b->n_blk) {
         for (int r = r0; r < r1; r++) {
-            if (b->phased)
-                k_huff_sync<true><<<b->n_blk, kHuffThreads, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, (uint4 *)b->d_quarter.p, agg, flags, r, (uint32_t)c->sync_preroll_bits, (uint32_t)c->debug_sync_iters);
-            else
-                k_huff_sync<false><<<b->n_blk, kHuffThreads, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, nullptr, agg, flags, r, (uint32_t)c->sync_preroll_bits, (uint32_t)c->debug_sync_iters);
+            k_huff_sync<<<b->n_blk, kHuffThreads, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, (uint4 *)b->d_quarter.p, agg, flags, r, (uint32_t)c->sync_preroll_bits, (uint32_t)c->debug_sync_iters);
             b->launches++; b->sync_rounds++;
         }
         cudaEventRecord(b->ev[2], s);
@@ -536,18 +509,13 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
         k_ref_mcus_pad<<<dim3(std::max(gx, 1u), n), 256, 0, s>>>(idev, (uint8_t *)b->d_out.p);
         k_idct_color<true><<<b->n_idct_tiles, kTileThreads, b->idct_smem, s>>>((const int16_t *)b->d_coef.p, dcp, idev, qtabs, tiles, (uint8_t *)b->d_out.p);
         b->launches += 2;
-    } else if (b->n_idct_tiles && b->use_tma) {
-        // persistent: one CTA per slot of the GPU (3 per SM), each loops over tiles with the next tile's TMA copy in flight
-        const unsigned grid = std::min<unsigned>(b->n_idct_tiles, (unsigned)c->sm_count * 3u);
-        k_idct_color_tma<<<grid, kTileThreads, kSmemIdctTma - kRgbMax + std::min<uint32_t>(b->rgb_max, kRgbMax), s>>>(b->tmap, dcp, idev, qtabs, tiles, b->n_idct_tiles, (uint8_t *)b->d_out.p, flags + kMaxRounds);
-        b->launches++;
     } else if (b->n_idct_tiles) {
         k_idct_color<false><<<b->n_idct_tiles, kTileThreads, b->idct_smem, s>>>((const int16_t *)b->d_coef.p, dcp, idev, qtabs, tiles, (uint8_t *)b->d_out.p);
         b->launches++;
     }
     cudaEventRecord(b->ev[4], s);
     cudaMemcpyAsync(b->h_state(), st, (size_t)n * sizeof(HuffImgState), cudaMemcpyDeviceToHost, s);
-    cudaMemcpyAsync(b->h_flags(), flags, kMaxRounds * 4 + 16, cudaMemcpyDeviceToHost, s);
+    cudaMemcpyAsync(b->h_flags(), flags, kMaxRounds * 4, cudaMemcpyDeviceToHost, s);
     return c->check(cudaGetLastError());
 }
 
@@ -583,7 +551,6 @@ inline int batch_sync(bj_batch *b) {
         r += 2;
     }
     b->rounds = r;
-    if (rc == BJ_OK && b->h_flags()[kMaxRounds] != 0) { c->last_error = "TMA copy of a coefficient tile did not complete"; return BJ_ERR_CUDA; }
     if (rc == BJ_OK) {
         cudaEventElapsedTime(&b->ms_entropy, b->ev[0], b->ev[3]);
         cudaEventElapsedTime(&b->ms_unstuff, b->ev[0], b->ev[1]);

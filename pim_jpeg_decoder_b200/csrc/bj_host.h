@@ -1,6 +1,5 @@
 // Host-side plumbing of the library: context, grow-only device buffers, per-image geometry.
 #pragma once
-#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string.h>
@@ -148,22 +147,14 @@ struct bj_ctx {
     int device = 0;
     int sm_count = 0;
     int subseq_bits = 0;                 // sub-sequence length of the synchronisation pass; 0 = automatic (per image)
-    int sync_phased = 1;                 // synchronisation pass: re-decodes stop where they meet the previous decode (kernels_huff.cuh)
     int slices = 0;                      // slices (write pass) per sub-sequence: 1, 2, 4, 8; 0 = default (1)
     size_t sub_batch_bytes = 0;          // 0 = default
     int sub_batch_ramp = 1;              // the first two sub-batches of a call are smaller (the copy-out starts earlier)
     int packed_outputs = 0;              // see batch_download_async
     int packed_inputs = 0;               // see batch_assign: 0 = upload straight from the caller's memory when it is known to be page-locked
                                          // (bj_host_alloc / bj_host_register), 1 = the caller says it is, -1 = always stage
-    int idct_tma = 0;                    // K2/K3: 1 = persistent kernel with TMA-fed, double-buffered coefficient tiles; 0 (default, faster: DESIGN.md section 9) =
-                                         // one CTA per tile, register-staged loads
-    typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *, const cuuint32_t *,
-                                      CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    EncodeTiledFn encode_tiled = nullptr; // cuTensorMapEncodeTiled, through cudaGetDriverEntryPoint (no link against libcuda)
     int debug_sync_iters = 0;            // measurement only: stop the in-CTA fix-up after this many iterations (0: run to the fixed point)
     int sync_preroll_bits = 0;           // synchronisation pass: bits a sub-sequence's first guess is decoded ahead of its start (kernels_huff.cuh: PREROLL)
-    int min_sub_bytes = 128;             // shortest sub-sequence the automatic layout picks (small batches)
-    int ri_split_threads = 0;            // a batch with fewer restart segments than this cuts them into shorter sub-sequences (0: never; B200JPEG_RI_SPLIT for experiments)
     int ref_m = 100;                     // BJ_OUT_REF_MCUS: MAX_MCU_PER_DPU of the host that reads the buffer (Makefile:2 of the reference)
     int debug_poison = 0;                // fill coefficient / DC / output buffers with 0xA5 before every decode (tests: every byte must be written)
     size_t max_image_pixels = (size_t)1 << 28;   // larger images are refused (BJ_ERR_UNSUPPORTED), like the reference's "Too high resolution"
@@ -171,7 +162,6 @@ struct bj_ctx {
     int sync_rounds = 0;                 // 0 = default (3 launches of the fix-up kernel before the first check)
     struct bj_batch *slots[bj::kSlots] = {};          // sub-batches of bj_decode_batch in flight (one stream each)
     bj::HostPool host_pool;
-    int host_threads = 0;                // 0 = default: min(4, hardware threads / 2)
     double stats[16] = {};               // counters of the last bj_decode_batch / job (b200jpeg.cu: ST_*)
     double totals[16] = {};              // ... summed over every call since bj_create
     cudaStream_t streams[bj::kSlots] = {};

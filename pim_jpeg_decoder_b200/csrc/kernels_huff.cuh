@@ -481,8 +481,14 @@ __device__ __forceinline__ uint32_t pack16(uint32_t lo, uint32_t hi) { return (l
 // round r>0: the first sub-sequence of the CTA takes the exit state of the previous CTA's last one; if that
 //          differs from what it used, the CTA re-converges.  flags[r] counts CTAs that changed in round r; the
 //          host launches rounds until a round reports 0.
-// Every decode also (re)writes the entry states of the sub-sequence's slices (slot 0 = the sub-sequence's own entry
-// state, written at the end); the last decode of a sub-sequence is the one from its final entry state.
+// A decode runs quarter by quarter (eighth by eighth for images with 8 slices) and keeps, per quarter, the state at its
+// end and the units started in it (`quarters`, 8 entries per sub-sequence).  From the second decode of a sub-sequence
+// on, a decode stops as soon as it meets the trajectory of the previous one: a re-decode whose state at the end of a
+// quarter equals the recorded one is done - the rest of its trajectory, its exit state and the later quarters' counts
+// are those of the previous decode.  Between quarters the sub-sequences still running are compacted onto the first
+// threads, like between the iterations.  At the end the write pass' slice table is filled: slot 0 with the
+// sub-sequence's own entry state, the other slices' entry states from the quarter records (a slice always starts at a
+// quarter boundary).
 // The state a decode that starts `back` bits in front of a sub-sequence - blind: unit 0, DC expected - has when it
 // reaches the sub-sequence's first bit (first step boundary at or after it).  Out of line: inlined into k_huff_sync it
 // costs the symbol loops of that kernel registers (measured: 8 bytes of spills, 1.5 -> 2.2 ms).
@@ -496,22 +502,9 @@ __device__ __noinline__ uint2 preroll_state(const uint32_t *__restrict__ words, 
     return make_uint2(o.p, o.cz);
 }
 
-struct SliceStore {
-    uint4 *base;
-    __device__ __forceinline__ void operator()(uint32_t k, uint32_t p, uint32_t cz, uint32_t cnt) const { base[k] = make_uint4(p, cz, cnt, 0u); }
-};
-
 struct NoRec {
     __device__ __forceinline__ void operator()(uint32_t, uint32_t, uint32_t, uint32_t) const {}
 };
-// PHASED: from the second decode of a sub-sequence on, a decode stops as soon as it meets the trajectory of the
-// previous one.  Every decode runs quarter by quarter (eighth by eighth for images with 8 slices) and keeps, per
-// quarter, the state at its end and the units started in it (`quarters`, 8 entries per sub-sequence); a re-decode whose
-// state at the end of a quarter equals the recorded one is done - the rest of its trajectory, its exit state and the
-// later quarters' counts are those of the previous decode.  Between quarters the sub-sequences still running are
-// compacted onto the first threads, like between the iterations.  The write pass' slice table is filled from the
-// quarter records at the end (a slice always starts at a quarter boundary).
-template <bool PHASED>
 // CTAs per SM the synchronisation pass is compiled for.  Every thread walks its own 128-byte lines of the stream, so
 // the L1 has to hold about one line per resident thread or the lines are evicted before their 32 words are used:
 // 5 CTAs with the shared-memory carve-out limited to 164 KB (92 KB of L1, batch.h) beat 6 CTAs with 56 KB of L1 by
@@ -535,8 +528,8 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
     __shared__ uint16_t s_work[2][kHuffThreads];
     __shared__ uint32_t s_nwork[2];
     __shared__ uint32_t s_flag;
-    __shared__ uint2 s_cur[PHASED ? kHuffThreads : 1];                      // PHASED: state at the end of the last quarter done
-    __shared__ uint16_t s_plist[2][PHASED ? kHuffThreads : 1];              // PHASED: sub-sequences still running in this iteration
+    __shared__ uint2 s_cur[kHuffThreads];                                   // state at the end of the last quarter done
+    __shared__ uint16_t s_plist[2][kHuffThreads];                           // sub-sequences still running in this iteration
     __shared__ uint32_t s_pn[2];
     __shared__ uint32_t s_w[kHuffThreads / 32 + 1];
     __shared__ uint32_t s_wf[kHuffThreads / 32 + 1];
@@ -595,7 +588,7 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
         }
     }
 
-    const uint32_t ql2 = slices_log2 > 2u ? slices_log2 : 2u;               // PHASED: quarters (or eighths) per sub-sequence
+    const uint32_t ql2 = slices_log2 > 2u ? slices_log2 : 2u;               // quarters (or eighths) per sub-sequence
     const uint32_t qbits = (im.sub_bytes >> ql2) * 8u;
     uint4 *img_quarters = quarters + ((size_t)im.sub_base << 3);
 
@@ -605,56 +598,41 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
         const uint32_t nw = s_nwork[cur];
         if (nw == 0) break;
         if (debug_max_iters && iter >= debug_max_iters) break;                // (measurement only: the result is not the fixed point)
-        if (!PHASED) {
-            for (uint32_t w = tid; w < nw; w += kHuffThreads) {
-                const uint32_t item = s_work[cur][w];
-                HuffState in;
-                in.p = s_in[item].x; in.cz = s_in[item].y;
-                uint32_t started;
-                SliceStore rec;
-                rec.base = img_slices + ((size_t)(first_j + item) << slices_log2);
+        const bool has_prev = round > 0 || iter > 0;                        // every sub-sequence on the list has been decoded before
+        for (uint32_t w = tid; w < nw; w += kHuffThreads) s_plist[0][w] = s_work[cur][w];
+        if (tid == 0) { s_pn[0] = nw; s_pn[1] = 0; }
+        int pc = 0;
+        for (uint32_t q = 0; q < (1u << ql2); q++) {
+            __syncthreads();
+            const uint32_t pn = s_pn[pc];
+            if (pn == 0) break;
+            for (uint32_t w = tid; w < pn; w += kHuffThreads) {
+                const uint32_t item = s_plist[pc][w];
                 const uint2 span = s_span[item];
-                const HuffState o = decode_span(words, luts, g, in, span.x, span.y, slice_bits, rec, &started);
-                s_out[item] = make_uint2(o.p, o.cz);
-                s_tot[item] = started;
-            }
-        } else {
-            const bool has_prev = round > 0 || iter > 0;                    // every sub-sequence on the list has been decoded before
-            for (uint32_t w = tid; w < nw; w += kHuffThreads) s_plist[0][w] = s_work[cur][w];
-            if (tid == 0) { s_pn[0] = nw; s_pn[1] = 0; }
-            int pc = 0;
-            for (uint32_t q = 0; q < (1u << ql2); q++) {
-                __syncthreads();
-                const uint32_t pn = s_pn[pc];
-                if (pn == 0) break;
-                for (uint32_t w = tid; w < pn; w += kHuffThreads) {
-                    const uint32_t item = s_plist[pc][w];
-                    const uint2 span = s_span[item];
-                    const uint32_t qs = span.x + q * qbits, qe = min(qs + qbits, span.y);
-                    const bool last = qe >= span.y;
-                    const uint2 e = q == 0 ? s_in[item] : s_cur[item];
-                    HuffState in;
-                    in.p = e.x; in.cz = e.y;
-                    uint32_t n;
-                    NoRec rec;
-                    const HuffState o = decode_span(words, luts, g, in, qs, qe, qbits, rec, &n);
-                    uint4 *qr = img_quarters + ((size_t)(first_j + item) << 3) + q;
-                    uint4 old = make_uint4(0u, 0u, 0u, 0u);
-                    if (has_prev) old = *qr;
-                    *qr = make_uint4(o.p, o.cz, n, 0u);
-                    s_tot[item] = (q == 0 && !has_prev ? 0u : s_tot[item]) + n - old.z;
-                    if (last) s_out[item] = make_uint2(o.p, o.cz);
-                    else if (!(has_prev && old.x == o.p && old.y == o.cz)) {        // not yet on the old trajectory: go on
-                        s_cur[item] = make_uint2(o.p, o.cz);
-                        s_plist[pc ^ 1][atomicAdd(&s_pn[pc ^ 1], 1u)] = (uint16_t)item;
-                    }
+                const uint32_t qs = span.x + q * qbits, qe = min(qs + qbits, span.y);
+                const bool last = qe >= span.y;
+                const uint2 e = q == 0 ? s_in[item] : s_cur[item];
+                HuffState in;
+                in.p = e.x; in.cz = e.y;
+                uint32_t n;
+                NoRec rec;
+                const HuffState o = decode_span(words, luts, g, in, qs, qe, qbits, rec, &n);
+                uint4 *qr = img_quarters + ((size_t)(first_j + item) << 3) + q;
+                uint4 old = make_uint4(0u, 0u, 0u, 0u);
+                if (has_prev) old = *qr;
+                *qr = make_uint4(o.p, o.cz, n, 0u);
+                s_tot[item] = (q == 0 && !has_prev ? 0u : s_tot[item]) + n - old.z;
+                if (last) s_out[item] = make_uint2(o.p, o.cz);
+                else if (!(has_prev && old.x == o.p && old.y == o.cz)) {            // not yet on the old trajectory: go on
+                    s_cur[item] = make_uint2(o.p, o.cz);
+                    s_plist[pc ^ 1][atomicAdd(&s_pn[pc ^ 1], 1u)] = (uint16_t)item;
                 }
-                __syncthreads();
-                if (tid == 0) s_pn[pc] = 0;
-                pc ^= 1;
             }
             __syncthreads();
+            if (tid == 0) s_pn[pc] = 0;
+            pc ^= 1;
         }
+        __syncthreads();
         if (tid == 0) s_nwork[cur ^ 1] = 0;
         __syncthreads();
         if (active && tid > 0 && !u.head) {
@@ -698,7 +676,7 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
         // exclusive: a head starts from zero; otherwise inclusive minus own
         st_in[gj] = s_in[tid];
         img_slices[(size_t)j << slices_log2] = make_uint4(s_in[tid].x, s_in[tid].y, 0u, 0u);
-        if (PHASED && slices_log2) {                                       // slice k starts where quarter k * step - 1 ended
+        if (slices_log2) {                                                 // slice k starts where quarter k * step - 1 ended
             const uint32_t step = 1u << (ql2 - slices_log2);
             const uint4 *qr = img_quarters + ((size_t)j << 3);
             const uint32_t nsl = u.end_bit > u.start_bit ? (u.end_bit - u.start_bit + slice_bits - 1u) / slice_bits : 1u;
@@ -849,11 +827,7 @@ k_huff_write(const HuffImg *__restrict__ imgs, HuffImgState *__restrict__ ist, c
             // (bit 6 of S = "the unit is complete" stays set until unit_end has handed over)
             cur.step_plain(luts, sink);
 #if BJ_WRITE_STEPS > 1
-#ifdef BJ_WRITE_ROLLED
-#pragma unroll 1
-#else
 #pragma unroll
-#endif
             for (int k = 1; k < BJ_WRITE_STEPS && !(cur.S & 0x40u); k++) cur.step_plain(luts, sink);
 #endif
             const bool fin = (cur.S & 0x40u) != 0u;

@@ -9,7 +9,6 @@
 // unit-major IDCT phase and the row-major colour phase), colour conversion is a second warp-cooperative phase
 // whose lanes walk along pixel rows, and pixels leave through 128-bit global stores.
 #pragma once
-#include <cuda.h>
 #include "bj_dev.h"
 #include "idct_color.cuh"
 
@@ -87,8 +86,8 @@ __device__ __forceinline__ void store_ref_rows(int16_t *ob, const int (&c0)[8], 
 //     block = (pr / 2) * ((W + 1) / 2) + pc / 2,  pos = (pr % 2) * 2 + pc % 2,
 //     short index = block * 768 + component * 256 + pos * 64 + row * 8 + x
 // (the split into MAX_MCU_PER_DPU chunks is the same linear buffer: a chunk is MAX_MCU_PER_DPU / 4 whole blocks).
-// Stages 1-3 of one tile, common to the two kernels below: the tile's coefficient units are in `s_du` (unit du's 16-byte
-// chunk c at chunk position c ^ (du & 7)), the image's quantiser set in `s_q`, the predicted DC values in `s_dc`.
+// Stages 1-3 of one tile of k_idct_color below: the tile's coefficient units are in `s_du` (unit du's 16-byte chunk c
+// at chunk position c ^ (du & 7)), the image's quantiser set in `s_q`, the predicted DC values in `s_dc`.
 // Stage 1 of one tile: dequantise + IDCT, one thread = one unit, in place in `s_du`.
 __device__ __forceinline__ void tile_idct(uint4 *s_du, const uint32_t *s_q, const uint16_t *s_dc, const int ndu, const int hs, const int vs,
                                           const int bpm, const bool dc_sep) {
@@ -340,91 +339,6 @@ k_idct_color(const int16_t *__restrict__ coef, const int16_t *__restrict__ dc_pl
     if (ncomp == 3 && hs == 2 && vs == 2) tile_color_store<REF_MCUS, 2, 2>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
     else if (ncomp == 3 && hs == 1 && vs == 1) tile_color_store<REF_MCUS, 1, 1>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
     else tile_color_store<REF_MCUS, 0, 0>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
-}
-
-// ------------------------------------------------------------------------------------------------ fast layout, TMA
-// The same tile work in a PERSISTENT kernel whose coefficient tiles arrive by TMA: one CTA per slot of the GPU loops
-// over tiles; while it computes tile k, the tensor-map copy of tile k + 1 (one `cp.async.bulk.tensor.2d` of up to 192
-// rows of 128 bytes = 24 KB, issued by one thread, completion on an mbarrier) fills the other shared-memory buffer.
-// The copy's 128-byte swizzle is exactly the layout the IDCT phase wants (chunk c of unit du at chunk c ^ (du & 7) when
-// the buffer is 1024-byte aligned), so there is no register staging, no shared-memory store and no address arithmetic
-// for the load at all.  A tile with fewer than 192 units still copies 192 rows (the rows behind it belong to the next
-// tile or are zero-filled past the end of the tensor); they are not used.
-constexpr int kTmaRows = kTileThreads;                   // box of the tensor map: 192 rows x 128 bytes
-constexpr int kTmaBufBytes = kTmaRows * 128;
-constexpr int kSmemIdctTma = 1024 + 2 * kTmaBufBytes + kSmemQ + 16 + 2 * kTileThreads + kRgbFront + kRgbMax + 64;   // (1024: alignment slack; 16: two mbarriers; then the DC values)
-
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-// false: the barrier did not complete within the bound (a broken tensor map would otherwise hang the GPU)
-__device__ __forceinline__ bool mbar_wait(uint64_t *bar, uint32_t parity) {
-    const uint32_t a = smem_u32(bar);
-    for (uint32_t spin = 0; spin < (1u << 24); spin++) {
-        uint32_t ok;
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(ok) : "r"(a), "r"(parity) : "memory");
-        if (ok) return true;
-    }
-    return false;
-}
-__device__ __forceinline__ void tma_load_2d(void *dst, const void *tmap, uint64_t *bar, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
-}
-
-__global__ void __launch_bounds__(kTileThreads, 3)
-k_idct_color_tma(const __grid_constant__ CUtensorMap tmap, const int16_t *__restrict__ dc_plane, const ImgDev *__restrict__ imgs,
-                 const QTab *__restrict__ qtabs, const TileDev *__restrict__ tiles, const uint32_t ntiles, uint8_t *__restrict__ out,
-                 uint32_t *__restrict__ err) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);   // the swizzle atom is 1024 bytes
-    uint32_t *s_q = reinterpret_cast<uint32_t *>(smem + 2 * kTmaBufBytes);
-    uint64_t *s_bar = reinterpret_cast<uint64_t *>(smem + 2 * kTmaBufBytes + kSmemQ);
-    uint16_t *s_dc = reinterpret_cast<uint16_t *>(smem + 2 * kTmaBufBytes + kSmemQ + 16);
-    uint8_t *s_rgb = smem + 2 * kTmaBufBytes + kSmemQ + 16 + 2 * kTileThreads + kRgbFront;
-
-    const int tid = threadIdx.x;
-    if (tid == 0) {
-        mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint32_t k = blockIdx.x;
-    if (tid == 0 && k < ntiles) {                                          // the first tile of this CTA
-        mbar_expect_tx(&s_bar[0], kTmaBufBytes);
-        tma_load_2d(smem, &tmap, &s_bar[0], 0, (int)__ldg(&tiles[k].du0));
-    }
-    for (uint32_t it = 0; k < ntiles; k += gridDim.x, it++) {
-        const uint32_t buf = it & 1u;
-        if (tid == 0 && k + gridDim.x < ntiles) {                          // the next tile into the other buffer (free since the barrier that ended the last iteration)
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            mbar_expect_tx(&s_bar[buf ^ 1u], kTmaBufBytes);
-            tma_load_2d(smem + (buf ^ 1u) * kTmaBufBytes, &tmap, &s_bar[buf ^ 1u], 0, (int)__ldg(&tiles[k + gridDim.x].du0));
-        }
-        TileDev t;
-        {
-            const uint4 tw = __ldg(reinterpret_cast<const uint4 *>(tiles) + k);
-            t.img = tw.x; t.my = (uint16_t)tw.y; t.mx0 = (uint16_t)(tw.y >> 16); t.nm = (uint16_t)tw.z; t.ndu = (uint16_t)(tw.z >> 16); t.du0 = tw.w;
-        }
-        const ImgDev *__restrict__ im = imgs + t.img;
-        const int hs = im->hs, vs = im->vs, ncomp = im->ncomp, bpm = im->bpm;
-        {
-            const uint32_t *__restrict__ q = &qtabs[im->qslot].q16[0][0];
-            for (int i = tid; i < 3 * kQPitch; i += kTileThreads) s_q[i] = __ldg(q + i);
-        }
-        s_dc[tid] = tid < (int)t.ndu ? (uint16_t)__ldg(dc_plane + (size_t)t.du0 + tid) : (uint16_t)0;
-        if (!mbar_wait(&s_bar[buf], (it >> 1) & 1u)) { if (tid == 0) atomicAdd(err, 1u); return; }   // (never: see mbar_wait)
-        __syncthreads();
-        tile_idct(reinterpret_cast<uint4 *>(smem + buf * kTmaBufBytes), s_q, s_dc, t.ndu, hs, vs, bpm, true);
-        __syncthreads();
-        tile_color_store<false, 0, 0>(reinterpret_cast<const uint4 *>(smem + buf * kTmaBufBytes), s_rgb, t, im, hs, vs, ncomp, bpm, out);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");        // this buffer was written through the generic proxy; the next copy into it is the async proxy's
-        __syncthreads();                                                   // s_rgb, s_q, s_dc and this buffer are free again
-    }
 }
 
 // REF_MCUS: what the DPUs leave in the parts of the buffer no pixel lives in - positions of the 2x2-padded grid outside

@@ -117,11 +117,10 @@ def test_stage_entropy_slices(dec, slices, bits, golden, golden_dir):
 
 
 @pytest.mark.parametrize("bits,slices,rounds", [(0, 0, 0), (128, 0, 0), (256, 2, 0), (1024, 0, 2), (4096, 4, 0), (512, 8, 0), (160, 0, 0), (0, 8, 0)])
-def test_stage_entropy_unphased_synchronisation(dec, bits, slices, rounds, golden, golden_dir):
-    """Option "sync_phased" = 0: the synchronisation pass decodes whole sub-sequences every time and records the write
-    pass' slices on the way (default: quarter by quarter, re-decodes stop where they meet the previous decode's
-    trajectory, the slice table is derived from the quarter records).  Same coefficients."""
-    dec.set_option("sync_phased", 0)
+def test_stage_entropy_sync_layouts(dec, bits, slices, rounds, golden, golden_dir):
+    """Every golden file under a grid of sub-sequence sizes, slice counts and fix-up rounds: the synchronisation pass
+    decodes quarter by quarter (eighth by eighth with 8 slices), re-decodes stop where they meet the previous decode's
+    trajectory, and the write pass' slice table is derived from the quarter records.  Same coefficients."""
     dec.set_option("subseq_bits", bits)
     dec.set_option("slices", slices)
     dec.set_option("sync_rounds", rounds)
@@ -132,27 +131,20 @@ def test_stage_entropy_unphased_synchronisation(dec, bits, slices, rounds, golde
             assert status == 0
             assert np.array_equal(coef, ol.Restated(data, 0).coef_zz), (name, bits, slices)
     finally:
-        dec.set_option("sync_phased", 1)
         dec.set_option("subseq_bits", 0)
         dec.set_option("slices", 0)
         dec.set_option("sync_rounds", 0)
 
 
-def test_full_path_unphased_synchronisation(dec, golden, golden_dir):
+def test_removed_kernel_options_refused(dec):
+    """The persistent TMA IDCT kernel and the synchronisation pass without early stop are gone: their options are
+    refused, and "sync_phased" = 1 names the one synchronisation pass that is left."""
     import pim_jpeg_decoder_b200 as bj
-    names = _names()
-    files = [_load(golden, golden_dir, n) for n in names] + [js.synth_jpeg(1280, 720, seed=5, subsampling=2), js.synth_jpeg(640, 480, seed=6, subsampling=0, restart_blocks=7)]
-    dec.set_option("sync_phased", 0)
-    try:
-        outs, status = dec.decode(files, bj.BJ_OUT_BMP)
-    finally:
-        dec.set_option("sync_phased", 1)
-    ref, st2 = dec.decode(files, bj.BJ_OUT_BMP)
-    assert status == st2 and all(s == 0 for s in status)
-    for a, b in zip(outs, ref):
-        assert np.array_equal(a, b)
-    for n, o in zip(names, outs):
-        assert sha(o) == golden[golden[n]["expect"]]["bmp_sha256"], n
+    for name, value in (("idct_tma", 0), ("idct_tma", 1), ("sync_phased", 0)):
+        with pytest.raises(bj.BjError) as e:
+            dec.set_option(name, value)
+        assert e.value.status == -1, (name, value)                   # BJ_ERR_ARG
+    dec.set_option("sync_phased", 1)
 
 
 @pytest.mark.parametrize("rounds,bits", [(1, 128), (2, 256), (7, 128), (12, 1024)])
