@@ -39,14 +39,14 @@ constexpr int kSmemLutMax = 3 * (kLutCapDC + kLutCapAC) * 4;
 constexpr int kSmemHuffWriteMax = kSmemHuffStage + kSmemLutMax;
 constexpr int kSmemHuffSyncMax = kSmemLutMax;
 
-inline int batch_kernels_init(bj_ctx *c) {
-    if (c->check(cudaFuncSetAttribute(k_huff_write, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffWriteMax)) != BJ_OK) return BJ_ERR_CUDA;
-    if (c->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
+inline int batch_kernels_init(Device *dev) {
+    if (dev->check(cudaFuncSetAttribute(k_huff_write, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffWriteMax)) != BJ_OK) return BJ_ERR_CUDA;
+    if (dev->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
 #ifndef BJ_SYNC_CARVEOUT
 #define BJ_SYNC_CARVEOUT 72            // % of 228 KB: 164 KB of shared memory for 5 CTAs, the rest is L1 (kernels_huff.cuh: BJ_SYNC_CTAS)
 #endif
 #if BJ_SYNC_CARVEOUT > 0
-    if (c->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributePreferredSharedMemoryCarveout, BJ_SYNC_CARVEOUT)) != BJ_OK) return BJ_ERR_CUDA;
+    if (dev->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributePreferredSharedMemoryCarveout, BJ_SYNC_CARVEOUT)) != BJ_OK) return BJ_ERR_CUDA;
 #endif
     return BJ_OK;
 }
@@ -54,7 +54,7 @@ inline int batch_kernels_init(bj_ctx *c) {
 }  // namespace bj
 
 struct bj_batch {
-    bj_ctx *ctx = nullptr;
+    bj::Device *dev = nullptr;
     int n = 0, format = 0;
     int rounds = 3;
 
@@ -123,18 +123,19 @@ constexpr int kMaxRounds = 64;
 //             then the scan itself - raw (stuffed, with RSTn; kinds[i] = BJ_SCAN_RAW) or the reference's
 //             Header::huffman_data (un-stuffed, markers removed; BJ_SCAN_UNSTUFFED, only without a restart interval:
 //             read_JPEG throws the RSTn positions away, SURVEY 0.8) - and nothing is parsed.
-inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format, size_t out_cap = ~(size_t)0,
+inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, const size_t *lens, int n, int format, size_t out_cap = ~(size_t)0,
                         const bj_image_desc *descs = nullptr, const int *kinds = nullptr) {
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
-    b->ctx = c; b->n = n; b->format = format;
+    const bj_ctx *c = dev->ctx;
+    b->dev = dev; b->n = n; b->format = format;
     b->uploaded = b->decoded = b->synced = false;
     b->desc.resize(n); b->parse_status.assign(n, BJ_OK);
-    if (c->check(cudaSetDevice(c->device)) != BJ_OK) return BJ_ERR_CUDA;
-    for (auto &e : b->ev) if (!e && c->check(cudaEventCreate(&e)) != BJ_OK) return BJ_ERR_CUDA;
+    if (dev->check(cudaSetDevice(dev->ordinal)) != BJ_OK) return BJ_ERR_CUDA;
+    for (auto &e : b->ev) if (!e && dev->check(cudaEventCreate(&e)) != BJ_OK) return BJ_ERR_CUDA;
 
     // ---- headers (per image, independent: worker pool).  Nothing behind the SOS header is read.
     std::vector<Geometry> geo(n);
-    c->host_pool.parallel_for(n, 64, [&](int i0, int i1) {
+    dev->host_pool.parallel_for(n, 64, [&](int i0, int i1) {
         for (int i = i0; i < i1; i++) {
             bj_image_desc &d = b->desc[i];
             int rc;
@@ -205,7 +206,7 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
     uint32_t nominal_sub = 512;
     uint64_t total_scan = 0;
     for (int i = 0; i < n; i++) if (b->parse_status[i] == BJ_OK) total_scan += b->desc[i].scan_len;
-    if (!fixed_sub) nominal_sub = (uint32_t)std::min<uint64_t>(512u, std::max<uint64_t>(kMinSubBytes, total_scan / ((uint64_t)c->sm_count * 3072u)));
+    if (!fixed_sub) nominal_sub = (uint32_t)std::min<uint64_t>(512u, std::max<uint64_t>(kMinSubBytes, total_scan / ((uint64_t)dev->sm_count * 3072u)));
     auto round_sub = [&](uint32_t len, uint32_t rl) { const uint32_t q = 4u << rl; return (std::max(len, 64u) + q - 1u) / q * q; };
     auto sub_layout_of = [&](uint32_t raw_len, uint32_t nseg, uint32_t *rl) -> uint32_t {
         *rl = c->slices ? fixed_rl : 0u;
@@ -393,7 +394,7 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
     // ---- stage the file bytes (only when they cannot go up from where they are; per image, independent: worker pool)
     if (!b->direct_src) {
         uint8_t *hf = reinterpret_cast<uint8_t *>(b->h_files.p);
-        c->host_pool.parallel_for(n, 16, [&](int i0, int i1) {
+        dev->host_pool.parallel_for(n, 16, [&](int i0, int i1) {
             for (int i = i0; i < i1; i++) {
                 if (b->parse_status[i] != BJ_OK) continue;
                 memcpy(hf + b->file_off[i], files[i], lens[i]);
@@ -417,16 +418,16 @@ inline int batch_assign(bj_batch *b, bj_ctx *c, const uint8_t *const *files, con
 
 // H2D of the file bytes and the per-image records; the per-CTA maps are then expanded on the device.
 inline int batch_upload(bj_batch *b, cudaStream_t s) {
-    bj_ctx *c = b->ctx;
-    if (c->check(cudaSetDevice(c->device)) != BJ_OK) return BJ_ERR_CUDA;
+    Device *dev = b->dev;
+    if (dev->check(cudaSetDevice(dev->ordinal)) != BJ_OK) return BJ_ERR_CUDA;
     b->last_stream = s;
     if (b->n == 0) { b->uploaded = true; return BJ_OK; }
-    int rc = c->check(cudaMemcpyAsync(b->d_files.p, b->direct_src ? (const void *)b->direct_src : b->h_files.p, b->files_bytes, cudaMemcpyHostToDevice, s));
-    if (rc == BJ_OK) rc = c->check(cudaMemcpyAsync(b->d_meta.p, b->h_meta.p, b->meta_bytes, cudaMemcpyHostToDevice, s));
+    int rc = dev->check(cudaMemcpyAsync(b->d_files.p, b->direct_src ? (const void *)b->direct_src : b->h_files.p, b->files_bytes, cudaMemcpyHostToDevice, s));
+    if (rc == BJ_OK) rc = dev->check(cudaMemcpyAsync(b->d_meta.p, b->h_meta.p, b->meta_bytes, cudaMemcpyHostToDevice, s));
     if (rc == BJ_OK) {
         k_expand_maps<<<b->n, 256, 0, s>>>(b->dmeta<HuffImg>(b->o_himg), b->dmeta<ImgDev>(b->o_idev), b->dmap<uint32_t>(b->m_utile), b->dmap<uint32_t>(b->m_blk),
                                           b->dmap<uint32_t>(b->m_wblk), b->dmap<uint32_t>(b->m_dcc), b->dmap<TileDev>(b->m_tiles));
-        rc = c->check(cudaGetLastError());
+        rc = dev->check(cudaGetLastError());
     }
     b->uploaded = rc == BJ_OK;
     return rc;
@@ -434,7 +435,7 @@ inline int batch_upload(bj_batch *b, cudaStream_t s) {
 
 // Launch sync rounds [r0, r1) and everything after them.
 inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
-    bj_ctx *c = b->ctx;
+    const bj_ctx *c = b->dev->ctx;
     const HuffImg *himg = b->dmeta<HuffImg>(b->o_himg);
     const ImgDev *idev = b->dmeta<ImgDev>(b->o_idev);
     const QTab *qtabs = b->dmeta<QTab>(b->o_qtab);
@@ -516,13 +517,13 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
     cudaEventRecord(b->ev[4], s);
     cudaMemcpyAsync(b->h_state(), st, (size_t)n * sizeof(HuffImgState), cudaMemcpyDeviceToHost, s);
     cudaMemcpyAsync(b->h_flags(), flags, kMaxRounds * 4, cudaMemcpyDeviceToHost, s);
-    return c->check(cudaGetLastError());
+    return b->dev->check(cudaGetLastError());
 }
 
 inline int batch_decode(bj_batch *b, cudaStream_t s) {
-    bj_ctx *c = b->ctx;
+    const bj_ctx *c = b->dev->ctx;
     if (!b->uploaded) return BJ_ERR_ARG;
-    if (c->check(cudaSetDevice(c->device)) != BJ_OK) return BJ_ERR_CUDA;
+    if (b->dev->check(cudaSetDevice(b->dev->ordinal)) != BJ_OK) return BJ_ERR_CUDA;
     b->last_stream = s;
     b->decoded = true; b->synced = false;
     if (b->n == 0) return BJ_OK;
@@ -536,18 +537,18 @@ inline int batch_decode(bj_batch *b, cudaStream_t s) {
 // Wait for the decode; if the last fix-up round still changed something (a sub-sequence that needed more than a
 // whole CTA to synchronise - pathological), run more rounds and redo what depends on them.
 inline int batch_sync(bj_batch *b) {
-    bj_ctx *c = b->ctx;
+    Device *dev = b->dev;
     if (!b->decoded) return BJ_ERR_ARG;
     if (b->n == 0) { b->synced = true; return BJ_OK; }
     cudaStream_t s = b->last_stream;
-    int rc = c->check(cudaStreamSynchronize(s));
+    int rc = dev->check(cudaStreamSynchronize(s));
     int r = b->rounds;
     b->redone = false;
     while (rc == BJ_OK && b->n_blk && b->multi_blk && b->h_flags()[r - 1] != 0) {
         b->redone = true;
-        if (r + 2 > kMaxRounds) { c->last_error = "entropy stage did not converge"; return BJ_ERR_CUDA; }
+        if (r + 2 > kMaxRounds) { dev->ctx->set_error("entropy stage did not converge"); return BJ_ERR_CUDA; }
         rc = batch_launch(b, s, r, r + 2);
-        if (rc == BJ_OK) rc = c->check(cudaStreamSynchronize(s));
+        if (rc == BJ_OK) rc = dev->check(cudaStreamSynchronize(s));
         r += 2;
     }
     b->rounds = r;
@@ -564,7 +565,7 @@ inline int batch_sync(bj_batch *b) {
 
 // Enqueue the device->host copies of every decoded image (no host wait).
 inline int batch_download_async(bj_batch *b, uint8_t *const *outs, cudaStream_t s) {
-    bj_ctx *c = b->ctx;
+    Device *dev = b->dev;
     int rc = BJ_OK;
     b->d2h_bytes = 0; b->d2h_copies = 0;
     // option "packed_outputs": the caller states that host buffers laid out like the device buffer (see
@@ -576,9 +577,9 @@ inline int batch_download_async(bj_batch *b, uint8_t *const *outs, cudaStream_t 
         if (b->parse_status[i] != BJ_OK || !outs[i]) { i++; continue; }
         int k = i;
         size_t end = b->out_off[i] + b->out_size[i];
-        while (c->packed_outputs && k + 1 < b->n && b->parse_status[k + 1] == BJ_OK && outs[k + 1] &&
+        while (dev->ctx->packed_outputs && k + 1 < b->n && b->parse_status[k + 1] == BJ_OK && outs[k + 1] &&
                outs[k + 1] == outs[i] + (b->out_off[k + 1] - b->out_off[i])) { k++; end = b->out_off[k] + b->out_size[k]; }
-        rc = c->check(cudaMemcpyAsync(outs[i], (const uint8_t *)b->d_out.p + b->out_off[i], end - b->out_off[i], cudaMemcpyDeviceToHost, s));
+        rc = dev->check(cudaMemcpyAsync(outs[i], (const uint8_t *)b->d_out.p + b->out_off[i], end - b->out_off[i], cudaMemcpyDeviceToHost, s));
         b->d2h_bytes += end - b->out_off[i]; b->d2h_copies++;
         i = k + 1;
     }
@@ -590,7 +591,7 @@ inline int batch_download(bj_batch *b, uint8_t *const *outs, cudaStream_t s) {
     int rc = BJ_OK;
     if (!b->synced) rc = batch_sync(b);           // the (rare) extra fix-up rounds must be settled before copying out
     if (rc == BJ_OK) rc = batch_download_async(b, outs, s);
-    if (rc == BJ_OK) rc = b->ctx->check(cudaStreamSynchronize(s));
+    if (rc == BJ_OK) rc = b->dev->check(cudaStreamSynchronize(s));
     return rc;
 }
 

@@ -126,9 +126,13 @@ constexpr int kSlots = 3;             // sub-batches in flight inside bj_decode_
 
 enum { POOL_COMPAT_MD = 0, POOL_COMPAT_MCUS, POOL_COEF, POOL_OUT, POOL_IMGS, POOL_TILES, POOL_COUNT };
 
+// counters of one bj_decode_batch / job (bj_get_stat: "decode_batch_<name>", "total_<name>")
+enum { ST_SUB = 0, ST_LAUNCH, ST_H2D, ST_D2H, ST_HOST_MS, ST_WAIT_MS, ST_D2H_COPIES, ST_MS_UNSTUFF, ST_MS_SYNC, ST_MS_WRITE, ST_MS_IDCT, ST_DIRECT, ST_COUNT };
+
 }  // namespace bj
 
 struct bj_job;
+struct bj_batch;
 
 namespace bj {
 // The thread behind bj_submit / bj_wait: runs the submitted batches one after the other (b200jpeg.cu).
@@ -141,11 +145,11 @@ struct AsyncWorker {
     void run();
     bool pending() { std::lock_guard<std::mutex> l(m); return !q.empty(); }
 };
+struct Device;
 }  // namespace bj
 
+// A context: the options and counters, and the GPUs it drives (one for bj_create, several for bj_create_multi).
 struct bj_ctx {
-    int device = 0;
-    int sm_count = 0;
     int subseq_bits = 0;                 // sub-sequence length of the synchronisation pass; 0 = automatic (per image)
     int slices = 0;                      // slices (write pass) per sub-sequence: 1, 2, 4, 8; 0 = default (1)
     size_t sub_batch_bytes = 0;          // 0 = default
@@ -160,26 +164,35 @@ struct bj_ctx {
     size_t max_image_pixels = (size_t)1 << 28;   // larger images are refused (BJ_ERR_UNSUPPORTED), like the reference's "Too high resolution"
     size_t sub_batch_out_bytes = (size_t)1 << 30; // decoded bytes per sub-batch of bj_decode_batch
     int sync_rounds = 0;                 // 0 = default (3 launches of the fix-up kernel before the first check)
-    struct bj_batch *slots[bj::kSlots] = {};          // sub-batches of bj_decode_batch in flight (one stream each)
-    bj::HostPool host_pool;
-    double stats[16] = {};               // counters of the last bj_decode_batch / job (b200jpeg.cu: ST_*)
-    double totals[16] = {};              // ... summed over every call since bj_create
-    cudaStream_t streams[bj::kSlots] = {};
-    cudaEvent_t ev_exec[2] = {nullptr, nullptr};      // bj_exec_mcus: around the kernel ("DPU execution" profile line)
-    std::vector<bj_ctx *> children;      // bj_create_multi: one single-device context per GPU; this one only deals the work
+    std::vector<bj::Device *> devs;      // never empty; staged and stage-level entries run on devs[0]
     bj::AsyncWorker *async = nullptr;    // bj_submit / bj_wait
-    bj::DevBuf pool[bj::POOL_COUNT];
+    double stats[bj::ST_COUNT] = {};     // counters of the last bj_decode_batch / job, folded over the devices
+    double totals[bj::ST_COUNT] = {};    // ... summed over every call since bj_create
+    std::mutex error_m;                  // the devices' host threads report errors side by side
     std::string last_error;
+    void set_error(const char *what) { std::lock_guard<std::mutex> l(error_m); last_error = what; }
+};
+
+namespace bj {
+
+// One GPU of a context: what its host thread works with.
+struct Device {
+    bj_ctx *ctx = nullptr;
+    int ordinal = 0;
+    int sm_count = 0;
+    bj_batch *slots[kSlots] = {};        // sub-batches of bj_decode_batch in flight (one stream each)
+    cudaStream_t streams[kSlots] = {};
+    cudaEvent_t ev_exec[2] = {nullptr, nullptr};      // bj_exec_mcus: around the kernel ("DPU execution" profile line)
+    DevBuf pool[POOL_COUNT];
+    HostPool host_pool;
     float last_exec_ms = 0.f;
     int check(cudaError_t e) {
         if (e == cudaSuccess) return BJ_OK;
-        last_error = cudaGetErrorString(e);
+        ctx->set_error(cudaGetErrorString(e));
         cudaGetLastError();
         return BJ_ERR_CUDA;
     }
 };
-
-namespace bj {
 
 struct Geometry {
     uint32_t nmx, nmy, nmcu, bpm, ndu;   // MCUs per row/column, total, data units per MCU, total data units
