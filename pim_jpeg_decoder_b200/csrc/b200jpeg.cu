@@ -180,8 +180,8 @@ extern "C" int bj_set_option(bj_ctx *c, const char *name, long value) {
     if (!strcmp(name, "max_image_pixels")) { if (value < 1) return BJ_ERR_ARG; c->max_image_pixels = (size_t)value; return BJ_OK; }
     if (!strcmp(name, "sub_batch_out_bytes")) { if (value < (1 << 16)) return BJ_ERR_ARG; c->sub_batch_out_bytes = (size_t)value; return BJ_OK; }
     if (!strcmp(name, "host_threads")) { if (value < 1 || value > 256) return BJ_ERR_ARG; for (Device *dev : c->devs) dev->host_pool.resize((int)value); return BJ_OK; }
-    if (!strcmp(name, "debug_sync_iters")) { if (value < 0) return BJ_ERR_ARG; c->debug_sync_iters = (int)value; return BJ_OK; }
-    if (!strcmp(name, "sync_preroll_bits")) { if (value < 0 || value > (1 << 16) || value % 32) return BJ_ERR_ARG; c->sync_preroll_bits = (int)value; return BJ_OK; }
+    // the synchronisation pass starts every sub-sequence from its own first bit; the option stays for bench.py --sync-preroll
+    if (!strcmp(name, "sync_preroll_bits")) return value == 0 ? BJ_OK : BJ_ERR_ARG;
     if (!strcmp(name, "sync_rounds")) { if (value < 0 || value > kMaxRounds) return BJ_ERR_ARG; c->sync_rounds = (int)value; return BJ_OK; }
     return BJ_ERR_ARG;
 }
@@ -473,13 +473,12 @@ static int decode_worker(Device *dev, RangeSource *src, const CallInput &in, int
     cudaEvent_t ev_base = nullptr;
     double host_t[kSlots][2] = {};
     const double wall0 = wall_ms();
-    static const bool blocking_wait = getenv("B200JPEG_SPIN_WAIT") == nullptr;
     auto finish = [&](int slot) -> int {
         bj_batch *b = dev->slots[slot];
         const double t0 = wall_ms();
         // sleep until the sub-batch's copy-out is done instead of polling for it (cudaStreamSynchronize spins by
         // default, and a polling host thread takes bandwidth from the copy-out it is waiting for)
-        if (blocking_wait && b->ev_done) cudaEventSynchronize(b->ev_done);
+        if (b->ev_done) cudaEventSynchronize(b->ev_done);
         int r = batch_sync(b);
         if (trace && r == BJ_OK && ev_base) {
             float k0 = 0, k1 = 0, out = 0;

@@ -38,16 +38,12 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 constexpr int kSmemLutMax = 3 * (kLutCapDC + kLutCapAC) * 4;
 constexpr int kSmemHuffWriteMax = kSmemHuffStage + kSmemLutMax;
 constexpr int kSmemHuffSyncMax = kSmemLutMax;
+constexpr int kSyncCarveout = 72;      // % of 228 KB: 164 KB of shared memory for 5 CTAs, the rest is L1 (kernels_huff.cuh: kSyncCtas)
 
 inline int batch_kernels_init(Device *dev) {
     if (dev->check(cudaFuncSetAttribute(k_huff_write, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffWriteMax)) != BJ_OK) return BJ_ERR_CUDA;
     if (dev->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
-#ifndef BJ_SYNC_CARVEOUT
-#define BJ_SYNC_CARVEOUT 72            // % of 228 KB: 164 KB of shared memory for 5 CTAs, the rest is L1 (kernels_huff.cuh: BJ_SYNC_CTAS)
-#endif
-#if BJ_SYNC_CARVEOUT > 0
-    if (dev->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributePreferredSharedMemoryCarveout, BJ_SYNC_CARVEOUT)) != BJ_OK) return BJ_ERR_CUDA;
-#endif
+    if (dev->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributePreferredSharedMemoryCarveout, kSyncCarveout)) != BJ_OK) return BJ_ERR_CUDA;
     return BJ_OK;
 }
 
@@ -486,7 +482,7 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
     }
     if (b->n_blk) {
         for (int r = r0; r < r1; r++) {
-            k_huff_sync<<<b->n_blk, kHuffThreads, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, (uint4 *)b->d_quarter.p, agg, flags, r, (uint32_t)c->sync_preroll_bits, (uint32_t)c->debug_sync_iters);
+            k_huff_sync<<<b->n_blk, kHuffThreads, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, (uint4 *)b->d_quarter.p, agg, flags, r);
             b->launches++; b->sync_rounds++;
         }
         cudaEventRecord(b->ev[2], s);

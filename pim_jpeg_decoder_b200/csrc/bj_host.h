@@ -157,8 +157,6 @@ struct bj_ctx {
     int packed_outputs = 0;              // see batch_download_async
     int packed_inputs = 0;               // see batch_assign: 0 = upload straight from the caller's memory when it is known to be page-locked
                                          // (bj_host_alloc / bj_host_register), 1 = the caller says it is, -1 = always stage
-    int debug_sync_iters = 0;            // measurement only: stop the in-CTA fix-up after this many iterations (0: run to the fixed point)
-    int sync_preroll_bits = 0;           // synchronisation pass: bits a sub-sequence's first guess is decoded ahead of its start (kernels_huff.cuh: PREROLL)
     int ref_m = 100;                     // BJ_OUT_REF_MCUS: MAX_MCU_PER_DPU of the host that reads the buffer (Makefile:2 of the reference)
     int debug_poison = 0;                // fill coefficient / DC / output buffers with 0xA5 before every decode (tests: every byte must be written)
     size_t max_image_pixels = (size_t)1 << 28;   // larger images are refused (BJ_ERR_UNSUPPORTED), like the reference's "Too high resolution"

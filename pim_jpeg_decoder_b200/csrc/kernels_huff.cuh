@@ -12,7 +12,7 @@
 //                                                          symbols per table lookup), entry states of the finer
 //                                                          slices the write pass works on, block-level prefix sums
 //   k_huff_write                                          (K1a) final decode of every slice from its synchronised
-//                                                          entry state, in rounds of up to BJ_WRITE_STEPS symbols per lane;
+//                                                          entry state, in rounds of up to kWriteSteps symbols per lane;
 //                                                          look-back, hand-over to the next unit and the warp-cooperative
 //                                                          stores of whole 128-byte units once per round
 //   k_zero_tail                                                 units the reference never reached read as zero
@@ -168,14 +168,12 @@ __device__ __forceinline__ void look_store(uint64_t *p, uint64_t v) {
 // One thread = kUnstuffChunks consecutive 16-byte chunks (64 bytes), a tile = 16 KB: the fixed costs of a tile - ticket,
 // barriers, the look-back's round trips through L2 - are paid once per 16 KB (with 4 KB tiles they were half of the
 // kernel's time: 77 600 CTAs that each live only a few microseconds).
-#ifndef BJ_UNSTUFF_CTAS
-#define BJ_UNSTUFF_CTAS 4                // measured on config 2: 4 CTAs per SM (56 registers) 0.425 ms, 5 (48) 0.449 ms, 6 (40, 8 bytes of spills) 0.434 ms
-#endif
+constexpr int kUnstuffCtas = 4;          // measured on config 2: 4 CTAs per SM (56 registers) 0.425 ms, 5 (48) 0.449 ms, 6 (40, 8 bytes of spills) 0.434 ms
 // Shared-memory staging of the surviving bytes: a thread writes its (up to) 64 bytes one by one, and the 32 threads of a
 // warp write 64 bytes apart - 16 of them into the same bank.  XOR-ing the word-in-block bits with the 128-byte block
 // index spreads a warp's byte stores over all 32 banks (and keeps the word reads of the store loop conflict free).
 __device__ __forceinline__ uint32_t unstuff_swz(uint32_t a) { return a ^ (((a >> 7) & 15u) << 2); }
-__global__ void __launch_bounds__(kUnstuffThreads, BJ_UNSTUFF_CTAS)
+__global__ void __launch_bounds__(kUnstuffThreads, kUnstuffCtas)
 k_unstuff(const uint8_t *__restrict__ files, const HuffImg *__restrict__ imgs, const uint32_t *__restrict__ tile_img,
           uint64_t *__restrict__ look, uint32_t *__restrict__ ticket, HuffImgState *__restrict__ st, uint32_t *__restrict__ clean,
           uint32_t *__restrict__ seg_off) {
@@ -489,19 +487,6 @@ __device__ __forceinline__ uint32_t pack16(uint32_t lo, uint32_t hi) { return (l
 // threads, like between the iterations.  At the end the write pass' slice table is filled: slot 0 with the
 // sub-sequence's own entry state, the other slices' entry states from the quarter records (a slice always starts at a
 // quarter boundary).
-// The state a decode that starts `back` bits in front of a sub-sequence - blind: unit 0, DC expected - has when it
-// reaches the sub-sequence's first bit (first step boundary at or after it).  Out of line: inlined into k_huff_sync it
-// costs the symbol loops of that kernel registers (measured: 8 bytes of spills, 1.5 -> 2.2 ms).
-__device__ __noinline__ uint2 preroll_state(const uint32_t *__restrict__ words, HuffGeom g, uint32_t start_bit, uint32_t back) {
-    HuffState in;
-    in.p = start_bit - back; in.cz = 0u;
-    uint32_t n;
-    LutMem luts;
-    struct { __device__ __forceinline__ void operator()(uint32_t, uint32_t, uint32_t, uint32_t) const {} } rec;
-    const HuffState o = decode_span(words, luts, g, in, in.p, start_bit, back, rec, &n);
-    return make_uint2(o.p, o.cz);
-}
-
 struct NoRec {
     __device__ __forceinline__ void operator()(uint32_t, uint32_t, uint32_t, uint32_t) const {}
 };
@@ -509,16 +494,13 @@ struct NoRec {
 // the L1 has to hold about one line per resident thread or the lines are evicted before their 32 words are used:
 // 5 CTAs with the shared-memory carve-out limited to 164 KB (92 KB of L1, batch.h) beat 6 CTAs with 56 KB of L1 by
 // a quarter (measured: 6: 2.09 ms, 5: 1.53 ms, 4: 2.16 ms, 3: 2.44 ms on config 2).
-#ifndef BJ_SYNC_CTAS
-#define BJ_SYNC_CTAS 5
-#endif
-__global__ void __launch_bounds__(kHuffThreads, BJ_SYNC_CTAS)
+constexpr int kSyncCtas = 5;
+__global__ void __launch_bounds__(kHuffThreads, kSyncCtas)
 k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ ist, const uint32_t *__restrict__ blk_img,
             const uint32_t *__restrict__ clean, const uint32_t *__restrict__ seg_off, const uint32_t *__restrict__ seg_sub0,
             const uint32_t *__restrict__ sub_seg, const uint32_t *__restrict__ lut_dc_pool, const uint32_t *__restrict__ lut_ac_pool,
             uint2 *__restrict__ st_in, uint2 *__restrict__ st_out, uint32_t *__restrict__ sub_tot, uint2 *__restrict__ sub_pre,
-            uint4 *__restrict__ slices, uint4 *__restrict__ quarters, BlkAgg *__restrict__ blk_agg, uint32_t *__restrict__ flags, int round,
-            uint32_t preroll_bits, uint32_t debug_max_iters) {
+            uint4 *__restrict__ slices, uint4 *__restrict__ quarters, BlkAgg *__restrict__ blk_agg, uint32_t *__restrict__ flags, int round) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     uint32_t *s_lut = reinterpret_cast<uint32_t *>(smem_raw);
     __shared__ uint2 s_in[kHuffThreads], s_out[kHuffThreads];
@@ -553,7 +535,6 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
     bool need = false;
     if (round == 0) {
         if (active) { s_in[tid] = make_uint2(u.start_bit, 0u); need = true; }
-        // (the guess is improved below, once the tables are staged: preroll)
     } else {
         if (active) { s_in[tid] = st_in[gj]; s_out[tid] = st_out[gj]; s_tot[tid] = sub_tot[gj]; }
         if (tid == 0 && !u.head && j > 0) {
@@ -574,20 +555,6 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
     const uint32_t slice_bits = (im.sub_bytes >> slices_log2) * 8u;
     uint4 *img_slices = slices + im.slice_base;
 
-    // PREROLL (round 0, option "sync_preroll_bits"): a sub-sequence that is not a segment head does not start from the
-    // blind guess "a unit begins at my first bit" but from where a decode that begins `preroll_bits` earlier (blind
-    // there: unit 0, DC) stands when it reaches the sub-sequence: a JPEG stream synchronises within some hundred bits,
-    // so this state is the true one for most sub-sequences, their first decode is already the final one and the
-    // hand-over below finds nothing to redo.  Whatever the guess, the fixed point of the iteration is the same: the
-    // preroll only buys speed.
-    if (round == 0 && preroll_bits != 0u) {
-        __syncthreads();                                                    // (the tables are staged)
-        if (active && !u.head) {
-            const uint32_t seg_bit0 = u.start_bit - u.k * im.sub_bytes * 8u;    // the segment's first bit: nothing to guess there
-            s_in[tid] = preroll_state(words, g, u.start_bit, min(preroll_bits, u.start_bit - seg_bit0));
-        }
-    }
-
     const uint32_t ql2 = slices_log2 > 2u ? slices_log2 : 2u;               // quarters (or eighths) per sub-sequence
     const uint32_t qbits = (im.sub_bytes >> ql2) * 8u;
     uint4 *img_quarters = quarters + ((size_t)im.sub_base << 3);
@@ -597,7 +564,6 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
         __syncthreads();
         const uint32_t nw = s_nwork[cur];
         if (nw == 0) break;
-        if (debug_max_iters && iter >= debug_max_iters) break;                // (measurement only: the result is not the fixed point)
         const bool has_prev = round > 0 || iter > 0;                        // every sub-sequence on the list has been decoded before
         for (uint32_t w = tid; w < nw; w += kHuffThreads) s_plist[0][w] = s_work[cur][w];
         if (tid == 0) { s_pn[0] = nw; s_pn[1] = 0; }
@@ -696,7 +662,7 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
 
 // ------------------------------------------------------------------------------------------------ K1a: write
 // One thread = one slice; a CTA's 256 slices are consecutive (kHuffThreads >> slices_log2 sub-sequences of one CTA
-// of the synchronisation pass).  A warp works in rounds: every lane takes up to BJ_WRITE_STEPS symbols
+// of the synchronisation pass).  A warp works in rounds: every lane takes up to kWriteSteps symbols
 // (WriteCursor::step_plain: no checks, no hand-over - the lanes stay together) and stops at the one that completes its
 // unit; then the lanes that completed a unit look back over it and hand over to their next unit together
 // (WriteCursor::unit_end), and the warp stores those units together.  With the hand-over inside every step (one or two
@@ -718,13 +684,9 @@ struct SmemUnitSink {
 
 constexpr int kSmemHuffStage = kHuffThreads * 128;
 
-#ifndef BJ_WRITE_STEPS
-#define BJ_WRITE_STEPS 8               // symbols a lane may take per round of the write pass (look-back, hand-over and unit stores once per round); config 2: one symbol per round with the hand-over inside the step 2.00 ms; rounds of 4 / 6 / 8 symbols 1.589 / 1.550 / 1.556 (profiles/r2_write_round_ab.txt); unrolled, with the leaner bit reader, 5 / 6 / 8: 1.513 / 1.503 / 1.493 (profiles/r2_write_unroll_ab.txt)
-#endif
-#ifndef BJ_WRITE_CTAS
-#define BJ_WRITE_CTAS 4                // shared memory allows 4; telling the compiler buys 52 registers instead of 40 (-2 %)
-#endif
-__global__ void __launch_bounds__(kHuffThreads, BJ_WRITE_CTAS)
+constexpr int kWriteSteps = 8;         // symbols a lane may take per round of the write pass (look-back, hand-over and unit stores once per round); config 2: one symbol per round with the hand-over inside the step 2.00 ms; rounds of 4 / 6 / 8 symbols 1.589 / 1.550 / 1.556 (profiles/r2_write_round_ab.txt); unrolled, with the leaner bit reader, 5 / 6 / 8: 1.513 / 1.503 / 1.493 (profiles/r2_write_unroll_ab.txt)
+constexpr int kWriteCtas = 4;          // shared memory allows 4; telling the compiler buys 52 registers instead of 40 (-2 %)
+__global__ void __launch_bounds__(kHuffThreads, kWriteCtas)
 k_huff_write(const HuffImg *__restrict__ imgs, HuffImgState *__restrict__ ist, const uint32_t *__restrict__ wblk_img,
              const uint32_t *__restrict__ clean, const uint32_t *__restrict__ seg_off, const uint32_t *__restrict__ seg_sub0,
              const uint32_t *__restrict__ sub_seg, const uint32_t *__restrict__ lut_dc_pool, const uint32_t *__restrict__ lut_ac_pool,
@@ -822,14 +784,12 @@ k_huff_write(const HuffImg *__restrict__ imgs, HuffImgState *__restrict__ ist, c
     if (!__all_sync(0xFFFFFFFFu, done)) {
         uint2 *slot = s_slot[warp];
         for (;;) {
-            // a round: up to BJ_WRITE_STEPS symbols per lane, stopping at the one that completes a unit; then the lanes
+            // a round: up to kWriteSteps symbols per lane, stopping at the one that completes a unit; then the lanes
             // that completed one look back over it and hand over to their next unit together, and the warp stores those units
             // (bit 6 of S = "the unit is complete" stays set until unit_end has handed over)
             cur.step_plain(luts, sink);
-#if BJ_WRITE_STEPS > 1
 #pragma unroll
-            for (int k = 1; k < BJ_WRITE_STEPS && !(cur.S & 0x40u); k++) cur.step_plain(luts, sink);
-#endif
+            for (int k = 1; k < kWriteSteps && !(cur.S & 0x40u); k++) cur.step_plain(luts, sink);
             const bool fin = (cur.S & 0x40u) != 0u;
             const uint32_t m = __ballot_sync(0xFFFFFFFFu, fin);
             if (m == 0) continue;

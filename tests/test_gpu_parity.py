@@ -137,14 +137,17 @@ def test_stage_entropy_sync_layouts(dec, bits, slices, rounds, golden, golden_di
 
 
 def test_removed_kernel_options_refused(dec):
-    """The persistent TMA IDCT kernel and the synchronisation pass without early stop are gone: their options are
-    refused, and "sync_phased" = 1 names the one synchronisation pass that is left."""
+    """The persistent TMA IDCT kernel, the synchronisation pass without early stop, its pre-roll and its iteration cap
+    are gone: their options are refused, and "sync_phased" = 1 and "sync_preroll_bits" = 0 name the one
+    synchronisation pass that is left."""
     import pim_jpeg_decoder_b200 as bj
-    for name, value in (("idct_tma", 0), ("idct_tma", 1), ("sync_phased", 0)):
+    for name, value in (("idct_tma", 0), ("idct_tma", 1), ("sync_phased", 0), ("sync_preroll_bits", 512),
+                        ("debug_sync_iters", 1)):
         with pytest.raises(bj.BjError) as e:
             dec.set_option(name, value)
         assert e.value.status == -1, (name, value)                   # BJ_ERR_ARG
     dec.set_option("sync_phased", 1)
+    dec.set_option("sync_preroll_bits", 0)
 
 
 @pytest.mark.parametrize("rounds,bits", [(1, 128), (2, 256), (7, 128), (12, 1024)])
