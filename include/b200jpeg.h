@@ -206,7 +206,10 @@ int bj_stage_entropy(bj_ctx *ctx, const uint8_t *file, size_t len, int16_t *coef
  *                      0 = chosen per image (2400-4096 bits, so that an image's sub-sequences fill whole CTAs;
  *                      a typical restart segment in one piece)
  *   "slices"           pieces of a sub-sequence the Huffman write pass works on (1, 2, 4 or 8; default 1: the write
- *                      pass works on whole sub-sequences)
+ *                      pass works on whole sub-sequences; at least 2 behind a 128-wide synchronisation CTA)
+ *   "sync_threads"     sub-sequences per CTA of the Huffman synchronisation pass (128 or 256); 0 = chosen per batch:
+ *                      128 when most of the batch's scan bytes are in images too small to fill a 256-wide CTA with
+ *                      sub-sequences of the automatic length, 256 otherwise and whenever "subseq_bits" is set
  *   "sync_rounds"      launches of the fix-up kernel before convergence is first checked
  *   "sub_batch_bytes"  compressed bytes per sub-batch of bj_decode_batch
  *   "sub_batch_ramp"   0: all sub-batches the same size (default 1: the first two are 1/8 and 1/3 of it, so that the

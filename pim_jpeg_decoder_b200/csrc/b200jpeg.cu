@@ -171,6 +171,7 @@ extern "C" int bj_set_option(bj_ctx *c, const char *name, long value) {
     if (!strcmp(name, "sub_batch_ramp")) { c->sub_batch_ramp = value != 0; return BJ_OK; }
     // the synchronisation pass with early stop of re-decodes is the only one; the option stays for bench.py --sync-phased
     if (!strcmp(name, "sync_phased")) return value == 1 ? BJ_OK : BJ_ERR_ARG;
+    if (!strcmp(name, "sync_threads")) { if (value != 0 && value != 128 && value != 256) return BJ_ERR_ARG; c->sync_threads = (int)value; return BJ_OK; }
     if (!strcmp(name, "slices")) { if (value != 0 && value != 1 && value != 2 && value != 4 && value != 8) return BJ_ERR_ARG; c->slices = (int)value; return BJ_OK; }
     if (!strcmp(name, "sub_batch_bytes")) { if (value < (1 << 16)) return BJ_ERR_ARG; c->sub_batch_bytes = (size_t)value; return BJ_OK; }
     if (!strcmp(name, "packed_outputs")) { c->packed_outputs = value != 0; return BJ_OK; }

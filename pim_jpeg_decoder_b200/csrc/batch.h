@@ -39,11 +39,14 @@ constexpr int kSmemLutMax = 3 * (kLutCapDC + kLutCapAC) * 4;
 constexpr int kSmemHuffWriteMax = kSmemHuffStage + kSmemLutMax;
 constexpr int kSmemHuffSyncMax = kSmemLutMax;
 constexpr int kSyncCarveout = 72;      // % of 228 KB: 164 KB of shared memory for 5 CTAs, the rest is L1 (kernels_huff.cuh: kSyncCtas)
+constexpr int kSyncCarveout128 = 72;   // the same 164 KB for 6 CTAs of the 128-wide instance
 
 inline int batch_kernels_init(Device *dev) {
     if (dev->check(cudaFuncSetAttribute(k_huff_write, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffWriteMax)) != BJ_OK) return BJ_ERR_CUDA;
-    if (dev->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
-    if (dev->check(cudaFuncSetAttribute(k_huff_sync, cudaFuncAttributePreferredSharedMemoryCarveout, kSyncCarveout)) != BJ_OK) return BJ_ERR_CUDA;
+    if (dev->check(cudaFuncSetAttribute(k_huff_sync<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
+    if (dev->check(cudaFuncSetAttribute(k_huff_sync<256>, cudaFuncAttributePreferredSharedMemoryCarveout, kSyncCarveout)) != BJ_OK) return BJ_ERR_CUDA;
+    if (dev->check(cudaFuncSetAttribute(k_huff_sync<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHuffSyncMax)) != BJ_OK) return BJ_ERR_CUDA;
+    if (dev->check(cudaFuncSetAttribute(k_huff_sync<128>, cudaFuncAttributePreferredSharedMemoryCarveout, kSyncCarveout128)) != BJ_OK) return BJ_ERR_CUDA;
     return BJ_OK;
 }
 
@@ -72,6 +75,7 @@ struct bj_batch {
     size_t m_tiles = 0, m_blk = 0, m_wblk = 0, m_utile = 0, m_dcc = 0, maps_bytes = 0;
     uint32_t idct_smem = 0;             // dynamic shared memory of k_idct_color: sized for the widest pixel tile of this batch
     uint32_t n_wblk = 0;                // CTAs of the Huffman write pass
+    uint32_t sync_nt = 256;             // CTA width of the Huffman synchronisation pass (sub-sequences per CTA): 128 or 256
     size_t n_slice_slots = 0;
     uint32_t n_idct_tiles = 0, n_blk = 0, n_utile = 0, n_dcc = 0, n_seg_entries = 0, n_sub_slots = 0, lut_smem = 0;
     size_t clean_words = 0, coef_units = 0, out_bytes = 0;
@@ -192,9 +196,15 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     // synchronises within about a thousand, so nearly every guess settles inside its own sub-sequence - but shorter
     // when the whole batch would not fill the GPU with threads, and then adjusted per image so that its sub-sequences
     // fill whole CTAs (a nearly empty second CTA costs a cross-CTA fix-up round); the write pass works on whole
-    // sub-sequences (1 slice).  An image with restart markers gets sub-sequences that hold a typical restart segment
+    // sub-sequences (1 slice; 2 behind a 128-wide CTA, below).  An image with restart markers gets sub-sequences that hold a typical restart segment
     // in one piece - segment heads need no speculation at all - and the write pass cuts them into 4 slices (8 when
     // the batch is small), whose entry states the synchronisation pass records.
+    // The CTA width of the synchronisation pass (sub-sequences per CTA) is chosen once per batch.  An image gets at least
+    // one CTA, so an image that a 256-wide CTA of nominal sub-sequences does not fill gets sub-sequences shorter than
+    // nominal (config 2, 75 KB of scan per image: 292 bytes).  Where most of the batch's scan bytes are in such images,
+    // the CTAs are 128 wide and an image gets as many of them as it fills with nominal sub-sequences, at least one:
+    // config 2 gets 128 sub-sequences of 588 bytes, well above the synchronisation distance.  The write pass keeps its
+    // work per thread: behind a 128-wide CTA every sub-sequence is cut into at least 2 slices.
     const uint32_t fixed_sub = c->subseq_bits ? (uint32_t)c->subseq_bits / 8u : 0u;
     uint32_t fixed_rl = c->slices == 2 ? 1u : c->slices == 4 ? 2u : c->slices == 8 ? 3u : 0u;
     if (fixed_sub) while (fixed_rl && fixed_sub % (1u << fixed_rl)) fixed_rl--;
@@ -203,9 +213,19 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     uint64_t total_scan = 0;
     for (int i = 0; i < n; i++) if (b->parse_status[i] == BJ_OK) total_scan += b->desc[i].scan_len;
     if (!fixed_sub) nominal_sub = (uint32_t)std::min<uint64_t>(512u, std::max<uint64_t>(kMinSubBytes, total_scan / ((uint64_t)dev->sm_count * 3072u)));
+    uint32_t nt = c->sync_threads ? (uint32_t)c->sync_threads : 256u;
+    if (!c->sync_threads && !fixed_sub) {
+        uint64_t small_scan = 0;                        // scan bytes in images that do not fill a 256-wide CTA of nominal sub-sequences
+        for (int i = 0; i < n; i++)
+            if (b->parse_status[i] == BJ_OK && b->desc[i].scan_len < (uint64_t)256u * nominal_sub) small_scan += b->desc[i].scan_len;
+        if (2 * small_scan >= total_scan && total_scan > 0) nt = 128u;
+    }
+    const uint32_t nt_log2 = nt == 128u ? 7u : 8u;
+    b->sync_nt = nt;
     auto round_sub = [&](uint32_t len, uint32_t rl) { const uint32_t q = 4u << rl; return (std::max(len, 64u) + q - 1u) / q * q; };
     auto sub_layout_of = [&](uint32_t raw_len, uint32_t nseg, uint32_t *rl) -> uint32_t {
         *rl = c->slices ? fixed_rl : 0u;
+        if (nt == 128u && *rl == 0u) *rl = 1u;
         if (fixed_sub) return fixed_sub;
         if (nseg > 1) {
             const uint32_t avg = raw_len / nseg;
@@ -214,9 +234,9 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
                 return round_sub(std::max(2 * avg, nominal_sub), *rl);
             }
         }
-        const uint32_t per_cta = nominal_sub * kHuffThreads;
-        const uint32_t m = std::max(1u, (raw_len + per_cta / 2) / per_cta);                  // CTAs for this image
-        const uint32_t slots = m * kHuffThreads;                                            // ceil(raw_len / len) + nseg must fit
+        const uint32_t per_cta = nominal_sub * nt;
+        const uint32_t m = std::max(1u, (raw_len + (nt == 128u ? 0u : per_cta / 2)) / per_cta);   // CTAs for this image
+        const uint32_t slots = m * nt;                                                      // ceil(raw_len / len) + nseg must fit
         if (slots <= nseg + 1) return round_sub(nominal_sub, *rl);
         return round_sub((raw_len + slots - nseg - 1) / (slots - nseg), *rl);
     };
@@ -304,7 +324,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         b->file_off[i] = b->direct_src ? (uint64_t)(uintptr_t)files[i] - span_lo : fbytes;
         hi.seg_base = seg_entries;
         hi.blk_base = nblk;
-        hi.sub_base = nblk * kHuffThreads;
+        hi.sub_base = nblk * nt;
         hi.tile_base = n_utile;
         hi.clean_word0 = (uint32_t)clean_words;
         hi.du_base = (uint32_t)coef_units;
@@ -328,13 +348,14 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
             hi.slices_log2 = (uint8_t)rl;
         }
         const uint32_t sub_cap = (uint32_t)((hi.raw_len + hi.sub_bytes - 1) / hi.sub_bytes) + hi.nseg;
-        hi.nblk = (sub_cap + kHuffThreads - 1) / kHuffThreads;
+        hi.nblk = (sub_cap + nt - 1) / nt;
         nblk += hi.nblk;
         if (hi.nblk > 1) b->multi_blk = true;
+        hi.wblk_log2 = (uint8_t)(nt_log2 + hi.slices_log2 - 8u);
         hi.wblk_base = n_wblk;
-        n_wblk += hi.nblk << hi.slices_log2;
+        n_wblk += hi.nblk << hi.wblk_log2;
         hi.slice_base = (uint32_t)slice_slots;
-        slice_slots += ((size_t)hi.nblk * kHuffThreads) << hi.slices_log2;
+        slice_slots += ((size_t)hi.nblk * nt) << hi.slices_log2;
         hi.ndcc = (g.nmcu + kDcThreads - 1) / kDcThreads;
         n_dcc += hi.ndcc;
         seg_entries += hi.nseg + 1;
@@ -361,7 +382,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     b->files_bytes = b->direct_src ? (size_t)(span_hi - span_lo) : fbytes + 64; b->clean_words = clean_words + 96; b->coef_units = coef_units; b->out_bytes = out_bytes;   // (96 words of slack: a damaged unit is read to its end, up to 63 symbols of 27 bits past the data)
     b->n_wblk = n_wblk; b->n_slice_slots = slice_slots;
     b->n_idct_tiles = n_tiles; b->n_blk = nblk; b->n_utile = n_utile;
-    b->n_dcc = n_dcc; b->n_seg_entries = seg_entries; b->n_sub_slots = nblk * kHuffThreads;
+    b->n_dcc = n_dcc; b->n_seg_entries = seg_entries; b->n_sub_slots = nblk * nt;
 
     // ---- descriptor blob (host -> device): one record per image, the table pools
     size_t o = 0;
@@ -482,7 +503,10 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
     }
     if (b->n_blk) {
         for (int r = r0; r < r1; r++) {
-            k_huff_sync<<<b->n_blk, kHuffThreads, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, (uint4 *)b->d_quarter.p, agg, flags, r);
+            if (b->sync_nt == 128)
+                k_huff_sync<128><<<b->n_blk, 128, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, (uint4 *)b->d_quarter.p, agg, flags, r);
+            else
+                k_huff_sync<256><<<b->n_blk, 256, lut_smem, s>>>(himg, st, blk_img, clean, seg_off, seg_sub0, sub_seg, luts_dc, luts_acs, st_in, st_out, tot, pre, slices, (uint4 *)b->d_quarter.p, agg, flags, r);
             b->launches++; b->sync_rounds++;
         }
         cudaEventRecord(b->ev[2], s);

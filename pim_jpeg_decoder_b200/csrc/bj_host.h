@@ -152,6 +152,7 @@ struct Device;
 struct bj_ctx {
     int subseq_bits = 0;                 // sub-sequence length of the synchronisation pass; 0 = automatic (per image)
     int slices = 0;                      // slices (write pass) per sub-sequence: 1, 2, 4, 8; 0 = default (1)
+    int sync_threads = 0;                // CTA width of the synchronisation pass: 128, 256; 0 = automatic (per batch)
     size_t sub_batch_bytes = 0;          // 0 = default
     int sub_batch_ramp = 1;              // the first two sub-batches of a call are smaller (the copy-out starts earlier)
     int packed_outputs = 0;              // see batch_download_async

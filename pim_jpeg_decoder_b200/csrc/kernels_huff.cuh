@@ -39,8 +39,8 @@ struct HuffImg {
     uint32_t tile_base, ntile;
     uint32_t seg_base;       // index into seg_off / seg_sub0 (nseg + 1 entries each)
     uint32_t nseg;           // segments expected from the header: ceil(nmcu / RI), 1 without DRI
-    uint32_t sub_base;       // first sub-sequence slot (multiple of kHuffThreads)
-    uint32_t blk_base, nblk; // CTAs of k_huff_sync / k_huff_write
+    uint32_t sub_base;       // first sub-sequence slot (multiple of the CTA width of k_huff_sync)
+    uint32_t blk_base, nblk; // CTAs of k_huff_sync
     uint32_t du_base, ndu;
     uint32_t nmcu, ri;       // ri = restart interval in MCUs (0: none)
     uint32_t dcc_base, ndcc; // CTAs of the DC prediction kernels (kDcThreads MCUs each)
@@ -50,10 +50,11 @@ struct HuffImg {
     uint8_t dc_slot[3], ac_slot[3];  // per component: staged slot
     uint8_t slices_log2;     // the write pass works on 2^slices_log2 slices of every sub-sequence
     uint8_t flags;           // kImgClean / kImgExact (input handed over as a scan, not as a file: bj_decode_batch_desc)
+    uint8_t wblk_log2;       // CTAs of k_huff_write per CTA of k_huff_sync: (width << slices_log2) / kHuffThreads = 2^wblk_log2
     uint16_t dc_n4[3], ac_n4[3];     // used size of each staged table in 16-byte chunks (tables are staged packed)
     uint32_t sub_bytes;      // length of this image's sub-sequences (synchronisation pass), a multiple of the slice count
-    uint32_t wblk_base;      // first CTA of k_huff_write (nblk << slices_log2 of them)
-    uint32_t slice_base;     // first slot of this image in the slice table ((nblk * kHuffThreads) << slices_log2 slots)
+    uint32_t wblk_base;      // first CTA of k_huff_write (nblk << wblk_log2 of them)
+    uint32_t slice_base;     // first slot of this image in the slice table ((nblk * width) << slices_log2 slots)
 };
 
 // Per image, written by the kernels.
@@ -338,7 +339,7 @@ k_expand_maps(const HuffImg *__restrict__ imgs, const ImgDev *__restrict__ idev,
     if (!im.valid) return;
     for (uint32_t k = threadIdx.x; k < im.ntile; k += blockDim.x) tile_img[im.tile_base + k] = img;
     for (uint32_t k = threadIdx.x; k < im.nblk; k += blockDim.x) blk_img[im.blk_base + k] = img;
-    for (uint32_t k = threadIdx.x; k < (im.nblk << im.slices_log2); k += blockDim.x) wblk_img[im.wblk_base + k] = img;
+    for (uint32_t k = threadIdx.x; k < (im.nblk << im.wblk_log2); k += blockDim.x) wblk_img[im.wblk_base + k] = img;
     for (uint32_t k = threadIdx.x; k < im.ndcc; k += blockDim.x) dcc_img[im.dcc_base + k] = img;
     const ImgDev &id = idev[img];
     const uint32_t tile_mcus = kTileThreads / id.bpm, per_row = (id.nmx + tile_mcus - 1) / tile_mcus;
@@ -494,8 +495,12 @@ struct NoRec {
 // the L1 has to hold about one line per resident thread or the lines are evicted before their 32 words are used:
 // 5 CTAs with the shared-memory carve-out limited to 164 KB (92 KB of L1, batch.h) beat 6 CTAs with 56 KB of L1 by
 // a quarter (measured: 6: 2.09 ms, 5: 1.53 ms, 4: 2.16 ms, 3: 2.44 ms on config 2).
+// The 128-wide instance (batch.h picks the width per batch) is compiled for twice as many CTAs, so it keeps the 48
+// registers per thread; it runs 6 per SM with the same 164 KB carve-out (config 2: 5 CTAs 1.47 ms, 6 1.29 ms, 8 1.47 ms,
+// 9 1.47 ms; profiles/r3_sync_width/carveout_sweep.txt).
 constexpr int kSyncCtas = 5;
-__global__ void __launch_bounds__(kHuffThreads, kSyncCtas)
+template <int NT>
+__global__ void __launch_bounds__(NT, kSyncCtas * kHuffThreads / NT)
 k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ ist, const uint32_t *__restrict__ blk_img,
             const uint32_t *__restrict__ clean, const uint32_t *__restrict__ seg_off, const uint32_t *__restrict__ seg_sub0,
             const uint32_t *__restrict__ sub_seg, const uint32_t *__restrict__ lut_dc_pool, const uint32_t *__restrict__ lut_ac_pool,
@@ -503,26 +508,26 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
             uint4 *__restrict__ slices, uint4 *__restrict__ quarters, BlkAgg *__restrict__ blk_agg, uint32_t *__restrict__ flags, int round) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     uint32_t *s_lut = reinterpret_cast<uint32_t *>(smem_raw);
-    __shared__ uint2 s_in[kHuffThreads], s_out[kHuffThreads];
-    __shared__ uint32_t s_tot[kHuffThreads];
-    __shared__ uint2 s_span[kHuffThreads];                                  // first bit, end bit
+    __shared__ uint2 s_in[NT], s_out[NT];
+    __shared__ uint32_t s_tot[NT];
+    __shared__ uint2 s_span[NT];                                            // first bit, end bit
     __shared__ __align__(256) uint4 s_units[16];
-    __shared__ uint16_t s_work[2][kHuffThreads];
+    __shared__ uint16_t s_work[2][NT];
     __shared__ uint32_t s_nwork[2];
     __shared__ uint32_t s_flag;
-    __shared__ uint2 s_cur[kHuffThreads];                                   // state at the end of the last quarter done
-    __shared__ uint16_t s_plist[2][kHuffThreads];                           // sub-sequences still running in this iteration
+    __shared__ uint2 s_cur[NT];                                             // state at the end of the last quarter done
+    __shared__ uint16_t s_plist[2][NT];                                     // sub-sequences still running in this iteration
     __shared__ uint32_t s_pn[2];
-    __shared__ uint32_t s_w[kHuffThreads / 32 + 1];
-    __shared__ uint32_t s_wf[kHuffThreads / 32 + 1];
+    __shared__ uint32_t s_w[NT / 32 + 1];
+    __shared__ uint32_t s_wf[NT / 32 + 1];
 
     const uint32_t img = blk_img[blockIdx.x];
     const HuffImg &im = imgs[img];
     const HuffImgState is = ist[img];
     const int tid = threadIdx.x;
-    const uint32_t j = (blockIdx.x - im.blk_base) * kHuffThreads + tid;    // image-local sub-sequence
+    const uint32_t j = (blockIdx.x - im.blk_base) * NT + tid;              // image-local sub-sequence
     const uint32_t gj = im.sub_base + j;
-    const uint32_t first_j = (blockIdx.x - im.blk_base) * kHuffThreads;
+    const uint32_t first_j = (blockIdx.x - im.blk_base) * NT;
     if (first_j >= is.nsub) return;                                        // whole CTA beyond the image's sub-sequences
     const bool active = j < is.nsub;
 
@@ -565,14 +570,14 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
         const uint32_t nw = s_nwork[cur];
         if (nw == 0) break;
         const bool has_prev = round > 0 || iter > 0;                        // every sub-sequence on the list has been decoded before
-        for (uint32_t w = tid; w < nw; w += kHuffThreads) s_plist[0][w] = s_work[cur][w];
+        for (uint32_t w = tid; w < nw; w += NT) s_plist[0][w] = s_work[cur][w];
         if (tid == 0) { s_pn[0] = nw; s_pn[1] = 0; }
         int pc = 0;
         for (uint32_t q = 0; q < (1u << ql2); q++) {
             __syncthreads();
             const uint32_t pn = s_pn[pc];
             if (pn == 0) break;
-            for (uint32_t w = tid; w < pn; w += kHuffThreads) {
+            for (uint32_t w = tid; w < pn; w += NT) {
                 const uint32_t item = s_plist[pc][w];
                 const uint2 span = s_span[item];
                 const uint32_t qs = span.x + q * qbits, qe = min(qs + qbits, span.y);
@@ -624,9 +629,9 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
     }
     if (lane == 31) { s_w[warp] = v0; s_wf[warp] = f; }
     __syncthreads();
-    if (tid == 0) {                                                        // 8 warp totals: serial segmented scan
+    if (tid == 0) {                                                        // NT / 32 warp totals: serial segmented scan
         uint32_t c0 = 0, cf = 0;
-        for (int w = 0; w < kHuffThreads / 32; w++) {
+        for (int w = 0; w < NT / 32; w++) {
             const uint32_t a0 = s_w[w], af = s_wf[w];
             s_w[w] = c0; s_wf[w] = cf;                                     // carry INTO warp w
             if (af) { c0 = a0; cf = 1; } else c0 += a0;
@@ -661,8 +666,8 @@ k_huff_sync(const HuffImg *__restrict__ imgs, const HuffImgState *__restrict__ i
 }
 
 // ------------------------------------------------------------------------------------------------ K1a: write
-// One thread = one slice; a CTA's 256 slices are consecutive (kHuffThreads >> slices_log2 sub-sequences of one CTA
-// of the synchronisation pass).  A warp works in rounds: every lane takes up to kWriteSteps symbols
+// One thread = one slice; a CTA's 256 slices are consecutive (kHuffThreads >> slices_log2 sub-sequences, all of one CTA
+// of the synchronisation pass, which is covered by 2^wblk_log2 CTAs).  A warp works in rounds: every lane takes up to kWriteSteps symbols
 // (WriteCursor::step_plain: no checks, no hand-over - the lanes stay together) and stops at the one that completes its
 // unit; then the lanes that completed a unit look back over it and hand over to their next unit together
 // (WriteCursor::unit_end), and the warp stores those units together.  With the hand-over inside every step (one or two
@@ -707,11 +712,11 @@ k_huff_write(const HuffImg *__restrict__ imgs, HuffImgState *__restrict__ ist, c
     const uint32_t slices_log2 = im.slices_log2;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t lw = blockIdx.x - im.wblk_base;                         // this image's write CTA
-    const uint32_t lb = lw >> slices_log2;                                 // ... which covers part of this CTA of the synchronisation pass
-    const uint32_t slot = (lw & ((1u << slices_log2) - 1u)) * kHuffThreads + tid;   // slice slot within that CTA
-    const uint32_t j = lb * kHuffThreads + (slot >> slices_log2);          // image-local sub-sequence
+    const uint32_t lb = lw >> im.wblk_log2;                                // ... which covers part of this CTA of the synchronisation pass
+    const uint32_t slot = lw * kHuffThreads + tid;                         // image-local slice slot
+    const uint32_t j = slot >> slices_log2;                                // image-local sub-sequence
     const uint32_t k = slot & ((1u << slices_log2) - 1u);                  // slice of it
-    if (lb * kHuffThreads + ((slot - tid) >> slices_log2) >= is.nsub) return;   // whole CTA beyond the image's sub-sequences
+    if (((slot - tid) >> slices_log2) >= is.nsub) return;                  // whole CTA beyond the image's sub-sequences
     bool active = j < is.nsub;
 
     // carry into this CTA: totals of the previous CTAs of the image back to the last one that contains a head
