@@ -133,6 +133,27 @@ size_t bj_ref_mcus_size(const bj_image_desc *desc, int max_mcu_per_dpu, int *nch
 int bj_decode_batch(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, int n, int format,
                     uint8_t *const *outs, int *status);
 
+/* REGION OF INTEREST.  A rectangle of the decoded image in pixels, top-left origin; {0,0,0,0} = the whole image.
+ * The output of an image with a ROI is what the same format holds for an image of w x h whose pixels are the full
+ * decode's pixels [y, y+h) x [x, x+w):
+ *   BJ_OUT_RGB8  w*h*3 bytes, top-down
+ *   BJ_OUT_BMP   the bytes write_BMP writes for a w x h image: 26-byte header with w and h, bottom-up B,G,R rows,
+ *                w%4 zero bytes after every row
+ * The parity rules of the whole image carry over: a damaged scan gives the crop of the partial image, a subsampled
+ * image with restart markers the crop of its restart-free twin.  A ROI does not fit when w or h is 0 (other than
+ * {0,0,0,0}) or when x + w > width or y + h > height; such an image gets a per-image BJ_ERR_ARG and the rest of the
+ * batch decodes.  The whole scan is still entropy-decoded (DC prediction chains through every unit before the crop), so
+ * "max_image_pixels" applies to the full image; only the MCUs that hold crop pixels go through the IDCT + colour stage,
+ * and only the crop's bytes are copied out.  BJ_OUT_REF_MCUS has no crop: the _roi entries refuse it (BJ_ERR_ARG) when
+ * rois != NULL.  rois == NULL: whole images, the call is exactly the entry without _roi. */
+typedef struct { uint32_t x, y, w, h; } bj_roi;
+/* Output bytes of an image with this ROI (roi == NULL: the whole image); 0 if the ROI does not fit, and for
+ * BJ_OUT_REF_MCUS. */
+size_t bj_roi_output_size(const bj_image_desc *desc, const bj_roi *roi, int format);
+/* bj_decode_batch with rois[i] for image i; outs[i] holds bj_roi_output_size() bytes. */
+int bj_decode_batch_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n,
+                        int format, uint8_t *const *outs, int *status);
+
 /* FULL PATH behind the UNCHANGED scanner.  Replaces decode_Huffman_data(header, MCU_buffer, dpu_offset) + pim.copy /
  * pim.exec / pim.copy (src/decoder_host.cpp:181, :268-312) for a host that keeps read_JPEG in front: it fills one
  * bj_image_desc per `Header` (field for field, see INTEGRATION.md) and hands over the scan bytes -
@@ -155,12 +176,19 @@ int bj_decode_batch_desc(bj_ctx *ctx, const bj_image_desc *descs, const uint8_t 
 typedef struct bj_job bj_job;
 int bj_submit(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, int n, int format,
               uint8_t *const *outs, int *status, bj_job **job);
+/* bj_submit with a ROI per image (see bj_decode_batch_roi); rois, too, must stay valid until bj_wait returns. */
+int bj_submit_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
+                  uint8_t *const *outs, int *status, bj_job **job);
 int bj_wait(bj_job *job);
 
 /* FULL PATH, staged (device-resident batch) - what bj_decode_batch is made of, and what bench.py times with the
  * inputs already in HBM. */
 typedef struct bj_batch bj_batch;
 int bj_batch_create(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, int n, int format, bj_batch **out);
+/* bj_batch_create with a ROI per image (see bj_decode_batch_roi): output offsets and sizes, bj_batch_device_output and
+ * the out_bytes / d2h_bytes of bj_batch_info are those of the crops; bj_batch_info.pixels counts full images. */
+int bj_batch_create_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n,
+                        int format, bj_batch **out);
 int bj_batch_upload(bj_batch *b, void *stream);                 /* H2D: file bytes + descriptors          */
 int bj_batch_decode(bj_batch *b, void *stream);                 /* enqueue all kernels; input and output stay in HBM */
 int bj_batch_sync(bj_batch *b);                                 /* wait; settles the (rare) extra Huffman fix-up rounds */

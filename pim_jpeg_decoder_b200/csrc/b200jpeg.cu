@@ -278,6 +278,12 @@ extern "C" int bj_peek_header(const uint8_t *file, size_t len, bj_image_desc *de
 
 extern "C" size_t bj_output_size(const bj_image_desc *d, int format) { return d ? output_bytes(*d, format, 100) : 0; }
 
+extern "C" size_t bj_roi_output_size(const bj_image_desc *d, const bj_roi *roi, int format) {
+    bj_roi r{};
+    if (!d || (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP) || !roi_rect(*d, roi, &r)) return 0;
+    return output_bytes(*d, format, 100, &r);
+}
+
 extern "C" size_t bj_ref_mcus_size(const bj_image_desc *d, int max_mcu_per_dpu, int *nchunks) {
     if (!d || max_mcu_per_dpu < 4 || max_mcu_per_dpu % 4) return 0;
     if (nchunks) *nchunks = (int)ref_mcus_chunks(*d, max_mcu_per_dpu);
@@ -318,15 +324,20 @@ extern "C" int bj_stage_idct_color(bj_ctx *c, const bj_image_desc *desc, const i
 
 // ------------------------------------------------------------------------------------------------ full path, staged
 
-extern "C" int bj_batch_create(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format, bj_batch **out) {
+extern "C" int bj_batch_create_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format, bj_batch **out) {
     if (!c || !out || n < 0 || (n > 0 && (!files || !lens))) return BJ_ERR_ARG;
+    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     *out = nullptr;
     bj_batch *b = new (std::nothrow) bj_batch();
     if (!b) return BJ_ERR_NOMEM;
-    const int rc = batch_assign(b, c->devs[0], files, lens, n, format);     // a staged batch lives on one device
+    const int rc = batch_assign(b, c->devs[0], files, lens, n, format, ~(size_t)0, nullptr, nullptr, rois);     // a staged batch lives on one device
     if (rc != BJ_OK) { b->release(); delete b; return rc; }
     *out = b;
     return BJ_OK;
+}
+
+extern "C" int bj_batch_create(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format, bj_batch **out) {
+    return bj_batch_create_roi(c, files, lens, nullptr, n, format, out);
 }
 
 extern "C" void bj_batch_destroy(bj_batch *b) {
@@ -455,6 +466,7 @@ struct RangeSource {
 struct CallInput {                       // what a call decodes: files, or (bj_decode_batch_desc) descriptors + scans
     const uint8_t *const *files; const size_t *lens;
     const bj_image_desc *descs; const int *kinds;
+    const bj_roi *rois;                  // (the _roi entries) a crop per image; nullptr: whole images
 };
 
 // One device's share of a call: pull ranges from `src` until it runs dry.  st[ST_COUNT]: this device's counters.
@@ -509,7 +521,8 @@ static int decode_worker(Device *dev, RangeSource *src, const CallInput &in, int
             bj_batch *b = dev->slots[slot];
             cudaStream_t s = dev->streams[slot];
             const double t0 = wall_ms();
-            rc = batch_assign(b, dev, files + i0, lens + i0, r1 - i0, format, c->sub_batch_out_bytes, in.descs ? in.descs + i0 : nullptr, in.kinds ? in.kinds + i0 : nullptr);
+            rc = batch_assign(b, dev, files + i0, lens + i0, r1 - i0, format, c->sub_batch_out_bytes, in.descs ? in.descs + i0 : nullptr, in.kinds ? in.kinds + i0 : nullptr,
+                           in.rois ? in.rois + i0 : nullptr);
             const int m = rc == BJ_OK ? b->n : 0;
             st[ST_HOST_MS] += wall_ms() - t0;
             host_t[slot][0] = t0 - wall0; host_t[slot][1] = wall_ms() - wall0;
@@ -568,12 +581,18 @@ static int decode_batch_now(bj_ctx *c, const CallInput &in, int n, int format, u
     return BJ_OK;
 }
 
-extern "C" int bj_decode_batch(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format,
-                               uint8_t *const *outs, int *status) {
+extern "C" int bj_decode_batch_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
+                                   uint8_t *const *outs, int *status) {
     if (!c || n < 0 || (n > 0 && (!files || !lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
+    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;                         // the reference's tile buffers have no crop
     if (c->async && c->async->pending()) return BJ_ERR_ARG;                          // jobs of bj_submit are still running on this context
-    return decode_batch_now(c, CallInput{files, lens, nullptr, nullptr}, n, format, outs, status);
+    return decode_batch_now(c, CallInput{files, lens, nullptr, nullptr, rois}, n, format, outs, status);
+}
+
+extern "C" int bj_decode_batch(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format,
+                               uint8_t *const *outs, int *status) {
+    return bj_decode_batch_roi(c, files, lens, nullptr, n, format, outs, status);
 }
 
 // The same for a caller that already holds the parsed header (the reference's `Header`, src/headers/jpeg.h:146-179) and
@@ -584,7 +603,7 @@ extern "C" int bj_decode_batch_desc(bj_ctx *c, const bj_image_desc *descs, const
     if (!c || n < 0 || (n > 0 && (!descs || !scans || !scan_lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     if (c->async && c->async->pending()) return BJ_ERR_ARG;
-    return decode_batch_now(c, CallInput{scans, scan_lens, descs, scan_kinds}, n, format, outs, status);
+    return decode_batch_now(c, CallInput{scans, scan_lens, descs, scan_kinds, nullptr}, n, format, outs, status);
 }
 
 // ------------------------------------------------------------------------------------------------ full path, asynchronous
@@ -593,7 +612,7 @@ extern "C" int bj_decode_batch_desc(bj_ctx *c, const bj_image_desc *descs, const
 // the queue between them (src/decoder_host.cpp:25-38,364-365) a caller gets by submitting batch k+1 (or reading its
 // files) while batch k decodes, and writing batch k-1's outputs meanwhile (host/decoder_b200.cpp does exactly that).
 struct bj_job {
-    const uint8_t *const *files; const size_t *lens; int n, format; uint8_t *const *outs; int *status;
+    const uint8_t *const *files; const size_t *lens; const bj_roi *rois; int n, format; uint8_t *const *outs; int *status;
     int rc = BJ_OK;
     bool done = false;
     bj_ctx *ctx = nullptr;
@@ -608,7 +627,7 @@ void bj::AsyncWorker::run() {
             if (q.empty()) return;
             j = q.front();
         }
-        const int rc = decode_batch_now(j->ctx, CallInput{j->files, j->lens, nullptr, nullptr}, j->n, j->format, j->outs, j->status);
+        const int rc = decode_batch_now(j->ctx, CallInput{j->files, j->lens, nullptr, nullptr, j->rois}, j->n, j->format, j->outs, j->status);
         {
             std::lock_guard<std::mutex> l(m);
             q.pop_front();
@@ -618,11 +637,13 @@ void bj::AsyncWorker::run() {
     }
 }
 
-extern "C" int bj_submit(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format, uint8_t *const *outs, int *status, bj_job **job) {
+extern "C" int bj_submit_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
+                             uint8_t *const *outs, int *status, bj_job **job) {
     if (!c || !job || n < 0 || (n > 0 && (!files || !lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
+    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     *job = nullptr;
-    bj_job *j = new (std::nothrow) bj_job{files, lens, n, format, outs, status};
+    bj_job *j = new (std::nothrow) bj_job{files, lens, rois, n, format, outs, status};
     if (!j) return BJ_ERR_NOMEM;
     j->ctx = c;
     if (!c->async) {
@@ -634,6 +655,10 @@ extern "C" int bj_submit(bj_ctx *c, const uint8_t *const *files, const size_t *l
     c->async->cv.notify_one();
     *job = j;
     return BJ_OK;
+}
+
+extern "C" int bj_submit(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format, uint8_t *const *outs, int *status, bj_job **job) {
+    return bj_submit_roi(c, files, lens, nullptr, n, format, outs, status, job);
 }
 
 extern "C" int bj_wait(bj_job *j) {

@@ -123,9 +123,12 @@ constexpr int kMaxRounds = 64;
 //             then the scan itself - raw (stuffed, with RSTn; kinds[i] = BJ_SCAN_RAW) or the reference's
 //             Header::huffman_data (un-stuffed, markers removed; BJ_SCAN_UNSTUFFED, only without a restart interval:
 //             read_JPEG throws the RSTn positions away, SURVEY 0.8) - and nothing is parsed.
+//   rois      (the _roi entries) image i is output as the crop rois[i] (bj_roi, include/b200jpeg.h): a ROI that does not
+//             fit its image gives that image BJ_ERR_ARG; output sizes, offsets and out_cap count the cropped bytes.
 inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, const size_t *lens, int n, int format, size_t out_cap = ~(size_t)0,
-                        const bj_image_desc *descs = nullptr, const int *kinds = nullptr) {
+                        const bj_image_desc *descs = nullptr, const int *kinds = nullptr, const bj_roi *rois = nullptr) {
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
+    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;                        // the reference's tile buffers have no crop
     const bj_ctx *c = dev->ctx;
     b->dev = dev; b->n = n; b->format = format;
     b->uploaded = b->decoded = b->synced = false;
@@ -150,7 +153,9 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
             } else
                 rc = (files[i] && lens[i]) ? parse_header(files[i], lens[i], &d, /*walk_scan=*/false) : BJ_ERR_INVALID_JPEG;
             if (rc == BJ_OK && d.scan_len >= ((size_t)1 << 31)) rc = BJ_ERR_UNSUPPORTED;   // byte counts travel in 31 bits
-            if (rc == BJ_OK && (size_t)d.width * d.height > c->max_image_pixels) rc = BJ_ERR_UNSUPPORTED;
+            if (rc == BJ_OK && (size_t)d.width * d.height > c->max_image_pixels) rc = BJ_ERR_UNSUPPORTED;   // (the full image: its whole scan is decoded)
+            bj_roi r{};
+            if (rc == BJ_OK && rois && !roi_rect(d, &rois[i], &r)) rc = BJ_ERR_ARG;
             if (rc == BJ_OK) geo[i] = geometry_of(d);
             b->parse_status[i] = rc;
         }
@@ -160,7 +165,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         size_t acc = 0;
         int m = 0;
         while (m < n) {
-            const size_t sz = b->parse_status[m] == BJ_OK ? align_up(output_bytes(b->desc[m], format, c->ref_m), 16) : 0;
+            const size_t sz = b->parse_status[m] == BJ_OK ? align_up(output_bytes(b->desc[m], format, c->ref_m, rois ? &rois[m] : nullptr), 16) : 0;
             if (m > 0 && acc + sz > out_cap) break;
             acc += sz; m++;
         }
@@ -362,13 +367,14 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         clean_words += hi.raw_len / 4 + 4;
         b->du_base[i] = (uint32_t)coef_units; b->ndu[i] = g.ndu;
         coef_units += g.ndu;
-        b->out_size[i] = output_bytes(d, format, c->ref_m);
+        const bj_roi *roi = rois ? &rois[i] : nullptr;
+        b->out_size[i] = output_bytes(d, format, c->ref_m, roi);
         b->out_off[i] = out_bytes;
-        fill_imgdev(d, g, format, hi.du_base, out_bytes, &idev[i]);
+        fill_imgdev(d, g, format, hi.du_base, out_bytes, &idev[i], roi);
         if (format == BJ_OUT_REF_MCUS) { idev[i].ref_blocks = ref_mcus_chunks(d, c->ref_m) * (uint32_t)(c->ref_m / 4); b->ref_blocks_max = std::max(b->ref_blocks_max, idev[i].ref_blocks); }
         idev[i].dc_sep = 1;
         idev[i].tile0 = n_tiles;
-        n_tiles += idct_tile_count(g);
+        n_tiles += idct_tile_count(idev[i]);
         if (prev >= 0 && same_qtab(d, b->desc[prev])) idev[i].qslot = idev[prev].qslot;
         else { idev[i].qslot = (uint32_t)qtabs.size(); qtabs.emplace_back(); fill_qtab(d, &qtabs.back()); }
         prev = i;

@@ -15,10 +15,10 @@ struct ImgDev {
     uint32_t nmx, nmy;            // MCUs per row / per column
     uint32_t du_base;             // index of this image's first data unit in the coefficient buffer
     uint32_t out_pitch;           // bytes between consecutive output rows
-    uint64_t out_row0;            // byte offset (in the batch output buffer) of image row y = 0
-    int32_t  row_dir;             // +1: row y at out_row0 + y*pitch (RGB8); -1: out_row0 - y*pitch (BMP, bottom-up)
-    uint32_t row_bytes;           // payload bytes per row (width*3)
-    uint32_t row_pad;             // zero bytes after the payload (BMP: width % 4)
+    uint64_t out_row0;            // byte offset (in the batch output buffer) of pixel (cx, cy), the crop's first
+    int32_t  row_dir;             // +1: image row y at out_row0 + (y - cy)*pitch (RGB8); -1: out_row0 - (y - cy)*pitch (BMP, bottom-up)
+    uint32_t row_bytes;           // payload bytes per row (cw*3)
+    uint32_t row_pad;             // zero bytes after the payload (BMP: cw % 4)
     uint8_t  hs, vs, ncomp, bpm;  // luma sampling, components, data units per MCU
     uint8_t  bgr;                 // 1: B,G,R byte order (BMP)
     uint8_t  valid;
@@ -27,7 +27,17 @@ struct ImgDev {
     uint32_t qslot;               // this image's quantiser set in the batch's pool of QTab (deduplicated across the batch)
     uint32_t tile0;               // index of this image's first K2/K3 tile in the batch's tile list
     uint32_t ref_blocks;          // BJ_OUT_REF_MCUS: 2x2-position blocks in this image's output (whole chunks of MAX_MCU_PER_DPU / 4)
+    uint32_t cx, cy, cw, ch;      // the pixels that are output (region of interest): [cx, cx + cw) x [cy, cy + ch); the whole image by default
+    uint16_t mx_lo, mx_hi;        // the MCU columns [mx_lo, mx_hi) and rows [my_lo, my_hi) that hold them (bj_host.h: set_crop).
+    uint16_t my_lo, my_hi;        // The K2/K3 tile list covers exactly these MCUs
 };
+
+// K2/K3 tiles per MCU row of the crop window: what the host sizes the tile list with and k_expand_maps fills it with
+__host__ __device__ inline uint32_t idct_tiles_per_row(const ImgDev &im) {
+    const uint32_t tile_mcus = kTileThreads / im.bpm;
+    return ((uint32_t)im.mx_hi - im.mx_lo + tile_mcus - 1) / tile_mcus;
+}
+__host__ __device__ inline uint32_t idct_tile_count(const ImgDev &im) { return ((uint32_t)im.my_hi - im.my_lo) * idct_tiles_per_row(im); }
 
 // One set of quantisation tables as the K2 kernel stages it: per component (quantiser << 16) in ZIG-ZAG (file) order.
 struct QTab {

@@ -210,27 +210,49 @@ inline Geometry geometry_of(const bj_image_desc &d) {
     return g;
 }
 
-// out_base: byte offset of this image's output inside the batch output buffer.
-inline void fill_imgdev(const bj_image_desc &d, const Geometry &g, int format, uint32_t du_base, uint64_t out_base, ImgDev *im) {
+// The rectangle a region of interest selects (bj_roi, include/b200jpeg.h): false if it does not fit the image.
+// roi == nullptr or {0,0,0,0}: the whole image.  The sums are taken in 64 bits: x + w must not wrap into range.
+inline bool roi_rect(const bj_image_desc &d, const bj_roi *roi, bj_roi *r) {
+    if (!roi || (roi->x == 0 && roi->y == 0 && roi->w == 0 && roi->h == 0)) { *r = bj_roi{0, 0, d.width, d.height}; return true; }
+    if (roi->w == 0 || roi->h == 0 || (uint64_t)roi->x + roi->w > d.width || (uint64_t)roi->y + roi->h > d.height) return false;
+    *r = *roi;
+    return true;
+}
+
+// The crop window of an image: its pixels and the MCUs that hold them (the only ones the K2/K3 tile list covers).
+inline void set_crop(const bj_roi &r, ImgDev *im) {
+    im->cx = r.x; im->cy = r.y; im->cw = r.w; im->ch = r.h;
+    const uint32_t mw = im->hs * 8u, mh = im->vs * 8u;
+    im->mx_lo = (uint16_t)(r.x / mw); im->mx_hi = (uint16_t)((r.x + r.w + mw - 1) / mw);
+    im->my_lo = (uint16_t)(r.y / mh); im->my_hi = (uint16_t)((r.y + r.h + mh - 1) / mh);
+}
+
+// out_base: byte offset of this image's output inside the batch output buffer.  roi: a rectangle roi_rect accepted
+// (nullptr: the whole image; BJ_OUT_REF_MCUS always takes the whole image).
+inline void fill_imgdev(const bj_image_desc &d, const Geometry &g, int format, uint32_t du_base, uint64_t out_base, ImgDev *im,
+                        const bj_roi *roi = nullptr) {
     memset(im, 0, sizeof(*im));
     im->width = d.width; im->height = d.height;
     im->nmx = g.nmx; im->nmy = g.nmy;
     im->du_base = du_base;
     im->hs = d.hs; im->vs = d.vs; im->ncomp = d.ncomp; im->bpm = (uint8_t)g.bpm;
-    im->row_bytes = d.width * 3;
     im->valid = 1;
+    bj_roi r{};
+    roi_rect(d, format == BJ_OUT_REF_MCUS ? nullptr : roi, &r);
+    set_crop(r, im);
+    im->row_bytes = r.w * 3;
     if (format == BJ_OUT_REF_MCUS) {
         im->row_pad = 0; im->out_pitch = 0; im->row_dir = 1; im->bgr = 0;
         im->out_row0 = out_base;                       // byte offset of the image's first chunk
     } else if (format == BJ_OUT_BMP) {
-        im->row_pad = d.width % 4;
-        im->out_pitch = d.width * 3 + im->row_pad;
-        im->out_row0 = out_base + 26 + (uint64_t)(d.height - 1) * im->out_pitch;
+        im->row_pad = r.w % 4;
+        im->out_pitch = r.w * 3 + im->row_pad;
+        im->out_row0 = out_base + 26 + (uint64_t)(r.h - 1) * im->out_pitch;
         im->row_dir = -1;
         im->bgr = 1;
     } else {
         im->row_pad = 0;
-        im->out_pitch = d.width * 3;
+        im->out_pitch = r.w * 3;
         im->out_row0 = out_base;
         im->row_dir = 1;
         im->bgr = 0;
@@ -273,15 +295,16 @@ inline uint32_t ref_mcus_chunks(const bj_image_desc &d, int M) {
     const uint32_t pw = (d.mcu_w_real + 1) / 2 * 2, ph = (d.mcu_h_real + 1) / 2 * 2;
     return (pw * ph + (uint32_t)M - 1) / (uint32_t)M;
 }
-inline size_t output_bytes(const bj_image_desc &d, int format, int M) {
-    const size_t w = d.width, h = d.height;
+// roi: as for fill_imgdev (BJ_OUT_REF_MCUS ignores it)
+inline size_t output_bytes(const bj_image_desc &d, int format, int M, const bj_roi *roi = nullptr) {
+    bj_roi r{};
+    roi_rect(d, roi, &r);
+    const size_t w = r.w, h = r.h;
     if (format == BJ_OUT_RGB8) return w * h * 3;
     if (format == BJ_OUT_BMP) return 26 + h * (w * 3 + w % 4);
     if (format == BJ_OUT_REF_MCUS) return (size_t)ref_mcus_chunks(d, M) * 64 * (size_t)M * 3 * sizeof(int16_t);
     return 0;
 }
-
-inline uint32_t idct_tile_count(const Geometry &g) { return g.nmy * ((g.nmx + g.tile_mcus - 1) / g.tile_mcus); }
 
 inline void append_tiles(const Geometry &g, uint32_t img, uint32_t du_base, std::vector<TileDev> *tiles) {
     for (uint32_t my = 0; my < g.nmy; my++)

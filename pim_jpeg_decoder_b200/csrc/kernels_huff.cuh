@@ -341,13 +341,15 @@ k_expand_maps(const HuffImg *__restrict__ imgs, const ImgDev *__restrict__ idev,
     for (uint32_t k = threadIdx.x; k < im.nblk; k += blockDim.x) blk_img[im.blk_base + k] = img;
     for (uint32_t k = threadIdx.x; k < (im.nblk << im.wblk_log2); k += blockDim.x) wblk_img[im.wblk_base + k] = img;
     for (uint32_t k = threadIdx.x; k < im.ndcc; k += blockDim.x) dcc_img[im.dcc_base + k] = img;
+    // K2/K3 tiles: the MCUs of the image's crop window only (the whole image unless a region of interest was asked for),
+    // row by row in chunks of tile_mcus; the coefficients of MCUs outside the window are never read
     const ImgDev &id = idev[img];
-    const uint32_t tile_mcus = kTileThreads / id.bpm, per_row = (id.nmx + tile_mcus - 1) / tile_mcus;
-    for (uint32_t q = threadIdx.x; q < id.nmy * per_row; q += blockDim.x) {
-        const uint32_t my = q / per_row, mx = (q - my * per_row) * tile_mcus;
+    const uint32_t tile_mcus = kTileThreads / id.bpm, per_row = idct_tiles_per_row(id);
+    for (uint32_t q = threadIdx.x; q < idct_tile_count(id); q += blockDim.x) {
+        const uint32_t qy = q / per_row, my = id.my_lo + qy, mx = id.mx_lo + (q - qy * per_row) * tile_mcus;
         TileDev t;
         t.img = img; t.my = (uint16_t)my; t.mx0 = (uint16_t)mx;
-        t.nm = (uint16_t)min(tile_mcus, id.nmx - mx);
+        t.nm = (uint16_t)min(tile_mcus, (uint32_t)id.mx_hi - mx);
         t.ndu = (uint16_t)(t.nm * id.bpm);
         t.du0 = id.du_base + (my * id.nmx + mx) * id.bpm;
         tiles[id.tile0 + q] = t;

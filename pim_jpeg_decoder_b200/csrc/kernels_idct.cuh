@@ -209,19 +209,23 @@ __device__ __forceinline__ void tile_color_store(const uint4 *s_du, uint8_t *s_r
 
     // ---- stage 3: copy-out.  Each pixel row of the tile is a contiguous byte run in HBM with arbitrary
     // alignment; it is written as 16-byte-aligned 128-bit stores whose payload is funnel-shifted out of the
-    // staging tile; only the first/last chunk of a run (and BMP pad bytes) go bytewise.
+    // staging tile; only the first/last chunk of a run (and BMP pad bytes) go bytewise.  Only the image's crop window
+    // leaves (the whole image unless a region of interest was asked for): tile rows y0 + r in [cy, cy + ch), columns
+    // [xs, xe) = the tile's columns inside [cx, cx + cw); pixel (x, y) goes to row y - cy, column x - cx of the output.
     {
         const int x0 = t.mx0 * hs * 8, y0 = t.my * vs * 8;
-        const int wpx = min(nseg * 8, (int)im->width - x0);
-        const int rows_valid = min(rows, (int)im->height - y0);
-        const int payload = wpx * 3;
-        const int len = payload + ((x0 + nseg * 8 >= (int)im->width) ? (int)im->row_pad : 0);
+        const int cx = (int)im->cx, cy = (int)im->cy, cx_end = cx + (int)im->cw;
+        const int xs = max(x0, cx), xe = min(x0 + nseg * 8, cx_end);
+        const int r_lo = max(cy - y0, 0), r_hi = min(rows, cy + (int)im->ch - y0);
+        const int payload = (xe - xs) * 3;
+        const int len = payload + (xe == cx_end ? (int)im->row_pad : 0);   // BMP pad bytes follow the run at the crop's right edge
         const int warp = tid >> 5, lane = tid & 31;
         const long long row_step = (long long)im->row_dir * (long long)im->out_pitch;
-        const long long off0 = (long long)im->out_row0 + row_step * (long long)y0 + (long long)x0 * 3;
-        for (int r = warp; r < rows_valid; r += kTileThreads / 32) {
+        const long long off0 = (long long)im->out_row0 + row_step * (long long)(y0 - cy) + (long long)(xs - cx) * 3;
+        const uint8_t *sp0 = s_rgb + (xs - x0) * 3;                        // (any byte alignment: the funnel shift below takes it)
+        for (int r = r_lo + warp; r < r_hi; r += kTileThreads / 32) {
             uint8_t *g = out + (off0 + row_step * r);
-            const uint8_t *sp = s_rgb + r * pitch;
+            const uint8_t *sp = sp0 + r * pitch;
             // the run [0, len) = head bytes up to the first 16-byte boundary, nfull whole aligned chunks, ntail bytes
             const int head = min((int)((16u - ((unsigned)(uintptr_t)g & 15u)) & 15u), len);
             const int nfull = (len - head) >> 4;
@@ -263,10 +267,10 @@ __device__ __forceinline__ void tile_color_store(const uint4 *s_du, uint8_t *s_r
                 __stcs(gp + i, make_uint4(vv[0], vv[1], vv[2], vv[3]));
             }
         }
-        // BMP file header (src/bmp_writer.cpp:26-41), written by the tile that owns the image's first MCU:
+        // BMP file header (src/bmp_writer.cpp:26-41) of the cw x ch output, written by the tile that holds pixel (cx, cy):
         // 'B','M', size(4), 0(4), 0x1A(4), 12(4), width(2), height(2), 1(2), 24(2)
-        if (im->bgr && t.my == 0 && t.mx0 == 0 && tid < 26) {
-            const unsigned W = im->width, H = im->height;
+        if (im->bgr && t.my == im->my_lo && t.mx0 == im->mx_lo && tid < 26) {
+            const unsigned W = im->cw, H = im->ch;
             const unsigned size = 26u + H * W * 3u + im->row_pad * H;
             unsigned v = 0;
             if (tid == 0) v = 'B';
