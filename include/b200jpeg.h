@@ -154,6 +154,30 @@ size_t bj_roi_output_size(const bj_image_desc *desc, const bj_roi *roi, int form
 int bj_decode_batch_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n,
                         int format, uint8_t *const *outs, int *status);
 
+/* REDUCED-SIZE DECODE.  Image i is output at 1/s of its size, s = scales[i] in {1, 2, 4, 8}.  For an image of W x H the
+ * scaled image is W' x H', W' = ceil(W / s), H' = ceil(H / s); its pixel (X, Y) is, per channel, (sum + n / 2) / n in
+ * integers, where sum and n are the channel sum and the count of the full decode's pixels in
+ * [sX, min(sX + s, W)) x [sY, min(sY + s, H)): a box average, n = s*s inside the image and less on the right and bottom
+ * edges.  s = 1 is the full decode.  (Not libjpeg's scaled IDCT: a box average of the full decode is defined exactly
+ * from the full decode, so the output is bit-exact against it.)
+ * rois[i] is then a rectangle of the SCALED image ({0,0,0,0}: all of it); it fits when w, h > 0, x + w <= W' and
+ * y + h <= H'.  The output is that crop of the scaled image in the format's layout (BJ_OUT_BMP: header with the crop's w
+ * and h, w%4 pad bytes per row).  The parity rules carry over: a damaged scan gives the scaled crop of the partial image,
+ * a subsampled image with restart markers that of its restart-free twin, gray images average R = G = B.  An image whose
+ * scale is not 1, 2, 4 or 8, or whose ROI does not fit the scaled image, gets a per-image BJ_ERR_ARG and the rest of the
+ * batch decodes.  The whole scan is still decoded, so "max_image_pixels" and bj_batch_info.pixels count the full image;
+ * output sizes and offsets, out_bytes, d2h_bytes and the sub-batch cut ("sub_batch_out_bytes") count the scaled crop.
+ * BJ_OUT_REF_MCUS is refused (BJ_ERR_ARG) when scales != NULL.  scales == NULL (or all 1): exactly the _roi entry.
+ * Both arrays, when given, must stay valid until the call returns (bj_submit_scaled: until bj_wait returns). */
+/* Output bytes of an image at 1/scale with this ROI of the scaled image (roi == NULL: all of it); 0 if the scale is not
+ * 1, 2, 4 or 8 or the ROI does not fit, and for BJ_OUT_REF_MCUS.  bj_roi_output_size(d, roi, f) ==
+ * bj_scaled_output_size(d, roi, 1, f). */
+size_t bj_scaled_output_size(const bj_image_desc *desc, const bj_roi *roi, int scale, int format);
+/* bj_decode_batch_roi with scales[i] for image i (scales may be NULL, rois may be NULL); outs[i] holds
+ * bj_scaled_output_size() bytes. */
+int bj_decode_batch_scaled(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois,
+                           const uint8_t *scales, int n, int format, uint8_t *const *outs, int *status);
+
 /* FULL PATH behind the UNCHANGED scanner.  Replaces decode_Huffman_data(header, MCU_buffer, dpu_offset) + pim.copy /
  * pim.exec / pim.copy (src/decoder_host.cpp:181, :268-312) for a host that keeps read_JPEG in front: it fills one
  * bj_image_desc per `Header` (field for field, see INTEGRATION.md) and hands over the scan bytes -
@@ -179,6 +203,10 @@ int bj_submit(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, int 
 /* bj_submit with a ROI per image (see bj_decode_batch_roi); rois, too, must stay valid until bj_wait returns. */
 int bj_submit_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
                   uint8_t *const *outs, int *status, bj_job **job);
+/* bj_submit with a ROI and a scale per image (see bj_decode_batch_scaled); rois and scales, too, must stay valid until
+ * bj_wait returns. */
+int bj_submit_scaled(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
+                     int n, int format, uint8_t *const *outs, int *status, bj_job **job);
 int bj_wait(bj_job *job);
 
 /* FULL PATH, staged (device-resident batch) - what bj_decode_batch is made of, and what bench.py times with the
@@ -189,6 +217,10 @@ int bj_batch_create(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens
  * the out_bytes / d2h_bytes of bj_batch_info are those of the crops; bj_batch_info.pixels counts full images. */
 int bj_batch_create_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n,
                         int format, bj_batch **out);
+/* bj_batch_create with a ROI and a scale per image (see bj_decode_batch_scaled): offsets, sizes and the out_bytes /
+ * d2h_bytes of bj_batch_info are those of the scaled crops; bj_batch_info.pixels counts full images. */
+int bj_batch_create_scaled(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois,
+                           const uint8_t *scales, int n, int format, bj_batch **out);
 int bj_batch_upload(bj_batch *b, void *stream);                 /* H2D: file bytes + descriptors          */
 int bj_batch_decode(bj_batch *b, void *stream);                 /* enqueue all kernels; input and output stay in HBM */
 int bj_batch_sync(bj_batch *b);                                 /* wait; settles the (rare) extra Huffman fix-up rounds */

@@ -8,4 +8,4 @@ program, ``Decoder.decode`` = decode_Huffman_data + DPU program + BMP pixel gath
 from ._lib import (BJ_ERR_ARG, BJ_ERR_CORRUPT_SCAN, BJ_ERR_CUDA, BJ_ERR_INVALID_JPEG, BJ_ERR_UNSUPPORTED, BJ_OK, BJ_OUT_BMP,  # noqa: F401
                    BJ_OUT_REF_MCUS, BJ_OUT_RGB8, BJ_SCAN_RAW, BJ_SCAN_UNSTUFFED, BatchInfo, BjError, ImageDesc, Roi, lib)
 from .decoder import (Batch, Decoder, Job, PinnedBuffer, decode_files, lpt_shards, parse_header, roi_output_size,  # noqa: F401
-                      shard_by_size)
+                      scaled_output_size, shard_by_size)

@@ -80,15 +80,20 @@ SYMBOLS = {
     "bj_peek_header": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(ImageDesc)]),
     "bj_output_size": (C.c_size_t, [C.POINTER(ImageDesc), C.c_int]),
     "bj_roi_output_size": (C.c_size_t, [C.POINTER(ImageDesc), C.POINTER(Roi), C.c_int]),
+    "bj_scaled_output_size": (C.c_size_t, [C.POINTER(ImageDesc), C.POINTER(Roi), C.c_int, C.c_int]),
     "bj_ref_mcus_size": (C.c_size_t, [C.POINTER(ImageDesc), C.c_int, C.POINTER(C.c_int)]),
     "bj_decode_batch_desc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bj_decode_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bj_decode_batch_roi": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "bj_decode_batch_scaled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bj_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "bj_submit_roi": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "bj_submit_scaled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                   C.POINTER(C.c_void_p)]),
     "bj_wait": (C.c_int, [C.c_void_p]),
     "bj_batch_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "bj_batch_create_roi": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "bj_batch_create_scaled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "bj_batch_upload": (C.c_int, [C.c_void_p, C.c_void_p]),
     "bj_batch_decode": (C.c_int, [C.c_void_p, C.c_void_p]),
     "bj_batch_sync": (C.c_int, [C.c_void_p]),

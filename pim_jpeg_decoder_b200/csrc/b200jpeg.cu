@@ -57,8 +57,9 @@ static int open_device(Device *dev) {
     cudaDeviceProp prop;
     if (rc == BJ_OK) rc = dev->check(cudaGetDeviceProperties(&prop, dev->ordinal));
     if (rc == BJ_OK) dev->sm_count = prop.multiProcessorCount;
-    if (rc == BJ_OK) rc = dev->check(cudaFuncSetAttribute(k_idct_color<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctColor));
-    if (rc == BJ_OK) rc = dev->check(cudaFuncSetAttribute(k_idct_color<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctColor));
+    if (rc == BJ_OK) rc = dev->check(cudaFuncSetAttribute(k_idct_color<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctColor));
+    if (rc == BJ_OK) rc = dev->check(cudaFuncSetAttribute(k_idct_color<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctColor));
+    if (rc == BJ_OK) rc = dev->check(cudaFuncSetAttribute(k_idct_color<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemIdctColor));
     if (rc == BJ_OK) rc = batch_kernels_init(dev);
     for (int i = 0; i < kSlots && rc == BJ_OK; i++) rc = dev->check(cudaStreamCreateWithFlags(&dev->streams[i], cudaStreamNonBlocking));
     for (int i = 0; i < 2 && rc == BJ_OK; i++) rc = dev->check(cudaEventCreate(&dev->ev_exec[i]));
@@ -278,11 +279,13 @@ extern "C" int bj_peek_header(const uint8_t *file, size_t len, bj_image_desc *de
 
 extern "C" size_t bj_output_size(const bj_image_desc *d, int format) { return d ? output_bytes(*d, format, 100) : 0; }
 
-extern "C" size_t bj_roi_output_size(const bj_image_desc *d, const bj_roi *roi, int format) {
+extern "C" size_t bj_scaled_output_size(const bj_image_desc *d, const bj_roi *roi, int scale, int format) {
     bj_roi r{};
-    if (!d || (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP) || !roi_rect(*d, roi, &r)) return 0;
-    return output_bytes(*d, format, 100, &r);
+    if (!d || (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP) || scale <= 0 || !roi_rect(*d, roi, (uint32_t)scale, &r)) return 0;
+    return output_bytes(*d, format, 100, &r, (uint32_t)scale);
 }
+
+extern "C" size_t bj_roi_output_size(const bj_image_desc *d, const bj_roi *roi, int format) { return bj_scaled_output_size(d, roi, 1, format); }
 
 extern "C" size_t bj_ref_mcus_size(const bj_image_desc *d, int max_mcu_per_dpu, int *nchunks) {
     if (!d || max_mcu_per_dpu < 4 || max_mcu_per_dpu % 4) return 0;
@@ -313,7 +316,7 @@ extern "C" int bj_stage_idct_color(bj_ctx *c, const bj_image_desc *desc, const i
     if (rc == BJ_OK) rc = dev->check(cudaMemcpyAsync(dti.p, tiles.data(), tiles.size() * sizeof(TileDev), cudaMemcpyHostToDevice, s));
     if (rc == BJ_OK) {
         const uint8_t *base = (const uint8_t *)dim.p;
-        k_idct_color<false><<<(unsigned)tiles.size(), kTileThreads, kSmemIdctColor, s>>>((const int16_t *)dco.p, nullptr, (const ImgDev *)base, (const QTab *)(base + offsetof(StageRec, q)),
+        k_idct_color<false, false><<<(unsigned)tiles.size(), kTileThreads, kSmemIdctColor, s>>>((const int16_t *)dco.p, nullptr, (const ImgDev *)base, (const QTab *)(base + offsetof(StageRec, q)),
                                                                                  (const TileDev *)dti.p, (uint8_t *)dout.p);
         rc = dev->check(cudaGetLastError());
     }
@@ -324,16 +327,21 @@ extern "C" int bj_stage_idct_color(bj_ctx *c, const bj_image_desc *desc, const i
 
 // ------------------------------------------------------------------------------------------------ full path, staged
 
-extern "C" int bj_batch_create_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format, bj_batch **out) {
+extern "C" int bj_batch_create_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales, int n,
+                                      int format, bj_batch **out) {
     if (!c || !out || n < 0 || (n > 0 && (!files || !lens))) return BJ_ERR_ARG;
-    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
+    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     *out = nullptr;
     bj_batch *b = new (std::nothrow) bj_batch();
     if (!b) return BJ_ERR_NOMEM;
-    const int rc = batch_assign(b, c->devs[0], files, lens, n, format, ~(size_t)0, nullptr, nullptr, rois);     // a staged batch lives on one device
+    const int rc = batch_assign(b, c->devs[0], files, lens, n, format, ~(size_t)0, nullptr, nullptr, rois, scales);     // a staged batch lives on one device
     if (rc != BJ_OK) { b->release(); delete b; return rc; }
     *out = b;
     return BJ_OK;
+}
+
+extern "C" int bj_batch_create_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format, bj_batch **out) {
+    return bj_batch_create_scaled(c, files, lens, rois, nullptr, n, format, out);
 }
 
 extern "C" int bj_batch_create(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format, bj_batch **out) {
@@ -466,7 +474,8 @@ struct RangeSource {
 struct CallInput {                       // what a call decodes: files, or (bj_decode_batch_desc) descriptors + scans
     const uint8_t *const *files; const size_t *lens;
     const bj_image_desc *descs; const int *kinds;
-    const bj_roi *rois;                  // (the _roi entries) a crop per image; nullptr: whole images
+    const bj_roi *rois;                  // (the _roi / _scaled entries) a crop per image; nullptr: whole images
+    const uint8_t *scales;               // (the _scaled entries) a scale denominator per image; nullptr: all 1
 };
 
 // One device's share of a call: pull ranges from `src` until it runs dry.  st[ST_COUNT]: this device's counters.
@@ -522,7 +531,7 @@ static int decode_worker(Device *dev, RangeSource *src, const CallInput &in, int
             cudaStream_t s = dev->streams[slot];
             const double t0 = wall_ms();
             rc = batch_assign(b, dev, files + i0, lens + i0, r1 - i0, format, c->sub_batch_out_bytes, in.descs ? in.descs + i0 : nullptr, in.kinds ? in.kinds + i0 : nullptr,
-                           in.rois ? in.rois + i0 : nullptr);
+                           in.rois ? in.rois + i0 : nullptr, in.scales ? in.scales + i0 : nullptr);
             const int m = rc == BJ_OK ? b->n : 0;
             st[ST_HOST_MS] += wall_ms() - t0;
             host_t[slot][0] = t0 - wall0; host_t[slot][1] = wall_ms() - wall0;
@@ -581,13 +590,18 @@ static int decode_batch_now(bj_ctx *c, const CallInput &in, int n, int format, u
     return BJ_OK;
 }
 
-extern "C" int bj_decode_batch_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
-                                   uint8_t *const *outs, int *status) {
+extern "C" int bj_decode_batch_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
+                                      int n, int format, uint8_t *const *outs, int *status) {
     if (!c || n < 0 || (n > 0 && (!files || !lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
-    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;                         // the reference's tile buffers have no crop
+    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;            // the reference's tile buffers have no crop or scale
     if (c->async && c->async->pending()) return BJ_ERR_ARG;                          // jobs of bj_submit are still running on this context
-    return decode_batch_now(c, CallInput{files, lens, nullptr, nullptr, rois}, n, format, outs, status);
+    return decode_batch_now(c, CallInput{files, lens, nullptr, nullptr, rois, scales}, n, format, outs, status);
+}
+
+extern "C" int bj_decode_batch_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
+                                   uint8_t *const *outs, int *status) {
+    return bj_decode_batch_scaled(c, files, lens, rois, nullptr, n, format, outs, status);
 }
 
 extern "C" int bj_decode_batch(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format,
@@ -603,7 +617,7 @@ extern "C" int bj_decode_batch_desc(bj_ctx *c, const bj_image_desc *descs, const
     if (!c || n < 0 || (n > 0 && (!descs || !scans || !scan_lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     if (c->async && c->async->pending()) return BJ_ERR_ARG;
-    return decode_batch_now(c, CallInput{scans, scan_lens, descs, scan_kinds, nullptr}, n, format, outs, status);
+    return decode_batch_now(c, CallInput{scans, scan_lens, descs, scan_kinds, nullptr, nullptr}, n, format, outs, status);
 }
 
 // ------------------------------------------------------------------------------------------------ full path, asynchronous
@@ -612,7 +626,7 @@ extern "C" int bj_decode_batch_desc(bj_ctx *c, const bj_image_desc *descs, const
 // the queue between them (src/decoder_host.cpp:25-38,364-365) a caller gets by submitting batch k+1 (or reading its
 // files) while batch k decodes, and writing batch k-1's outputs meanwhile (host/decoder_b200.cpp does exactly that).
 struct bj_job {
-    const uint8_t *const *files; const size_t *lens; const bj_roi *rois; int n, format; uint8_t *const *outs; int *status;
+    const uint8_t *const *files; const size_t *lens; const bj_roi *rois; const uint8_t *scales; int n, format; uint8_t *const *outs; int *status;
     int rc = BJ_OK;
     bool done = false;
     bj_ctx *ctx = nullptr;
@@ -627,7 +641,7 @@ void bj::AsyncWorker::run() {
             if (q.empty()) return;
             j = q.front();
         }
-        const int rc = decode_batch_now(j->ctx, CallInput{j->files, j->lens, nullptr, nullptr, j->rois}, j->n, j->format, j->outs, j->status);
+        const int rc = decode_batch_now(j->ctx, CallInput{j->files, j->lens, nullptr, nullptr, j->rois, j->scales}, j->n, j->format, j->outs, j->status);
         {
             std::lock_guard<std::mutex> l(m);
             q.pop_front();
@@ -637,13 +651,13 @@ void bj::AsyncWorker::run() {
     }
 }
 
-extern "C" int bj_submit_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
-                             uint8_t *const *outs, int *status, bj_job **job) {
+extern "C" int bj_submit_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales, int n,
+                                int format, uint8_t *const *outs, int *status, bj_job **job) {
     if (!c || !job || n < 0 || (n > 0 && (!files || !lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
-    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
+    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     *job = nullptr;
-    bj_job *j = new (std::nothrow) bj_job{files, lens, rois, n, format, outs, status};
+    bj_job *j = new (std::nothrow) bj_job{files, lens, rois, scales, n, format, outs, status};
     if (!j) return BJ_ERR_NOMEM;
     j->ctx = c;
     if (!c->async) {
@@ -655,6 +669,11 @@ extern "C" int bj_submit_roi(bj_ctx *c, const uint8_t *const *files, const size_
     c->async->cv.notify_one();
     *job = j;
     return BJ_OK;
+}
+
+extern "C" int bj_submit_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
+                             uint8_t *const *outs, int *status, bj_job **job) {
+    return bj_submit_scaled(c, files, lens, rois, nullptr, n, format, outs, status, job);
 }
 
 extern "C" int bj_submit(bj_ctx *c, const uint8_t *const *files, const size_t *lens, int n, int format, uint8_t *const *outs, int *status, bj_job **job) {

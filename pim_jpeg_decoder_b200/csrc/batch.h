@@ -74,6 +74,7 @@ struct bj_batch {
     // offsets inside the map buffer (written on the device by k_expand_maps)
     size_t m_tiles = 0, m_blk = 0, m_wblk = 0, m_utile = 0, m_dcc = 0, maps_bytes = 0;
     uint32_t idct_smem = 0;             // dynamic shared memory of k_idct_color: sized for the widest pixel tile of this batch
+    bool scaled = false;                // some image is output at reduced size: the scaled instance of k_idct_color runs
     uint32_t n_wblk = 0;                // CTAs of the Huffman write pass
     uint32_t sync_nt = 256;             // CTA width of the Huffman synchronisation pass (sub-sequences per CTA): 128 or 256
     size_t n_slice_slots = 0;
@@ -123,12 +124,14 @@ constexpr int kMaxRounds = 64;
 //             then the scan itself - raw (stuffed, with RSTn; kinds[i] = BJ_SCAN_RAW) or the reference's
 //             Header::huffman_data (un-stuffed, markers removed; BJ_SCAN_UNSTUFFED, only without a restart interval:
 //             read_JPEG throws the RSTn positions away, SURVEY 0.8) - and nothing is parsed.
-//   rois      (the _roi entries) image i is output as the crop rois[i] (bj_roi, include/b200jpeg.h): a ROI that does not
-//             fit its image gives that image BJ_ERR_ARG; output sizes, offsets and out_cap count the cropped bytes.
+//   rois      (the _roi / _scaled entries) image i is output as the crop rois[i] (bj_roi, include/b200jpeg.h) of its image
+//   scales    scaled by 1 / scales[i] (the _scaled entries; 1, 2, 4 or 8): a scale other than those, or a ROI that does not
+//             fit the scaled image, gives that image BJ_ERR_ARG; output sizes, offsets and out_cap count the bytes of the
+//             scaled crop.
 inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, const size_t *lens, int n, int format, size_t out_cap = ~(size_t)0,
-                        const bj_image_desc *descs = nullptr, const int *kinds = nullptr, const bj_roi *rois = nullptr) {
+                        const bj_image_desc *descs = nullptr, const int *kinds = nullptr, const bj_roi *rois = nullptr, const uint8_t *scales = nullptr) {
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
-    if (rois && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;                        // the reference's tile buffers have no crop
+    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;            // the reference's tile buffers have no crop or scale
     const bj_ctx *c = dev->ctx;
     b->dev = dev; b->n = n; b->format = format;
     b->uploaded = b->decoded = b->synced = false;
@@ -155,7 +158,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
             if (rc == BJ_OK && d.scan_len >= ((size_t)1 << 31)) rc = BJ_ERR_UNSUPPORTED;   // byte counts travel in 31 bits
             if (rc == BJ_OK && (size_t)d.width * d.height > c->max_image_pixels) rc = BJ_ERR_UNSUPPORTED;   // (the full image: its whole scan is decoded)
             bj_roi r{};
-            if (rc == BJ_OK && rois && !roi_rect(d, &rois[i], &r)) rc = BJ_ERR_ARG;
+            if (rc == BJ_OK && (rois || scales) && !roi_rect(d, rois ? &rois[i] : nullptr, scales ? scales[i] : 1u, &r)) rc = BJ_ERR_ARG;
             if (rc == BJ_OK) geo[i] = geometry_of(d);
             b->parse_status[i] = rc;
         }
@@ -165,7 +168,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         size_t acc = 0;
         int m = 0;
         while (m < n) {
-            const size_t sz = b->parse_status[m] == BJ_OK ? align_up(output_bytes(b->desc[m], format, c->ref_m, rois ? &rois[m] : nullptr), 16) : 0;
+            const size_t sz = b->parse_status[m] == BJ_OK ? align_up(output_bytes(b->desc[m], format, c->ref_m, rois ? &rois[m] : nullptr, scales ? scales[m] : 1u), 16) : 0;
             if (m > 0 && acc + sz > out_cap) break;
             acc += sz; m++;
         }
@@ -257,7 +260,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     size_t fbytes = 0, clean_words = 0, out_bytes = 0, coef_units = 0;
     uint32_t seg_entries = 0, nblk = 0, n_utile = 0, n_wblk = 0, n_dcc = 0, n_tiles = 0;
     int prev = -1;                                  // last valid image: its table slots are reused when the tables match
-    b->pixels = 0; b->scan_bytes_max = 0; b->ref_blocks_max = 0; b->nseg_max = 0; b->lut_smem = 0; b->multi_blk = false;
+    b->pixels = 0; b->scan_bytes_max = 0; b->ref_blocks_max = 0; b->nseg_max = 0; b->lut_smem = 0; b->multi_blk = false; b->scaled = false;
     uint32_t rgb_max = 0;
     auto same_tables = [](const bj_image_desc &a, const bj_image_desc &q) {
         if (a.ncomp != q.ncomp || memcmp(a.dc_id, q.dc_id, 3) || memcmp(a.ac_id, q.ac_id, 3)) return false;
@@ -368,9 +371,11 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         b->du_base[i] = (uint32_t)coef_units; b->ndu[i] = g.ndu;
         coef_units += g.ndu;
         const bj_roi *roi = rois ? &rois[i] : nullptr;
-        b->out_size[i] = output_bytes(d, format, c->ref_m, roi);
+        const uint32_t scale = scales ? scales[i] : 1u;
+        b->out_size[i] = output_bytes(d, format, c->ref_m, roi, scale);
         b->out_off[i] = out_bytes;
-        fill_imgdev(d, g, format, hi.du_base, out_bytes, &idev[i], roi);
+        fill_imgdev(d, g, format, hi.du_base, out_bytes, &idev[i], roi, scale);
+        if (scale != 1) b->scaled = true;
         if (format == BJ_OUT_REF_MCUS) { idev[i].ref_blocks = ref_mcus_chunks(d, c->ref_m) * (uint32_t)(c->ref_m / 4); b->ref_blocks_max = std::max(b->ref_blocks_max, idev[i].ref_blocks); }
         idev[i].dc_sep = 1;
         idev[i].tile0 = n_tiles;
@@ -534,10 +539,13 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
     if (b->n_idct_tiles && b->format == BJ_OUT_REF_MCUS) {
         const unsigned gx = std::min<unsigned>(64u, (b->ref_blocks_max * 12u + 255u) / 256u);
         k_ref_mcus_pad<<<dim3(std::max(gx, 1u), n), 256, 0, s>>>(idev, (uint8_t *)b->d_out.p);
-        k_idct_color<true><<<b->n_idct_tiles, kTileThreads, b->idct_smem, s>>>((const int16_t *)b->d_coef.p, dcp, idev, qtabs, tiles, (uint8_t *)b->d_out.p);
+        k_idct_color<true, false><<<b->n_idct_tiles, kTileThreads, b->idct_smem, s>>>((const int16_t *)b->d_coef.p, dcp, idev, qtabs, tiles, (uint8_t *)b->d_out.p);
         b->launches += 2;
+    } else if (b->n_idct_tiles && b->scaled) {
+        k_idct_color<false, true><<<b->n_idct_tiles, kTileThreads, b->idct_smem, s>>>((const int16_t *)b->d_coef.p, dcp, idev, qtabs, tiles, (uint8_t *)b->d_out.p);
+        b->launches++;
     } else if (b->n_idct_tiles) {
-        k_idct_color<false><<<b->n_idct_tiles, kTileThreads, b->idct_smem, s>>>((const int16_t *)b->d_coef.p, dcp, idev, qtabs, tiles, (uint8_t *)b->d_out.p);
+        k_idct_color<false, false><<<b->n_idct_tiles, kTileThreads, b->idct_smem, s>>>((const int16_t *)b->d_coef.p, dcp, idev, qtabs, tiles, (uint8_t *)b->d_out.p);
         b->launches++;
     }
     cudaEventRecord(b->ev[4], s);

@@ -23,13 +23,14 @@ struct ImgDev {
     uint8_t  bgr;                 // 1: B,G,R byte order (BMP)
     uint8_t  valid;
     uint8_t  dc_sep;              // 1: slot 0 of every unit is unused, the DC value comes from the DC plane (informative: the kernel is told by its dc_plane argument)
-    uint8_t  pad_[1];
+    uint8_t  scale_log2;          // reduced-size output: each output pixel is the mean of a (1 << scale_log2)^2 box of the full decode
     uint32_t qslot;               // this image's quantiser set in the batch's pool of QTab (deduplicated across the batch)
     uint32_t tile0;               // index of this image's first K2/K3 tile in the batch's tile list
     uint32_t ref_blocks;          // BJ_OUT_REF_MCUS: 2x2-position blocks in this image's output (whole chunks of MAX_MCU_PER_DPU / 4)
-    uint32_t cx, cy, cw, ch;      // the pixels that are output (region of interest): [cx, cx + cw) x [cy, cy + ch); the whole image by default
-    uint16_t mx_lo, mx_hi;        // the MCU columns [mx_lo, mx_hi) and rows [my_lo, my_hi) that hold them (bj_host.h: set_crop).
-    uint16_t my_lo, my_hi;        // The K2/K3 tile list covers exactly these MCUs
+    uint32_t cx, cy, cw, ch;      // the pixels that are output (region of interest), in the coordinates of the scaled image:
+                                  // [cx, cx + cw) x [cy, cy + ch); the whole (scaled) image by default
+    uint16_t mx_lo, mx_hi;        // the MCU columns [mx_lo, mx_hi) and rows [my_lo, my_hi) that hold their full-size pixels
+    uint16_t my_lo, my_hi;        // (bj_host.h: set_crop).  The K2/K3 tile list covers exactly these MCUs
 };
 
 // K2/K3 tiles per MCU row of the crop window: what the host sizes the tile list with and k_expand_maps fills it with

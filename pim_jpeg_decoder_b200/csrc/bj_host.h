@@ -210,36 +210,48 @@ inline Geometry geometry_of(const bj_image_desc &d) {
     return g;
 }
 
-// The rectangle a region of interest selects (bj_roi, include/b200jpeg.h): false if it does not fit the image.
-// roi == nullptr or {0,0,0,0}: the whole image.  The sums are taken in 64 bits: x + w must not wrap into range.
-inline bool roi_rect(const bj_image_desc &d, const bj_roi *roi, bj_roi *r) {
-    if (!roi || (roi->x == 0 && roi->y == 0 && roi->w == 0 && roi->h == 0)) { *r = bj_roi{0, 0, d.width, d.height}; return true; }
-    if (roi->w == 0 || roi->h == 0 || (uint64_t)roi->x + roi->w > d.width || (uint64_t)roi->y + roi->h > d.height) return false;
+// Reduced-size output: log2 of a scale denominator 1, 2, 4 or 8; -1 for any other value.
+inline int scale_log2_of(uint32_t scale) { return scale == 1 ? 0 : scale == 2 ? 1 : scale == 4 ? 2 : scale == 8 ? 3 : -1; }
+
+// The rectangle a region of interest selects in the image scaled by 1 / scale (ceil(width / scale) x ceil(height / scale),
+// include/b200jpeg.h): false if the scale is not 1, 2, 4 or 8 or the ROI does not fit the scaled image.  roi == nullptr or
+// {0,0,0,0}: the whole scaled image.  The sums are taken in 64 bits: x + w must not wrap into range.
+inline bool roi_rect(const bj_image_desc &d, const bj_roi *roi, uint32_t scale, bj_roi *r) {
+    const int sl = scale_log2_of(scale);
+    if (sl < 0) return false;
+    const uint32_t W = (d.width + scale - 1) >> sl, H = (d.height + scale - 1) >> sl;
+    if (!roi || (roi->x == 0 && roi->y == 0 && roi->w == 0 && roi->h == 0)) { *r = bj_roi{0, 0, W, H}; return true; }
+    if (roi->w == 0 || roi->h == 0 || (uint64_t)roi->x + roi->w > W || (uint64_t)roi->y + roi->h > H) return false;
     *r = *roi;
     return true;
 }
 
-// The crop window of an image: its pixels and the MCUs that hold them (the only ones the K2/K3 tile list covers).
-inline void set_crop(const bj_roi &r, ImgDev *im) {
+// The crop window of an image: its pixels in the scaled image, and the MCUs that hold their full-size footprint
+// [s cx, min(s (cx + cw), width)) x [s cy, min(s (cy + ch), height)) (the only ones the K2/K3 tile list covers).
+inline void set_crop(const bj_roi &r, int scale_log2, ImgDev *im) {
     im->cx = r.x; im->cy = r.y; im->cw = r.w; im->ch = r.h;
+    im->scale_log2 = (uint8_t)scale_log2;
     const uint32_t mw = im->hs * 8u, mh = im->vs * 8u;
-    im->mx_lo = (uint16_t)(r.x / mw); im->mx_hi = (uint16_t)((r.x + r.w + mw - 1) / mw);
-    im->my_lo = (uint16_t)(r.y / mh); im->my_hi = (uint16_t)((r.y + r.h + mh - 1) / mh);
+    const uint32_t x_lo = r.x << scale_log2, x_hi = (uint32_t)std::min<uint64_t>((uint64_t)(r.x + r.w) << scale_log2, im->width);
+    const uint32_t y_lo = r.y << scale_log2, y_hi = (uint32_t)std::min<uint64_t>((uint64_t)(r.y + r.h) << scale_log2, im->height);
+    im->mx_lo = (uint16_t)(x_lo / mw); im->mx_hi = (uint16_t)((x_hi + mw - 1) / mw);
+    im->my_lo = (uint16_t)(y_lo / mh); im->my_hi = (uint16_t)((y_hi + mh - 1) / mh);
 }
 
-// out_base: byte offset of this image's output inside the batch output buffer.  roi: a rectangle roi_rect accepted
-// (nullptr: the whole image; BJ_OUT_REF_MCUS always takes the whole image).
+// out_base: byte offset of this image's output inside the batch output buffer.  roi, scale: a request roi_rect accepted
+// (nullptr, 1: the whole image; BJ_OUT_REF_MCUS always takes the whole image at full size).
 inline void fill_imgdev(const bj_image_desc &d, const Geometry &g, int format, uint32_t du_base, uint64_t out_base, ImgDev *im,
-                        const bj_roi *roi = nullptr) {
+                        const bj_roi *roi = nullptr, uint32_t scale = 1) {
     memset(im, 0, sizeof(*im));
     im->width = d.width; im->height = d.height;
     im->nmx = g.nmx; im->nmy = g.nmy;
     im->du_base = du_base;
     im->hs = d.hs; im->vs = d.vs; im->ncomp = d.ncomp; im->bpm = (uint8_t)g.bpm;
     im->valid = 1;
+    if (format == BJ_OUT_REF_MCUS) { roi = nullptr; scale = 1; }
     bj_roi r{};
-    roi_rect(d, format == BJ_OUT_REF_MCUS ? nullptr : roi, &r);
-    set_crop(r, im);
+    roi_rect(d, roi, scale, &r);
+    set_crop(r, scale_log2_of(scale), im);
     im->row_bytes = r.w * 3;
     if (format == BJ_OUT_REF_MCUS) {
         im->row_pad = 0; im->out_pitch = 0; im->row_dir = 1; im->bgr = 0;
@@ -295,10 +307,10 @@ inline uint32_t ref_mcus_chunks(const bj_image_desc &d, int M) {
     const uint32_t pw = (d.mcu_w_real + 1) / 2 * 2, ph = (d.mcu_h_real + 1) / 2 * 2;
     return (pw * ph + (uint32_t)M - 1) / (uint32_t)M;
 }
-// roi: as for fill_imgdev (BJ_OUT_REF_MCUS ignores it)
-inline size_t output_bytes(const bj_image_desc &d, int format, int M, const bj_roi *roi = nullptr) {
+// roi, scale: as for fill_imgdev (BJ_OUT_REF_MCUS ignores them)
+inline size_t output_bytes(const bj_image_desc &d, int format, int M, const bj_roi *roi = nullptr, uint32_t scale = 1) {
     bj_roi r{};
-    roi_rect(d, roi, &r);
+    roi_rect(d, roi, scale, &r);
     const size_t w = r.w, h = r.h;
     if (format == BJ_OUT_RGB8) return w * h * 3;
     if (format == BJ_OUT_BMP) return 26 + h * (w * 3 + w % 4);

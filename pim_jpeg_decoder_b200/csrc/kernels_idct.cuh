@@ -19,6 +19,9 @@ constexpr int kSmemQ = 1024;                             // 3 * kQPitch words, p
 constexpr int kRgbFront = 16;                            // slack in front of the staging tile (the copy-out reads whole words)
 constexpr int kRgbMax = 1536 * 8 * 3;                    // widest tile: gray, 192 MCUs x 8 px x 8 rows x 3 B
 constexpr int kSmemIdctColor = kSmemDu + kSmemQ + kRgbFront + kRgbMax + 64;
+// Scaled output: the compact tile of box averages (at most a quarter of the widest pixel tile) lives at the front of
+// s_du, with kRgbFront bytes in front and, behind it, the 20 bytes the copy-out's last-chunk read may reach past a row.
+static_assert(kRgbFront + kRgbMax / 4 + 20 <= kSmemDu, "the compact tile of a scaled image fits in s_du");
 
 __device__ __forceinline__ uint4 pack_row(const int (&X)[64], int r) {
     uint4 v;
@@ -129,10 +132,186 @@ __device__ __forceinline__ void tile_idct(uint4 *s_du, const uint32_t *s_q, cons
     }
 }
 
+// Stage 3 of one tile: copy-out.  `src`: the tile's packed pixels, `pitch` bytes per row, `ncols` x `rows` pixels whose
+// top-left pixel is (x0, y0) of the output image (the full image, or the scaled one); the image record's crop window and
+// output layout are in the same coordinates.
+__device__ __forceinline__ void tile_copy_out(const uint8_t *src, const int pitch, const int x0, const int y0, const int ncols, const int rows,
+                                              const TileDev &t, const ImgDev *__restrict__ im, uint8_t *__restrict__ out) {
+    const int tid = threadIdx.x;
+    // Each pixel row of the tile is a contiguous byte run in HBM with arbitrary
+    // alignment; it is written as 16-byte-aligned 128-bit stores whose payload is funnel-shifted out of the
+    // staging tile; only the first/last chunk of a run (and BMP pad bytes) go bytewise.  Only the image's crop window
+    // leaves (the whole image unless a region of interest was asked for): tile rows y0 + r in [cy, cy + ch), columns
+    // [xs, xe) = the tile's columns inside [cx, cx + cw); pixel (x, y) goes to row y - cy, column x - cx of the output.
+    {
+        const int cx = (int)im->cx, cy = (int)im->cy, cx_end = cx + (int)im->cw;
+        const int xs = max(x0, cx), xe = min(x0 + ncols, cx_end);
+        const int r_lo = max(cy - y0, 0), r_hi = min(rows, cy + (int)im->ch - y0);
+        const int payload = (xe - xs) * 3;
+        const int len = payload + (xe == cx_end ? (int)im->row_pad : 0);   // BMP pad bytes follow the run at the crop's right edge
+        const int warp = tid >> 5, lane = tid & 31;
+        const long long row_step = (long long)im->row_dir * (long long)im->out_pitch;
+        const long long off0 = (long long)im->out_row0 + row_step * (long long)(y0 - cy) + (long long)(xs - cx) * 3;
+        const uint8_t *sp0 = src + (xs - x0) * 3;                        // (any byte alignment: the funnel shift below takes it)
+        for (int r = r_lo + warp; r < r_hi; r += kTileThreads / 32) {
+            uint8_t *g = out + (off0 + row_step * r);
+            const uint8_t *sp = sp0 + r * pitch;
+            // the run [0, len) = head bytes up to the first 16-byte boundary, nfull whole aligned chunks, ntail bytes
+            const int head = min((int)((16u - ((unsigned)(uintptr_t)g & 15u)) & 15u), len);
+            const int nfull = (len - head) >> 4;
+            const int tail0 = head + 16 * nfull;
+            // head and tail bytes in one store: lanes 0-15 a head byte each, lanes 16-31 a tail byte each
+            {
+                const int idx = lane < 16 ? lane : tail0 + lane - 16;
+                const bool ok = lane < 16 ? lane < head : idx < len;
+                if (ok) g[idx] = idx < payload ? sp[idx] : (uint8_t)0;
+            }
+            // body: whole aligned 16-byte chunks.  Those that hold only pixel bytes first (no masking); BMP pad bytes
+            // (at most 3 per row) can only lie in the last whole chunk
+            const uint8_t *p0 = sp + head;
+            const unsigned a = (unsigned)__cvta_generic_to_shared(p0);
+            const unsigned sh = (a & 3u) * 8u;
+            const unsigned wa = a & ~3u;                                   // shared-memory address of the first word
+            uint4 *gp = reinterpret_cast<uint4 *>(g + head);
+            const int nbody = min(nfull, max(payload - head, 0) >> 4);
+            for (int i = lane; i < nbody; i += 32) {
+                uint32_t w0, w1, w2, w3, w4;
+                asm volatile("ld.shared.u32 %0, [%5];\n\tld.shared.u32 %1, [%5+4];\n\tld.shared.u32 %2, [%5+8];\n\tld.shared.u32 %3, [%5+12];\n\tld.shared.u32 %4, [%5+16];"
+                             : "=r"(w0), "=r"(w1), "=r"(w2), "=r"(w3), "=r"(w4) : "r"(wa + 16u * (unsigned)i));
+                uint4 v;
+                v.x = __funnelshift_r(w0, w1, sh); v.y = __funnelshift_r(w1, w2, sh);
+                v.z = __funnelshift_r(w2, w3, sh); v.w = __funnelshift_r(w3, w4, sh);
+                __stcs(gp + i, v);
+            }
+            if (nbody < nfull && lane == 0) {                              // the chunk with pad bytes (zero) in it
+                const int i = nbody;
+                const uint32_t *wp = reinterpret_cast<const uint32_t *>(p0 - (a & 3u));
+                const uint32_t w0 = wp[4 * i], w1 = wp[4 * i + 1], w2 = wp[4 * i + 2], w3 = wp[4 * i + 3], w4 = wp[4 * i + 4];
+                uint32_t vv[4] = {__funnelshift_r(w0, w1, sh), __funnelshift_r(w1, w2, sh), __funnelshift_r(w2, w3, sh), __funnelshift_r(w3, w4, sh)};
+                const int keep = payload - head - 16 * i;                  // data bytes in the chunk, < 16
+#pragma unroll
+                for (int w = 0; w < 4; w++) {
+                    const int kb = keep - 4 * w;
+                    vv[w] = kb >= 4 ? vv[w] : (kb <= 0 ? 0u : (vv[w] & (0xFFFFFFFFu >> (32 - 8 * kb))));
+                }
+                __stcs(gp + i, make_uint4(vv[0], vv[1], vv[2], vv[3]));
+            }
+        }
+        // BMP file header (src/bmp_writer.cpp:26-41) of the cw x ch output, written by the tile that holds pixel (cx, cy):
+        // 'B','M', size(4), 0(4), 0x1A(4), 12(4), width(2), height(2), 1(2), 24(2)
+        if (im->bgr && t.my == im->my_lo && t.mx0 == im->mx_lo && tid < 26) {
+            const unsigned W = im->cw, H = im->ch;
+            const unsigned size = 26u + H * W * 3u + im->row_pad * H;
+            unsigned v = 0;
+            if (tid == 0) v = 'B';
+            else if (tid == 1) v = 'M';
+            else if (tid < 6) v = size >> ((tid - 2) * 8);
+            else if (tid == 10) v = 0x1A;
+            else if (tid == 14) v = 12;
+            else if (tid == 18) v = W;
+            else if (tid == 19) v = W >> 8;
+            else if (tid == 20) v = H;
+            else if (tid == 21) v = H >> 8;
+            else if (tid == 22) v = 1;
+            else if (tid == 24) v = 24;
+            const long long hdr = (long long)im->out_row0 - (long long)(H - 1) * (long long)im->out_pitch - 26;
+            out[hdr + tid] = (uint8_t)v;
+        }
+    }
+}
+
+// Reciprocals of the box sizes n = 1..64 of the reduction below: kBoxRcp.r[n] = ceil(2^31 / n).  For a < 2^15,
+// __umulhi(2a, r[n]) = floor(a * r[n] / 2^31) = floor(a / n) exactly (a * (r[n] * n - 2^31) < 2^15 * 64 < 2^31).
+struct BoxRcp {
+    uint32_t r[65];
+    constexpr BoxRcp() : r() {
+        for (uint32_t n = 1; n <= 64; n++) r[n] = (uint32_t)((((uint64_t)1 << 31) + n - 1) / n);
+    }
+};
+__constant__ BoxRcp kBoxRcp = BoxRcp();
+
+// Box reduction of one tile (scaled output, s = 1 << SL in {2, 4, 8}): output pixel (X, Y) of the tile is the rounded
+// mean, per channel, of the pixels [sX, sX + s) x [sY, sY + s) of the `ncols` x `rows` pixel tile `src` (`pitch` bytes per
+// row, top-left pixel (x0, y0) of the full image) that lie inside the image: pixels at x >= width or y >= height (MCU
+// padding) count in neither sum nor divisor.  x0, y0, ncols and rows are multiples of 8, so every box lies inside the
+// tile.  Into `dst`: (ncols / s) x (rows / s) pixels, 3 * ncols / s bytes per row.
+// One item = one quad of 4 horizontally adjacent pixels (three words of `src`) in the s rows of one output row.  Lanes
+// take consecutive quads: word addresses 3 apart, which no two lanes of a warp share a bank with.  A quad is 2 output
+// pixels at s = 2 and 1 at s = 4; at s = 8 the two lanes of a quad pair add their sums with a shuffle.  The bytes are
+// summed two per word in 16-bit lanes (at most 8 * 255 per column, 64 * 255 per box).  Only quads that reach past the
+// image's right edge mask bytes out; the rounded division is a multiply by the box size's reciprocal.
+template <int SL>
+__device__ __forceinline__ void tile_box_reduce(const uint8_t *src, const int pitch, const int ncols, const int rows, const int x0, const int y0,
+                                                const ImgDev *__restrict__ im, uint8_t *dst) {
+    constexpr int S = 1 << SL;
+    const int tid = threadIdx.x;
+    const int nq = ncols >> 2, orows = rows >> SL, opitch = (ncols >> SL) * 3;
+    const int items = orows * nq;                                    // (nq is even: ncols is a multiple of 8)
+    const unsigned inv = 0xFFFFFFFFu / (unsigned)nq + 1u;
+    const int wpitch = pitch >> 2;
+    const int W = (int)im->width - x0, H = (int)im->height - y0;   // (the image's extent seen from the tile's origin)
+    for (int base = 0; base < items; base += kTileThreads) {         // (uniform trip count: the s = 8 shuffle needs every lane)
+        const int it = base + tid;
+        const int oy = (int)__umulhi((unsigned)it, inv), q = it - oy * nq;
+        const int nr = it < items ? min(S, H - (oy << SL)) : 0;      // rows of the box inside the image
+        const int nv = W - 4 * q;                                    // pixels of the quad inside the image (4 or more: all)
+        uint32_t m[3] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu};
+        if (nv < 4) {
+#pragma unroll
+            for (int j = 0; j < 3; j++) {
+                const int kb = 3 * max(nv, 0) - 4 * j;
+                m[j] = kb >= 4 ? 0xFFFFFFFFu : (kb <= 0 ? 0u : (0xFFFFFFFFu >> (32 - 8 * kb)));
+            }
+        }
+        uint32_t lo[3] = {0, 0, 0}, hi[3] = {0, 0, 0};               // bytes 4j, 4j + 2 / 4j + 1, 4j + 3 of the quad, column sums
+        const uint32_t *wp = reinterpret_cast<const uint32_t *>(src) + (oy << SL) * wpitch + 3 * q;
+#pragma unroll
+        for (int r = 0; r < S; r++) {
+            if (r < nr) {
+#pragma unroll
+                for (int j = 0; j < 3; j++) {
+                    const uint32_t w = wp[r * wpitch + j] & m[j];
+                    lo[j] += w & 0x00FF00FFu;
+                    hi[j] += (w >> 8) & 0x00FF00FFu;
+                }
+            }
+        }
+        // per-pixel channel sums: byte k = 3p + c of the quad
+        unsigned S_[12];
+#pragma unroll
+        for (int j = 0; j < 3; j++) {
+            S_[4 * j] = lo[j] & 0xFFFFu; S_[4 * j + 1] = hi[j] & 0xFFFFu; S_[4 * j + 2] = lo[j] >> 16; S_[4 * j + 3] = hi[j] >> 16;
+        }
+        unsigned v[2][3];
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+            v[0][c] = S_[c] + S_[3 + c];
+            v[1][c] = S_[6 + c] + S_[9 + c];
+            if (SL >= 2) v[0][c] += v[1][c];
+            if (SL == 3) v[0][c] += __shfl_xor_sync(0xFFFFFFFFu, v[0][c], 1);
+        }
+        constexpr int NOUT = SL == 1 ? 2 : 1;                        // output pixels of this lane
+        const int X = SL == 1 ? 2 * q : (SL == 2 ? q : q >> 1);      // the first one's column in the tile
+        const bool mine = SL != 3 || (q & 1) == 0;                   // (s = 8: the even lane of the pair writes)
+#pragma unroll
+        for (int k = 0; k < NOUT; k++) {
+            const int nc = min(S, W - ((X + k) << SL));               // columns of the box inside the image
+            if (mine && nr > 0 && nc > 0) {                          // (a box of MCU padding only is never copied out)
+                const unsigned n = (unsigned)(nc * nr);
+                const unsigned rcp = kBoxRcp.r[n];
+                uint8_t *d = dst + oy * opitch + (X + k) * 3;
+#pragma unroll
+                for (int c = 0; c < 3; c++) d[c] = (uint8_t)__umulhi((v[k][c] + (n >> 1)) << 1, rcp);
+            }
+        }
+    }
+}
+
 // Stages 2 and 3 of one tile: colour conversion into the staging tile `s_rgb`, copy-out (REF_MCUS: straight to HBM).
 // HS, VS: the luma sampling factors as compile-time constants for three-component images (the index arithmetic of the
 // colour stage folds: 4:2:0 and 4:4:4 have their own instances), or 0, 0: whatever the image record says.
-template <bool REF_MCUS, int HS, int VS>
+// SCALED: images may ask for reduced-size output (ImgDev::scale_log2 > 0); without it the record's scale is not read.
+template <bool REF_MCUS, bool SCALED, int HS, int VS>
 __device__ __forceinline__ void tile_color_store(const uint4 *s_du, uint8_t *s_rgb, const TileDev &t, const ImgDev *__restrict__ im, const int hs_rt,
                                                  const int vs_rt, const int ncomp_rt, const int bpm_rt, uint8_t *__restrict__ out) {
     const int hs = HS ? HS : hs_rt, vs = HS ? VS : vs_rt, ncomp = HS ? 3 : ncomp_rt, bpm = HS ? HS * VS + 2 : bpm_rt;
@@ -207,93 +386,28 @@ __device__ __forceinline__ void tile_color_store(const uint4 *s_du, uint8_t *s_r
     if (REF_MCUS) return;
     __syncthreads();
 
-    // ---- stage 3: copy-out.  Each pixel row of the tile is a contiguous byte run in HBM with arbitrary
-    // alignment; it is written as 16-byte-aligned 128-bit stores whose payload is funnel-shifted out of the
-    // staging tile; only the first/last chunk of a run (and BMP pad bytes) go bytewise.  Only the image's crop window
-    // leaves (the whole image unless a region of interest was asked for): tile rows y0 + r in [cy, cy + ch), columns
-    // [xs, xe) = the tile's columns inside [cx, cx + cw); pixel (x, y) goes to row y - cy, column x - cx of the output.
-    {
-        const int x0 = t.mx0 * hs * 8, y0 = t.my * vs * 8;
-        const int cx = (int)im->cx, cy = (int)im->cy, cx_end = cx + (int)im->cw;
-        const int xs = max(x0, cx), xe = min(x0 + nseg * 8, cx_end);
-        const int r_lo = max(cy - y0, 0), r_hi = min(rows, cy + (int)im->ch - y0);
-        const int payload = (xe - xs) * 3;
-        const int len = payload + (xe == cx_end ? (int)im->row_pad : 0);   // BMP pad bytes follow the run at the crop's right edge
-        const int warp = tid >> 5, lane = tid & 31;
-        const long long row_step = (long long)im->row_dir * (long long)im->out_pitch;
-        const long long off0 = (long long)im->out_row0 + row_step * (long long)(y0 - cy) + (long long)(xs - cx) * 3;
-        const uint8_t *sp0 = s_rgb + (xs - x0) * 3;                        // (any byte alignment: the funnel shift below takes it)
-        for (int r = r_lo + warp; r < r_hi; r += kTileThreads / 32) {
-            uint8_t *g = out + (off0 + row_step * r);
-            const uint8_t *sp = sp0 + r * pitch;
-            // the run [0, len) = head bytes up to the first 16-byte boundary, nfull whole aligned chunks, ntail bytes
-            const int head = min((int)((16u - ((unsigned)(uintptr_t)g & 15u)) & 15u), len);
-            const int nfull = (len - head) >> 4;
-            const int tail0 = head + 16 * nfull;
-            // head and tail bytes in one store: lanes 0-15 a head byte each, lanes 16-31 a tail byte each
-            {
-                const int idx = lane < 16 ? lane : tail0 + lane - 16;
-                const bool ok = lane < 16 ? lane < head : idx < len;
-                if (ok) g[idx] = idx < payload ? sp[idx] : (uint8_t)0;
-            }
-            // body: whole aligned 16-byte chunks.  Those that hold only pixel bytes first (no masking); BMP pad bytes
-            // (at most 3 per row) can only lie in the last whole chunk
-            const uint8_t *p0 = sp + head;
-            const unsigned a = (unsigned)__cvta_generic_to_shared(p0);
-            const unsigned sh = (a & 3u) * 8u;
-            const unsigned wa = a & ~3u;                                   // shared-memory address of the first word
-            uint4 *gp = reinterpret_cast<uint4 *>(g + head);
-            const int nbody = min(nfull, max(payload - head, 0) >> 4);
-            for (int i = lane; i < nbody; i += 32) {
-                uint32_t w0, w1, w2, w3, w4;
-                asm volatile("ld.shared.u32 %0, [%5];\n\tld.shared.u32 %1, [%5+4];\n\tld.shared.u32 %2, [%5+8];\n\tld.shared.u32 %3, [%5+12];\n\tld.shared.u32 %4, [%5+16];"
-                             : "=r"(w0), "=r"(w1), "=r"(w2), "=r"(w3), "=r"(w4) : "r"(wa + 16u * (unsigned)i));
-                uint4 v;
-                v.x = __funnelshift_r(w0, w1, sh); v.y = __funnelshift_r(w1, w2, sh);
-                v.z = __funnelshift_r(w2, w3, sh); v.w = __funnelshift_r(w3, w4, sh);
-                __stcs(gp + i, v);
-            }
-            if (nbody < nfull && lane == 0) {                              // the chunk with pad bytes (zero) in it
-                const int i = nbody;
-                const uint32_t *wp = reinterpret_cast<const uint32_t *>(p0 - (a & 3u));
-                const uint32_t w0 = wp[4 * i], w1 = wp[4 * i + 1], w2 = wp[4 * i + 2], w3 = wp[4 * i + 3], w4 = wp[4 * i + 4];
-                uint32_t vv[4] = {__funnelshift_r(w0, w1, sh), __funnelshift_r(w1, w2, sh), __funnelshift_r(w2, w3, sh), __funnelshift_r(w3, w4, sh)};
-                const int keep = payload - head - 16 * i;                  // data bytes in the chunk, < 16
-#pragma unroll
-                for (int w = 0; w < 4; w++) {
-                    const int kb = keep - 4 * w;
-                    vv[w] = kb >= 4 ? vv[w] : (kb <= 0 ? 0u : (vv[w] & (0xFFFFFFFFu >> (32 - 8 * kb))));
-                }
-                __stcs(gp + i, make_uint4(vv[0], vv[1], vv[2], vv[3]));
-            }
-        }
-        // BMP file header (src/bmp_writer.cpp:26-41) of the cw x ch output, written by the tile that holds pixel (cx, cy):
-        // 'B','M', size(4), 0(4), 0x1A(4), 12(4), width(2), height(2), 1(2), 24(2)
-        if (im->bgr && t.my == im->my_lo && t.mx0 == im->mx_lo && tid < 26) {
-            const unsigned W = im->cw, H = im->ch;
-            const unsigned size = 26u + H * W * 3u + im->row_pad * H;
-            unsigned v = 0;
-            if (tid == 0) v = 'B';
-            else if (tid == 1) v = 'M';
-            else if (tid < 6) v = size >> ((tid - 2) * 8);
-            else if (tid == 10) v = 0x1A;
-            else if (tid == 14) v = 12;
-            else if (tid == 18) v = W;
-            else if (tid == 19) v = W >> 8;
-            else if (tid == 20) v = H;
-            else if (tid == 21) v = H >> 8;
-            else if (tid == 22) v = 1;
-            else if (tid == 24) v = 24;
-            const long long hdr = (long long)im->out_row0 - (long long)(H - 1) * (long long)im->out_pitch - 26;
-            out[hdr + tid] = (uint8_t)v;
-        }
+    // ---- stage 3: copy-out of the pixel tile.  Scaled output: each s x s box of it is first averaged into the compact
+    // tile, which lives at the front of s_du (free once stage 2 has read it), and the copy-out works on that.  (The
+    // compact tile is addressed as an offset from s_rgb, not as a second pointer: with the pointer, ptxas spills two
+    // registers across stage 1.)
+    const int x0 = t.mx0 * hs * 8, y0 = t.my * vs * 8;
+    const int sl = SCALED ? im->scale_log2 : 0;
+    int src_off = 0;
+    if (SCALED && sl) {
+        src_off = kRgbFront - (kSmemDu + kSmemQ + kRgbFront);
+        if (sl == 1) tile_box_reduce<1>(s_rgb, pitch, nseg * 8, rows, x0, y0, im, s_rgb + src_off);
+        else if (sl == 2) tile_box_reduce<2>(s_rgb, pitch, nseg * 8, rows, x0, y0, im, s_rgb + src_off);
+        else tile_box_reduce<3>(s_rgb, pitch, nseg * 8, rows, x0, y0, im, s_rgb + src_off);
+        __syncthreads();
     }
+    tile_copy_out(s_rgb + src_off, ((nseg * 8) >> sl) * 3, x0 >> sl, y0 >> sl, (nseg * 8) >> sl, rows >> sl, t, im, out);
 }
 
-template <bool REF_MCUS>
+template <bool REF_MCUS, bool SCALED>
 __global__ void __launch_bounds__(kTileThreads, 4)
 k_idct_color(const int16_t *__restrict__ coef, const int16_t *__restrict__ dc_plane, const ImgDev *__restrict__ imgs,
              const QTab *__restrict__ qtabs, const TileDev *__restrict__ tiles, uint8_t *__restrict__ out) {
+    static_assert(!(REF_MCUS && SCALED), "the reference's tile layout has no scaled form");
     extern __shared__ __align__(16) uint8_t smem[];
     uint4 *s_du = reinterpret_cast<uint4 *>(smem);
     uint32_t *s_q = reinterpret_cast<uint32_t *>(smem + kSmemDu);
@@ -340,9 +454,9 @@ k_idct_color(const int16_t *__restrict__ coef, const int16_t *__restrict__ dc_pl
 
     tile_idct(s_du, s_q, s_dc, ndu, hs, vs, bpm, dc_plane != nullptr);
     __syncthreads();
-    if (ncomp == 3 && hs == 2 && vs == 2) tile_color_store<REF_MCUS, 2, 2>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
-    else if (ncomp == 3 && hs == 1 && vs == 1) tile_color_store<REF_MCUS, 1, 1>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
-    else tile_color_store<REF_MCUS, 0, 0>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
+    if (ncomp == 3 && hs == 2 && vs == 2) tile_color_store<REF_MCUS, SCALED, 2, 2>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
+    else if (ncomp == 3 && hs == 1 && vs == 1) tile_color_store<REF_MCUS, SCALED, 1, 1>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
+    else tile_color_store<REF_MCUS, SCALED, 0, 0>(s_du, s_rgb, t, im, hs, vs, ncomp, bpm, out);
 }
 
 // REF_MCUS: what the DPUs leave in the parts of the buffer no pixel lives in - positions of the 2x2-padded grid outside

@@ -6,7 +6,7 @@
     pim.copy / pim.exec / pim.copy     (:276-308)          Decoder.exec_mcus(metadata, mcus)      [compat layout]
     read_JPEG                          (jpeg_scanner:345)  parse_header(bytes)
     decode_Huffman_data + exec + write_BMP gather          Decoder.decode(files, fmt) / Batch     [fast layout]
-    (a crop of each image: rois=, see roi_output_size)
+    (a crop of each image: rois=, see roi_output_size; at 1/2, 1/4 or 1/8 size: scales=, see scaled_output_size)
     main(argv): sort by size, decode, write <name>.bmp     decode_files(paths)
 """
 import ctypes as C
@@ -34,12 +34,36 @@ def _roi_table(rois, n):
     return a, a.ctypes.data_as(C.c_void_p)
 
 
+def _scale_table(scales, n):
+    """scales: None (full size), one int for every image, or n of them - each 1, 2, 4 or 8 (any other value is refused per
+    image by the library).  -> (keepalive uint8 array or None, pointer for the C ABI)"""
+    if scales is None:
+        return None, None
+    v = np.broadcast_to(np.asarray(scales), (n,))
+    if v.dtype.kind not in "iuf":
+        raise TypeError(f"scales must be numbers, not {v.dtype}")
+    # a value that is not a whole number in 1..8 would wrap or truncate to some other scale in the uint8 cast: it goes
+    # to the library as 0, which refuses that image (BJ_ERR_ARG) like any other scale it does not have
+    ok = (v >= 1) & (v <= 8) & (v == np.floor(v)) if v.dtype.kind == "f" else (v >= 1) & (v <= 8)
+    a = np.ascontiguousarray(np.where(ok, v, 0).astype(np.uint8))
+    return a, a.ctypes.data_as(C.c_void_p)
+
+
 def roi_output_size(desc, roi, fmt=L.BJ_OUT_RGB8):
     """Output bytes of the image `desc` (ImageDesc) cropped to `roi` ((x, y, w, h), a Roi, or None for the whole image);
     0 if the ROI does not fit the image, and for BJ_OUT_REF_MCUS."""
     if roi is not None and not isinstance(roi, L.Roi):
         roi = L.Roi(*(int(v) for v in roi))
     return L.lib().bj_roi_output_size(C.byref(desc), C.byref(roi) if roi is not None else None, fmt)
+
+
+def scaled_output_size(desc, roi, scale, fmt=L.BJ_OUT_RGB8):
+    """Output bytes of the image `desc` at 1/scale of its size (scale 1, 2, 4 or 8) cropped to `roi`, a rectangle of the
+    scaled image ((x, y, w, h), a Roi, or None for all of it); 0 if the scale or the ROI is refused, and for
+    BJ_OUT_REF_MCUS."""
+    if roi is not None and not isinstance(roi, L.Roi):
+        roi = L.Roi(*(int(v) for v in roi))
+    return L.lib().bj_scaled_output_size(C.byref(desc), C.byref(roi) if roi is not None else None, int(scale), fmt)
 
 
 class PinnedBuffer:
@@ -76,15 +100,17 @@ def _file_arrays(files):
 
 class Batch:
     """A device-resident batch (bj_batch): upload -> decode -> download, each asynchronous on the context's stream.
-    rois: None, or one (x, y, w, h) crop per image (see roi_output_size)."""
+    rois: None, or one (x, y, w, h) crop per image (see roi_output_size); scales: None, or a scale denominator for every
+    image or one per image (see scaled_output_size; a ROI is then a rectangle of the scaled image)."""
 
-    def __init__(self, dec, files, fmt=L.BJ_OUT_RGB8, rois=None):
+    def __init__(self, dec, files, fmt=L.BJ_OUT_RGB8, rois=None, scales=None):
         self.dec = dec
         self.n = len(files)
         self._keep, ptrs, lens = _file_arrays(files)
         _, rp = _roi_table(rois, self.n)
+        _, sp = _scale_table(scales, self.n)
         self.h = C.c_void_p()
-        L.check(L.lib().bj_batch_create_roi(dec.ctx, ptrs, lens, rp, self.n, fmt, C.byref(self.h)), "bj_batch_create_roi", dec.ctx)
+        L.check(L.lib().bj_batch_create_scaled(dec.ctx, ptrs, lens, rp, sp, self.n, fmt, C.byref(self.h)), "bj_batch_create_scaled", dec.ctx)
         self.offsets, self.sizes, self.parse_status = [], [], []
         for i in range(self.n):
             off, nb = C.c_size_t(), C.c_size_t()
@@ -229,23 +255,27 @@ class Decoder:
         return out
 
     # ---- full path, one call (host buffers in, host buffers out)
-    def decode(self, files, fmt=L.BJ_OUT_RGB8, outs=None, rois=None):
+    def decode(self, files, fmt=L.BJ_OUT_RGB8, outs=None, rois=None, scales=None):
         """Returns (list of uint8 arrays or None for rejected files, list of per-image status).  rois: None, or one
-        (x, y, w, h) crop per image (see roi_output_size); an image whose ROI does not fit gets BJ_ERR_ARG."""
+        (x, y, w, h) crop per image (see roi_output_size); scales: None, or a scale denominator (1, 2, 4, 8) for every
+        image or one per image (see scaled_output_size).  An image whose scale or ROI is refused gets BJ_ERR_ARG."""
         n = len(files)
         keep, ptrs, lens = _file_arrays(files)
         ra, rp = _roi_table(rois, n)
+        sa, sp = _scale_table(scales, n)
         if outs is None:
             outs = []
             for i, f in enumerate(files):
                 st, d = parse_header(f)
                 size = 0
-                if st == L.BJ_OK:
-                    size = L.lib().bj_output_size(C.byref(d), fmt) if ra is None else roi_output_size(d, ra[i], fmt)
+                if st == L.BJ_OK and ra is None and sa is None:
+                    size = L.lib().bj_output_size(C.byref(d), fmt)          # (BJ_OUT_REF_MCUS included: it has no crop or scale)
+                elif st == L.BJ_OK:
+                    size = scaled_output_size(d, None if ra is None else ra[i], 1 if sa is None else sa[i], fmt)
                 outs.append(np.zeros(size, dtype=np.uint8) if size else None)
         optrs = (C.c_void_p * max(n, 1))(*[o.__array_interface__["data"][0] if o is not None else None for o in outs])
         status = (C.c_int * max(n, 1))()
-        L.check(L.lib().bj_decode_batch_roi(self.ctx, ptrs, lens, rp, n, fmt, optrs, status), "bj_decode_batch_roi", self.ctx)
+        L.check(L.lib().bj_decode_batch_scaled(self.ctx, ptrs, lens, rp, sp, n, fmt, optrs, status), "bj_decode_batch_scaled", self.ctx)
         st = list(status)[:n]
         return [o if s in (L.BJ_OK, L.BJ_ERR_CORRUPT_SCAN) else None for o, s in zip(outs, st)], st
 
@@ -267,35 +297,38 @@ class Decoder:
             outs = [o.view(np.int16) for o in outs]
         return outs, list(status)[:n]
 
-    def decode_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None):
+    def decode_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None, scales=None):
         """bj_decode_batch for a batch-pipeline caller: the n files sit in ONE host buffer `src` (uint8 array, ideally
         a PinnedBuffer) at byte offsets `src_off` with lengths `src_len`; image i is written to `dst[dst_off[i]:]`
-        (bj_output_size bytes, or bj_roi_output_size with `rois`: an (n, 4) uint32 array of (x, y, w, h) crops).  The
-        pointer tables are built with vector arithmetic, so the host-side cost per call does not grow with a Python
-        loop over images.  Returns the per-image status as an int32 array."""
+        (bj_output_size bytes, or bj_scaled_output_size with `rois`: an (n, 4) uint32 array of (x, y, w, h) crops, and
+        `scales`: a scale denominator for every image or one per image).  The pointer tables are built with vector
+        arithmetic, so the host-side cost per call does not grow with a Python loop over images.  Returns the
+        per-image status as an int32 array."""
         n = len(src_off)
         ip = (np.asarray(src_off, dtype=np.uint64) + np.uint64(src.__array_interface__["data"][0]))
         il = np.ascontiguousarray(src_len, dtype=np.uint64)
         op = (np.asarray(dst_off, dtype=np.uint64) + np.uint64(dst.__array_interface__["data"][0]))
         ra, rp = _roi_table(rois, n)
+        sa, sp = _scale_table(scales, n)
         status = np.zeros(max(n, 1), dtype=np.int32)
-        L.check(L.lib().bj_decode_batch_roi(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, n, fmt,
-                                            op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p)), "bj_decode_batch_roi", self.ctx)
+        L.check(L.lib().bj_decode_batch_scaled(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, sp, n, fmt,
+                                               op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p)), "bj_decode_batch_scaled", self.ctx)
         return status[:n]
 
 
-    def submit_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None):
+    def submit_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None, scales=None):
         """decode_packed without waiting (bj_submit): returns a Job; job.wait() gives the status array."""
         n = len(src_off)
         ip = (np.asarray(src_off, dtype=np.uint64) + np.uint64(src.__array_interface__["data"][0]))
         il = np.ascontiguousarray(src_len, dtype=np.uint64)
         op = (np.asarray(dst_off, dtype=np.uint64) + np.uint64(dst.__array_interface__["data"][0]))
         ra, rp = _roi_table(rois, n)
+        sa, sp = _scale_table(scales, n)
         status = np.zeros(max(n, 1), dtype=np.int32)
         h = C.c_void_p()
-        L.check(L.lib().bj_submit_roi(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, n, fmt,
-                                      op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p), C.byref(h)), "bj_submit_roi", self.ctx)
-        return Job(self, h, (ip, il, op, ra, src, dst), status, n)
+        L.check(L.lib().bj_submit_scaled(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, sp, n, fmt,
+                                         op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p), C.byref(h)), "bj_submit_scaled", self.ctx)
+        return Job(self, h, (ip, il, op, ra, sa, src, dst), status, n)
 
 
 def lpt_shards(costs, world_size):
