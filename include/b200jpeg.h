@@ -178,6 +178,39 @@ size_t bj_scaled_output_size(const bj_image_desc *desc, const bj_roi *roi, int s
 int bj_decode_batch_scaled(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois,
                            const uint8_t *scales, int n, int format, uint8_t *const *outs, int *status);
 
+/* FIXED-SIZE OUTPUT.  Image i is output at exactly sizes[i] = {w, h} pixels: the source is what the _scaled entry
+ * outputs for it - the crop rois[i] of the image scaled by 1/scales[i] - of cw x ch pixels, and output pixel (X, Y) is,
+ * per channel, the integer bilinear sample of the source with half-pixel centres (as torch's interpolate(...,
+ * mode="bilinear", align_corners=False, antialias=False)):
+ *     taps(n_src, n_dst, X):   num = max((2X + 1) * n_src - n_dst, 0), den = 2 * n_dst  (64-bit integers)
+ *                              i0 = num / den, f = ((num % den) * 256) / den,  i1 = min(i0 + 1, n_src - 1)
+ *     x0, x1, fx = taps(cw, w, X);   y0, y1, fy = taps(ch, h, Y)
+ *     top = (256 - fx) * S[y0][x0] + fx * S[y0][x1],  bot = (256 - fx) * S[y1][x0] + fx * S[y1][x1]
+ *     out = ((256 - fy) * top + fy * bot + 32768) >> 16
+ * At w x h = cw x ch this is the source itself; an exact 2x reduction of an even-sized source is its 2x2 box average.
+ * There is no antialiasing filter: a reduction by more than 2x aliases, as torch's antialias=False does.  Pick the scale
+ * so that the bilinear stage reduces by less than 2x (the Python helper resize_plan does): the box average of the
+ * scaled decode is the filter.  Output layouts are those of a w x h image: BJ_OUT_RGB8 w*h*3 bytes top-down,
+ * BJ_OUT_BMP a 26-byte header with w and h, bottom-up B,G,R rows and w%4 pad bytes after each.
+ * {0,0} (or sizes == NULL) is no resize: exactly the _scaled entry's output.  The parity rules carry over: a damaged
+ * scan gives the resized crop of the partial image, a subsampled image with restart markers that of its restart-free
+ * twin, a gray image R = G = B.  Refused per image, the rest of the batch decodes: only one of w, h is 0 or either is
+ * above 65535 (BJ_ERR_ARG); w*h above "max_image_pixels" (BJ_ERR_UNSUPPORTED, as a full image would be); a bad scale or
+ * ROI (BJ_ERR_ARG).  BJ_OUT_REF_MCUS is refused for the whole call when sizes != NULL.  Output sizes and offsets,
+ * out_bytes and d2h_bytes count the final w x h output; the sub-batch cut ("sub_batch_out_bytes") counts it plus the
+ * scaled crop the resize reads, which the sub-batch holds in HBM too; "max_image_pixels" and bj_batch_info.pixels count
+ * the full image.  All three arrays, when given, must stay valid until the call returns (bj_submit_resized: until
+ * bj_wait returns). */
+typedef struct { uint32_t w, h; } bj_size;
+/* Output bytes of an image at 1/scale, cropped to roi and resized to *size; 0 for anything refused above (w*h is
+ * checked against the default "max_image_pixels", 2^28) and for BJ_OUT_REF_MCUS.  size == NULL or {0,0}:
+ * bj_scaled_output_size(desc, roi, scale, format). */
+size_t bj_resized_output_size(const bj_image_desc *desc, const bj_roi *roi, int scale, const bj_size *size, int format);
+/* bj_decode_batch_scaled with sizes[i] for image i (rois, scales and sizes may each be NULL); outs[i] holds
+ * bj_resized_output_size() bytes. */
+int bj_decode_batch_resized(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois,
+                            const uint8_t *scales, const bj_size *sizes, int n, int format, uint8_t *const *outs, int *status);
+
 /* FULL PATH behind the UNCHANGED scanner.  Replaces decode_Huffman_data(header, MCU_buffer, dpu_offset) + pim.copy /
  * pim.exec / pim.copy (src/decoder_host.cpp:181, :268-312) for a host that keeps read_JPEG in front: it fills one
  * bj_image_desc per `Header` (field for field, see INTEGRATION.md) and hands over the scan bytes -
@@ -207,6 +240,9 @@ int bj_submit_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, 
  * bj_wait returns. */
 int bj_submit_scaled(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
                      int n, int format, uint8_t *const *outs, int *status, bj_job **job);
+/* bj_submit with a ROI, a scale and a target size per image (see bj_decode_batch_resized). */
+int bj_submit_resized(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
+                      const bj_size *sizes, int n, int format, uint8_t *const *outs, int *status, bj_job **job);
 int bj_wait(bj_job *job);
 
 /* FULL PATH, staged (device-resident batch) - what bj_decode_batch is made of, and what bench.py times with the
@@ -221,6 +257,11 @@ int bj_batch_create_roi(bj_ctx *ctx, const uint8_t *const *files, const size_t *
  * d2h_bytes of bj_batch_info are those of the scaled crops; bj_batch_info.pixels counts full images. */
 int bj_batch_create_scaled(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois,
                            const uint8_t *scales, int n, int format, bj_batch **out);
+/* bj_batch_create with a ROI, a scale and a target size per image (see bj_decode_batch_resized): offsets, sizes,
+ * bj_batch_device_output and the out_bytes / d2h_bytes of bj_batch_info are those of the final outputs; ms_idct of
+ * bj_batch_info is the IDCT + colour stage alone. */
+int bj_batch_create_resized(bj_ctx *ctx, const uint8_t *const *files, const size_t *lens, const bj_roi *rois,
+                            const uint8_t *scales, const bj_size *sizes, int n, int format, bj_batch **out);
 int bj_batch_upload(bj_batch *b, void *stream);                 /* H2D: file bytes + descriptors          */
 int bj_batch_decode(bj_batch *b, void *stream);                 /* enqueue all kernels; input and output stay in HBM */
 int bj_batch_sync(bj_batch *b);                                 /* wait; settles the (rare) extra Huffman fix-up rounds */
@@ -296,10 +337,11 @@ int bj_set_option(bj_ctx *ctx, const char *name, long value);
  * "decode_batch_d2h_bytes", "decode_batch_d2h_copies", "decode_batch_host_ms" (header parse + layout [+ staging copy]),
  * "decode_batch_wait_ms" (caller blocked on the GPU), "host_threads", "devices", and the kernel time per stage summed
  * over the sub-batches - the reference's per-stage "Profiles" lines (src/decoder_host.cpp:379-394) -
- * "decode_batch_ms_unstuff", "decode_batch_ms_sync", "decode_batch_ms_write", "decode_batch_ms_idct";
+ * "decode_batch_ms_unstuff", "decode_batch_ms_sync", "decode_batch_ms_write", "decode_batch_ms_idct",
+ * "decode_batch_ms_resize" (the fixed-size output's resize kernel; 0 when no image of a sub-batch is resized);
  * "decode_batch_direct_uploads" (sub-batches whose files went up straight from the caller's page-locked memory).
  * "total_<counter>" (total_sub_batches, total_launches, total_h2d_bytes, total_d2h_bytes, total_host_ms, total_wait_ms,
- * total_d2h_copies, total_ms_unstuff, total_ms_sync, total_ms_write, total_ms_idct, total_direct_uploads): the same
+ * total_d2h_copies, total_ms_unstuff, total_ms_sync, total_ms_write, total_ms_idct, total_ms_resize, total_direct_uploads): the same
  * summed over every bj_decode_batch / bj_submit job since the context was created.
  * For a context of several GPUs: byte and launch counts are sums, times the maximum over the devices.
  * Environment: B200JPEG_TRACE=1 prints one line per sub-batch of bj_decode_batch (host prepare, kernels, copy-out). */

@@ -6,6 +6,6 @@ program, ``Decoder.decode`` = decode_Huffman_data + DPU program + BMP pixel gath
 ``./bin/decoder <jpeg...>`` CLI) used by the tests and the benchmark.  There is no CPU decode path.
 """
 from ._lib import (BJ_ERR_ARG, BJ_ERR_CORRUPT_SCAN, BJ_ERR_CUDA, BJ_ERR_INVALID_JPEG, BJ_ERR_UNSUPPORTED, BJ_OK, BJ_OUT_BMP,  # noqa: F401
-                   BJ_OUT_REF_MCUS, BJ_OUT_RGB8, BJ_SCAN_RAW, BJ_SCAN_UNSTUFFED, BatchInfo, BjError, ImageDesc, Roi, lib)
-from .decoder import (Batch, Decoder, Job, PinnedBuffer, decode_files, lpt_shards, parse_header, roi_output_size,  # noqa: F401
-                      scaled_output_size, shard_by_size)
+                   BJ_OUT_REF_MCUS, BJ_OUT_RGB8, BJ_SCAN_RAW, BJ_SCAN_UNSTUFFED, BatchInfo, BjError, ImageDesc, Roi, Size, lib)
+from .decoder import (Batch, Decoder, Job, PinnedBuffer, decode_files, lpt_shards, parse_header, resize_plan,  # noqa: F401
+                      resized_output_size, roi_output_size, scaled_output_size, shard_by_size)

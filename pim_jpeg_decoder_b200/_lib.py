@@ -49,6 +49,11 @@ class Roi(C.Structure):
     _fields_ = [("x", C.c_uint32), ("y", C.c_uint32), ("w", C.c_uint32), ("h", C.c_uint32)]
 
 
+class Size(C.Structure):
+    """bj_size: a target size w x h in pixels; {0, 0} = no resize"""
+    _fields_ = [("w", C.c_uint32), ("h", C.c_uint32)]
+
+
 class BatchInfo(C.Structure):
     """bj_batch_info"""
     _fields_ = [
@@ -81,19 +86,26 @@ SYMBOLS = {
     "bj_output_size": (C.c_size_t, [C.POINTER(ImageDesc), C.c_int]),
     "bj_roi_output_size": (C.c_size_t, [C.POINTER(ImageDesc), C.POINTER(Roi), C.c_int]),
     "bj_scaled_output_size": (C.c_size_t, [C.POINTER(ImageDesc), C.POINTER(Roi), C.c_int, C.c_int]),
+    "bj_resized_output_size": (C.c_size_t, [C.POINTER(ImageDesc), C.POINTER(Roi), C.c_int, C.POINTER(Size), C.c_int]),
     "bj_ref_mcus_size": (C.c_size_t, [C.POINTER(ImageDesc), C.c_int, C.POINTER(C.c_int)]),
     "bj_decode_batch_desc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bj_decode_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bj_decode_batch_roi": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bj_decode_batch_scaled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "bj_decode_batch_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                          C.c_void_p]),
     "bj_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "bj_submit_roi": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "bj_submit_scaled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                    C.POINTER(C.c_void_p)]),
+    "bj_submit_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                    C.c_void_p, C.POINTER(C.c_void_p)]),
     "bj_wait": (C.c_int, [C.c_void_p]),
     "bj_batch_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "bj_batch_create_roi": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "bj_batch_create_scaled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "bj_batch_create_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                          C.POINTER(C.c_void_p)]),
     "bj_batch_upload": (C.c_int, [C.c_void_p, C.c_void_p]),
     "bj_batch_decode": (C.c_int, [C.c_void_p, C.c_void_p]),
     "bj_batch_sync": (C.c_int, [C.c_void_p]),

@@ -195,7 +195,7 @@ extern "C" int bj_get_stat(const bj_ctx *c, const char *name, double *value) {
     // host_ms: parse + layout + pack, wait_ms: host blocked on the GPU; ms_*: kernel time per stage, summed over the
     // sub-batches (CUDA events) - the reference's per-stage "Profiles" lines (src/decoder_host.cpp:379-394)
     static const char *const names[ST_COUNT] = {"sub_batches", "launches", "h2d_bytes", "d2h_bytes", "host_ms", "wait_ms", "d2h_copies",
-                                                "ms_unstuff", "ms_sync", "ms_write", "ms_idct", "direct_uploads"};
+                                                "ms_unstuff", "ms_sync", "ms_write", "ms_idct", "direct_uploads", "ms_resize"};
     const struct { const char *prefix; const double *counters; } sets[] = {{"decode_batch_", c->stats}, {"total_", c->totals}};
     for (const auto &set : sets) {
         const size_t len = strlen(set.prefix);
@@ -285,6 +285,15 @@ extern "C" size_t bj_scaled_output_size(const bj_image_desc *d, const bj_roi *ro
     return output_bytes(*d, format, 100, &r, (uint32_t)scale);
 }
 
+extern "C" size_t bj_resized_output_size(const bj_image_desc *d, const bj_roi *roi, int scale, const bj_size *size, int format) {
+    const int kind = resize_kind(size);
+    if (kind == 0) return bj_scaled_output_size(d, roi, scale, format);
+    bj_roi r{};
+    if (!d || (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP) || scale <= 0 || !roi_rect(*d, roi, (uint32_t)scale, &r) || kind < 0) return 0;
+    if ((uint64_t)size->w * size->h > kDefaultMaxImagePixels) return 0;   // (no context here: the option's default)
+    return output_bytes(*d, format, 100, &r, (uint32_t)scale, size);
+}
+
 extern "C" size_t bj_roi_output_size(const bj_image_desc *d, const bj_roi *roi, int format) { return bj_scaled_output_size(d, roi, 1, format); }
 
 extern "C" size_t bj_ref_mcus_size(const bj_image_desc *d, int max_mcu_per_dpu, int *nchunks) {
@@ -327,17 +336,22 @@ extern "C" int bj_stage_idct_color(bj_ctx *c, const bj_image_desc *desc, const i
 
 // ------------------------------------------------------------------------------------------------ full path, staged
 
-extern "C" int bj_batch_create_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales, int n,
-                                      int format, bj_batch **out) {
+extern "C" int bj_batch_create_resized(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
+                                       const bj_size *sizes, int n, int format, bj_batch **out) {
     if (!c || !out || n < 0 || (n > 0 && (!files || !lens))) return BJ_ERR_ARG;
-    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
+    if ((rois || scales || sizes) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     *out = nullptr;
     bj_batch *b = new (std::nothrow) bj_batch();
     if (!b) return BJ_ERR_NOMEM;
-    const int rc = batch_assign(b, c->devs[0], files, lens, n, format, ~(size_t)0, nullptr, nullptr, rois, scales);     // a staged batch lives on one device
+    const int rc = batch_assign(b, c->devs[0], files, lens, n, format, ~(size_t)0, nullptr, nullptr, rois, scales, sizes);     // a staged batch lives on one device
     if (rc != BJ_OK) { b->release(); delete b; return rc; }
     *out = b;
     return BJ_OK;
+}
+
+extern "C" int bj_batch_create_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales, int n,
+                                      int format, bj_batch **out) {
+    return bj_batch_create_resized(c, files, lens, rois, scales, nullptr, n, format, out);
 }
 
 extern "C" int bj_batch_create_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format, bj_batch **out) {
@@ -476,6 +490,7 @@ struct CallInput {                       // what a call decodes: files, or (bj_d
     const bj_image_desc *descs; const int *kinds;
     const bj_roi *rois;                  // (the _roi / _scaled entries) a crop per image; nullptr: whole images
     const uint8_t *scales;               // (the _scaled entries) a scale denominator per image; nullptr: all 1
+    const bj_size *sizes;                // (the _resized entries) a target size per image; nullptr: none resized
 };
 
 // One device's share of a call: pull ranges from `src` until it runs dry.  st[ST_COUNT]: this device's counters.
@@ -506,7 +521,7 @@ static int decode_worker(Device *dev, RangeSource *src, const CallInput &in, int
             float k0 = 0, k1 = 0, out = 0;
             cudaEventSynchronize(b->ev[5]);
             cudaEventElapsedTime(&k0, ev_base, b->ev[0]);
-            cudaEventElapsedTime(&k1, ev_base, b->ev[4]); cudaEventElapsedTime(&out, ev_base, b->ev[5]);
+            cudaEventElapsedTime(&k1, ev_base, b->ev[b->n_rtiles ? 6 : 4]); cudaEventElapsedTime(&out, ev_base, b->ev[5]);
             fprintf(stderr, "b200jpeg trace: dev %d sub-batch of %4d images (%6.1f MB out, %s)  host prepare %6.2f..%6.2f  kernels %6.2f..%6.2f  copied out %6.2f\n",
                     dev->ordinal, b->n, b->d2h_bytes / 1e6, b->direct_src ? "direct upload" : "staged upload", host_t[slot][0], host_t[slot][1], k0, k1, out);
         }
@@ -515,7 +530,7 @@ static int decode_worker(Device *dev, RangeSource *src, const CallInput &in, int
         st[ST_WAIT_MS] += wall_ms() - t0;
         if (status) for (int i = 0; i < count[slot]; i++) status[first[slot] + i] = r == BJ_OK ? batch_image_status(b, i) : r;
         st[ST_LAUNCH] += b->launches; st[ST_H2D] += (double)(b->files_bytes + b->meta_bytes); st[ST_D2H] += (double)b->d2h_bytes; st[ST_D2H_COPIES] += b->d2h_copies;
-        if (r == BJ_OK) { st[ST_MS_UNSTUFF] += b->ms_unstuff; st[ST_MS_SYNC] += b->ms_sync; st[ST_MS_WRITE] += b->ms_write; st[ST_MS_IDCT] += b->ms_idct; }
+        if (r == BJ_OK) { st[ST_MS_UNSTUFF] += b->ms_unstuff; st[ST_MS_SYNC] += b->ms_sync; st[ST_MS_WRITE] += b->ms_write; st[ST_MS_IDCT] += b->ms_idct; st[ST_MS_RESIZE] += b->ms_resize; }
         busy[slot] = false;
         return r;
     };
@@ -531,7 +546,7 @@ static int decode_worker(Device *dev, RangeSource *src, const CallInput &in, int
             cudaStream_t s = dev->streams[slot];
             const double t0 = wall_ms();
             rc = batch_assign(b, dev, files + i0, lens + i0, r1 - i0, format, c->sub_batch_out_bytes, in.descs ? in.descs + i0 : nullptr, in.kinds ? in.kinds + i0 : nullptr,
-                           in.rois ? in.rois + i0 : nullptr, in.scales ? in.scales + i0 : nullptr);
+                           in.rois ? in.rois + i0 : nullptr, in.scales ? in.scales + i0 : nullptr, in.sizes ? in.sizes + i0 : nullptr);
             const int m = rc == BJ_OK ? b->n : 0;
             st[ST_HOST_MS] += wall_ms() - t0;
             host_t[slot][0] = t0 - wall0; host_t[slot][1] = wall_ms() - wall0;
@@ -581,7 +596,7 @@ static int decode_batch_now(bj_ctx *c, const CallInput &in, int n, int format, u
     for (auto &t : th) t.join();
     // the devices work side by side: counts add up, a time is the longest device's
     for (int i = 0; i < ST_COUNT; i++) {
-        const bool is_time = i == ST_HOST_MS || i == ST_WAIT_MS || (i >= ST_MS_UNSTUFF && i <= ST_MS_IDCT);
+        const bool is_time = i == ST_HOST_MS || i == ST_WAIT_MS || (i >= ST_MS_UNSTUFF && i <= ST_MS_IDCT) || i == ST_MS_RESIZE;
         double v = st[i];
         for (size_t d = 1; d < nd; d++) v = is_time ? std::max(v, st[d * ST_COUNT + i]) : v + st[d * ST_COUNT + i];
         c->stats[i] = v; c->totals[i] += v;
@@ -590,13 +605,18 @@ static int decode_batch_now(bj_ctx *c, const CallInput &in, int n, int format, u
     return BJ_OK;
 }
 
-extern "C" int bj_decode_batch_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
-                                      int n, int format, uint8_t *const *outs, int *status) {
+extern "C" int bj_decode_batch_resized(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
+                                       const bj_size *sizes, int n, int format, uint8_t *const *outs, int *status) {
     if (!c || n < 0 || (n > 0 && (!files || !lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
-    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;            // the reference's tile buffers have no crop or scale
+    if ((rois || scales || sizes) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;   // the reference's tile buffers have no crop, scale or size
     if (c->async && c->async->pending()) return BJ_ERR_ARG;                          // jobs of bj_submit are still running on this context
-    return decode_batch_now(c, CallInput{files, lens, nullptr, nullptr, rois, scales}, n, format, outs, status);
+    return decode_batch_now(c, CallInput{files, lens, nullptr, nullptr, rois, scales, sizes}, n, format, outs, status);
+}
+
+extern "C" int bj_decode_batch_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
+                                      int n, int format, uint8_t *const *outs, int *status) {
+    return bj_decode_batch_resized(c, files, lens, rois, scales, nullptr, n, format, outs, status);
 }
 
 extern "C" int bj_decode_batch_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,
@@ -617,7 +637,7 @@ extern "C" int bj_decode_batch_desc(bj_ctx *c, const bj_image_desc *descs, const
     if (!c || n < 0 || (n > 0 && (!descs || !scans || !scan_lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     if (c->async && c->async->pending()) return BJ_ERR_ARG;
-    return decode_batch_now(c, CallInput{scans, scan_lens, descs, scan_kinds, nullptr, nullptr}, n, format, outs, status);
+    return decode_batch_now(c, CallInput{scans, scan_lens, descs, scan_kinds, nullptr, nullptr, nullptr}, n, format, outs, status);
 }
 
 // ------------------------------------------------------------------------------------------------ full path, asynchronous
@@ -626,7 +646,7 @@ extern "C" int bj_decode_batch_desc(bj_ctx *c, const bj_image_desc *descs, const
 // the queue between them (src/decoder_host.cpp:25-38,364-365) a caller gets by submitting batch k+1 (or reading its
 // files) while batch k decodes, and writing batch k-1's outputs meanwhile (host/decoder_b200.cpp does exactly that).
 struct bj_job {
-    const uint8_t *const *files; const size_t *lens; const bj_roi *rois; const uint8_t *scales; int n, format; uint8_t *const *outs; int *status;
+    const uint8_t *const *files; const size_t *lens; const bj_roi *rois; const uint8_t *scales; const bj_size *sizes; int n, format; uint8_t *const *outs; int *status;
     int rc = BJ_OK;
     bool done = false;
     bj_ctx *ctx = nullptr;
@@ -641,7 +661,7 @@ void bj::AsyncWorker::run() {
             if (q.empty()) return;
             j = q.front();
         }
-        const int rc = decode_batch_now(j->ctx, CallInput{j->files, j->lens, nullptr, nullptr, j->rois, j->scales}, j->n, j->format, j->outs, j->status);
+        const int rc = decode_batch_now(j->ctx, CallInput{j->files, j->lens, nullptr, nullptr, j->rois, j->scales, j->sizes}, j->n, j->format, j->outs, j->status);
         {
             std::lock_guard<std::mutex> l(m);
             q.pop_front();
@@ -651,13 +671,13 @@ void bj::AsyncWorker::run() {
     }
 }
 
-extern "C" int bj_submit_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales, int n,
-                                int format, uint8_t *const *outs, int *status, bj_job **job) {
+extern "C" int bj_submit_resized(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales,
+                                 const bj_size *sizes, int n, int format, uint8_t *const *outs, int *status, bj_job **job) {
     if (!c || !job || n < 0 || (n > 0 && (!files || !lens || !outs))) return BJ_ERR_ARG;
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
-    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
+    if ((rois || scales || sizes) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
     *job = nullptr;
-    bj_job *j = new (std::nothrow) bj_job{files, lens, rois, scales, n, format, outs, status};
+    bj_job *j = new (std::nothrow) bj_job{files, lens, rois, scales, sizes, n, format, outs, status};
     if (!j) return BJ_ERR_NOMEM;
     j->ctx = c;
     if (!c->async) {
@@ -669,6 +689,11 @@ extern "C" int bj_submit_scaled(bj_ctx *c, const uint8_t *const *files, const si
     c->async->cv.notify_one();
     *job = j;
     return BJ_OK;
+}
+
+extern "C" int bj_submit_scaled(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, const uint8_t *scales, int n,
+                                int format, uint8_t *const *outs, int *status, bj_job **job) {
+    return bj_submit_resized(c, files, lens, rois, scales, nullptr, n, format, outs, status, job);
 }
 
 extern "C" int bj_submit_roi(bj_ctx *c, const uint8_t *const *files, const size_t *lens, const bj_roi *rois, int n, int format,

@@ -14,6 +14,7 @@
 #include "bj_host.h"
 #include "kernels_huff.cuh"
 #include "kernels_idct.cuh"
+#include "kernels_resize.cuh"
 #include "parse.h"
 
 namespace bj {
@@ -64,13 +65,15 @@ struct bj_batch {
     std::vector<uint32_t> du_base, ndu;
     std::vector<bj::HuffImg> himg;       // per-image records (kept here between calls: no reallocation in steady state)
     std::vector<bj::ImgDev> idev;
+    std::vector<bj::ResizeDev> rsz;      // fixed-size output: one record per resized image ...
+    std::vector<uint32_t> rtile0;        // ... and the prefix of their output tile counts (k_resize_bilinear's map)
 
     // host staging (pinned): file bytes; descriptor blob; results
     bj::PinBuf h_files, h_meta, h_res;
     size_t files_bytes = 0, meta_bytes = 0;
     const uint8_t *direct_src = nullptr;   // set: the files are uploaded straight from the caller's (pinned) memory, files_bytes from here
     // offsets inside the descriptor blob (host -> device)
-    size_t o_himg = 0, o_idev = 0, o_qtab = 0, o_lutdc = 0, o_lutac = 0, o_lutacs = 0;
+    size_t o_himg = 0, o_idev = 0, o_qtab = 0, o_lutdc = 0, o_lutac = 0, o_lutacs = 0, o_rsz = 0, o_rtile = 0;
     // offsets inside the map buffer (written on the device by k_expand_maps)
     size_t m_tiles = 0, m_blk = 0, m_wblk = 0, m_utile = 0, m_dcc = 0, maps_bytes = 0;
     uint32_t idct_smem = 0;             // dynamic shared memory of k_idct_color: sized for the widest pixel tile of this batch
@@ -80,20 +83,22 @@ struct bj_batch {
     size_t n_slice_slots = 0;
     uint32_t n_idct_tiles = 0, n_blk = 0, n_utile = 0, n_dcc = 0, n_seg_entries = 0, n_sub_slots = 0, lut_smem = 0;
     size_t clean_words = 0, coef_units = 0, out_bytes = 0;
+    size_t inter_off = 0, inter_bytes = 0;   // fixed-size output: the resize sources (RGB8 scaled crops) in d_out, behind the final outputs
+    uint32_t n_rsz = 0, n_rtiles = 0;        // resized images, CTAs of k_resize_bilinear
     uint64_t pixels = 0, scan_bytes_max = 0;
     uint32_t nseg_max = 0;              // most restart segments of one image
     uint32_t ref_blocks_max = 0;        // BJ_OUT_REF_MCUS: blocks of the largest image (grid of the padding kernel)
 
     // device
     bj::DevBuf d_files, d_meta, d_maps, d_look, d_clean, d_seg, d_subseg, d_stin, d_stout, d_tot, d_pre, d_slice, d_quarter, d_blkagg, d_state, d_flags, d_coef, d_dc, d_dcagg, d_out;
-    cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // start, un-stuffed, synchronised, written, pixels, copied out
+    cudaEvent_t ev[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // start, un-stuffed, synchronised, written, pixels, copied out, resized
     cudaEvent_t ev_done = nullptr;       // one-call path: recorded behind the copy-out, created for a sleeping wait
     cudaStream_t last_stream = nullptr;
     bool uploaded = false, decoded = false, synced = false;
     bool multi_blk = false;              // some image's sub-sequences span more than one CTA of the synchronisation pass
     bool redone = false;                 // batch_sync had to run extra fix-up rounds: everything after them was computed again
     uint32_t launches = 0, sync_rounds = 0;
-    float ms_entropy = 0.f, ms_idct = 0.f, ms_unstuff = 0.f, ms_sync = 0.f, ms_write = 0.f;
+    float ms_entropy = 0.f, ms_idct = 0.f, ms_unstuff = 0.f, ms_sync = 0.f, ms_write = 0.f, ms_resize = 0.f;
     uint64_t d2h_bytes = 0;
     uint32_t d2h_copies = 0;
 
@@ -128,10 +133,15 @@ constexpr int kMaxRounds = 64;
 //   scales    scaled by 1 / scales[i] (the _scaled entries; 1, 2, 4 or 8): a scale other than those, or a ROI that does not
 //             fit the scaled image, gives that image BJ_ERR_ARG; output sizes, offsets and out_cap count the bytes of the
 //             scaled crop.
+//   sizes     (the _resized entries) resized to sizes[i] (bj_size; {0,0}: not resized): a refused size gives that image
+//             BJ_ERR_ARG, one above max_image_pixels BJ_ERR_UNSUPPORTED.  The IDCT + colour stage writes a resized
+//             image's scaled crop as RGB8 into the intermediate region behind the final outputs, k_resize_bilinear reads
+//             it from there.  Output sizes and offsets count the final output; out_cap counts it plus the intermediate.
 inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, const size_t *lens, int n, int format, size_t out_cap = ~(size_t)0,
-                        const bj_image_desc *descs = nullptr, const int *kinds = nullptr, const bj_roi *rois = nullptr, const uint8_t *scales = nullptr) {
+                        const bj_image_desc *descs = nullptr, const int *kinds = nullptr, const bj_roi *rois = nullptr, const uint8_t *scales = nullptr,
+                        const bj_size *sizes = nullptr) {
     if (format != BJ_OUT_RGB8 && format != BJ_OUT_BMP && format != BJ_OUT_REF_MCUS) return BJ_ERR_ARG;
-    if ((rois || scales) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;            // the reference's tile buffers have no crop or scale
+    if ((rois || scales || sizes) && format == BJ_OUT_REF_MCUS) return BJ_ERR_ARG;   // the reference's tile buffers have no crop, scale or size
     const bj_ctx *c = dev->ctx;
     b->dev = dev; b->n = n; b->format = format;
     b->uploaded = b->decoded = b->synced = false;
@@ -159,16 +169,26 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
             if (rc == BJ_OK && (size_t)d.width * d.height > c->max_image_pixels) rc = BJ_ERR_UNSUPPORTED;   // (the full image: its whole scan is decoded)
             bj_roi r{};
             if (rc == BJ_OK && (rois || scales) && !roi_rect(d, rois ? &rois[i] : nullptr, scales ? scales[i] : 1u, &r)) rc = BJ_ERR_ARG;
+            if (rc == BJ_OK && sizes && resize_kind(&sizes[i]) < 0) rc = BJ_ERR_ARG;
+            if (rc == BJ_OK && sizes && (size_t)sizes[i].w * sizes[i].h > c->max_image_pixels) rc = BJ_ERR_UNSUPPORTED;   // (a tiny request must not claim GBs of output)
             if (rc == BJ_OK) geo[i] = geometry_of(d);
             b->parse_status[i] = rc;
         }
     });
+    // the target size of image i, nullptr if it is not resized
+    auto size_of = [&](int i) -> const bj_size * { return sizes && resize_kind(&sizes[i]) > 0 ? &sizes[i] : nullptr; };
     // ---- how many of the candidates this batch takes
     if (out_cap != ~(size_t)0) {
         size_t acc = 0;
         int m = 0;
         while (m < n) {
-            const size_t sz = b->parse_status[m] == BJ_OK ? align_up(output_bytes(b->desc[m], format, c->ref_m, rois ? &rois[m] : nullptr, scales ? scales[m] : 1u), 16) : 0;
+            const bj_roi *roi = rois ? &rois[m] : nullptr;
+            const uint32_t scale = scales ? scales[m] : 1u;
+            size_t sz = 0;
+            if (b->parse_status[m] == BJ_OK) {
+                sz = align_up(output_bytes(b->desc[m], format, c->ref_m, roi, scale, size_of(m)), 16);
+                if (size_of(m)) sz += align_up(output_bytes(b->desc[m], BJ_OUT_RGB8, c->ref_m, roi, scale), 16);   // (the resize's source)
+            }
             if (m > 0 && acc + sz > out_cap) break;
             acc += sz; m++;
         }
@@ -261,6 +281,9 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     uint32_t seg_entries = 0, nblk = 0, n_utile = 0, n_wblk = 0, n_dcc = 0, n_tiles = 0;
     int prev = -1;                                  // last valid image: its table slots are reused when the tables match
     b->pixels = 0; b->scan_bytes_max = 0; b->ref_blocks_max = 0; b->nseg_max = 0; b->lut_smem = 0; b->multi_blk = false; b->scaled = false;
+    b->rsz.clear(); b->rtile0.clear();
+    size_t inter_bytes = 0;                         // the resize sources, offsets from the intermediate region's start
+    uint64_t n_rtiles = 0;
     uint32_t rgb_max = 0;
     auto same_tables = [](const bj_image_desc &a, const bj_image_desc &q) {
         if (a.ncomp != q.ncomp || memcmp(a.dc_id, q.dc_id, 3) || memcmp(a.ac_id, q.ac_id, 3)) return false;
@@ -372,9 +395,18 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         coef_units += g.ndu;
         const bj_roi *roi = rois ? &rois[i] : nullptr;
         const uint32_t scale = scales ? scales[i] : 1u;
-        b->out_size[i] = output_bytes(d, format, c->ref_m, roi, scale);
+        const bj_size *size = size_of(i);
+        b->out_size[i] = output_bytes(d, format, c->ref_m, roi, scale, size);
         b->out_off[i] = out_bytes;
-        fill_imgdev(d, g, format, hi.du_base, out_bytes, &idev[i], roi, scale);
+        if (size) {                                 // the IDCT + colour stage writes the scaled crop as RGB8 (moved behind the final outputs below)
+            fill_imgdev(d, g, BJ_OUT_RGB8, hi.du_base, inter_bytes, &idev[i], roi, scale);
+            b->rsz.emplace_back();
+            fill_resize(*size, format, out_bytes, idev[i], &b->rsz.back());
+            b->rtile0.push_back((uint32_t)n_rtiles);
+            n_rtiles += resize_tile_count(*size);
+            inter_bytes += align_up(output_bytes(d, BJ_OUT_RGB8, c->ref_m, roi, scale), 16);
+        } else
+            fill_imgdev(d, g, format, hi.du_base, out_bytes, &idev[i], roi, scale);
         if (scale != 1) b->scaled = true;
         if (format == BJ_OUT_REF_MCUS) { idev[i].ref_blocks = ref_mcus_chunks(d, c->ref_m) * (uint32_t)(c->ref_m / 4); b->ref_blocks_max = std::max(b->ref_blocks_max, idev[i].ref_blocks); }
         idev[i].dc_sep = 1;
@@ -387,8 +419,13 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         rgb_max = std::max<uint32_t>(rgb_max, std::min<uint32_t>(g.tile_mcus, g.nmx) * d.hs * 8u * d.vs * 8u * 3u);
         b->pixels += (uint64_t)d.width * d.height;
         b->scan_bytes_max += d.scan_len;
-        if (coef_units > 0xFFFFFFF0ull || clean_words > 0xFFFFFFF0ull || slice_slots > 0xFFFFFFF0ull) return BJ_ERR_ARG;   // split the batch
+        if (coef_units > 0xFFFFFFF0ull || clean_words > 0xFFFFFFF0ull || slice_slots > 0xFFFFFFF0ull || n_rtiles > 0x7FFFFFFFull) return BJ_ERR_ARG;   // split the batch
     }
+    // ---- the intermediate region: behind the final outputs, so that the copy-out's runs never include it
+    b->inter_off = align_up(out_bytes, 256); b->inter_bytes = inter_bytes;
+    for (int i = 0; i < n; i++) if (b->parse_status[i] == BJ_OK && size_of(i)) idev[i].out_row0 += b->inter_off;
+    for (ResizeDev &rz : b->rsz) rz.src_off += b->inter_off;
+    b->n_rsz = (uint32_t)b->rsz.size(); b->n_rtiles = (uint32_t)n_rtiles;
     b->idct_smem = kSmemDu + kSmemQ + kRgbFront + std::min<uint32_t>(rgb_max, kRgbMax) + 64;
     b->files_bytes = b->direct_src ? (size_t)(span_hi - span_lo) : fbytes + 64; b->clean_words = clean_words + 96; b->coef_units = coef_units; b->out_bytes = out_bytes;   // (96 words of slack: a damaged unit is read to its end, up to 63 symbols of 27 bits past the data)
     b->n_wblk = n_wblk; b->n_slice_slots = slice_slots;
@@ -403,6 +440,8 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     b->o_lutdc = o; o = align_up(o + luts_dc.size() * 4, 256);
     b->o_lutac = o; o = align_up(o + luts_ac.size() * 4, 256);
     b->o_lutacs = o; o = align_up(o + luts_acs.size() * 4, 256);
+    b->o_rsz = o;   o = align_up(o + b->rsz.size() * sizeof(ResizeDev), 256);
+    b->o_rtile = o; o = align_up(o + b->rtile0.size() * 4, 256);
     b->meta_bytes = o;
     // ---- map buffer (device only: k_expand_maps)
     o = 0;
@@ -419,6 +458,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     if (!luts_dc.empty()) memcpy(b->hmeta<uint32_t>(b->o_lutdc), luts_dc.data(), luts_dc.size() * 4);
     if (!luts_ac.empty()) memcpy(b->hmeta<uint32_t>(b->o_lutac), luts_ac.data(), luts_ac.size() * 4);
     if (!luts_acs.empty()) memcpy(b->hmeta<uint32_t>(b->o_lutacs), luts_acs.data(), luts_acs.size() * 4);
+    if (!b->rsz.empty()) { memcpy(b->hmeta<ResizeDev>(b->o_rsz), b->rsz.data(), b->rsz.size() * sizeof(ResizeDev)); memcpy(b->hmeta<uint32_t>(b->o_rtile), b->rtile0.data(), b->rtile0.size() * 4); }
     // ---- stage the file bytes (only when they cannot go up from where they are; per image, independent: worker pool)
     if (!b->direct_src) {
         uint8_t *hf = reinterpret_cast<uint8_t *>(b->h_files.p);
@@ -440,7 +480,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         b->d_dc.reserve(coef_units * 2 + 64) || b->d_dcagg.reserve((size_t)b->n_dcc * sizeof(DcAgg) + 16) ||
         b->d_blkagg.reserve((size_t)nblk * sizeof(BlkAgg) + 16) ||
         b->d_state.reserve((size_t)n * sizeof(HuffImgState) + 16) || b->d_flags.reserve(kMaxRounds * 4 + 16) ||
-        b->d_coef.reserve(coef_units * 128 + 16) || b->d_out.reserve(out_bytes + 64)) return BJ_ERR_NOMEM;
+        b->d_coef.reserve(coef_units * 128 + 16) || b->d_out.reserve(b->inter_off + inter_bytes + 64)) return BJ_ERR_NOMEM;
     return BJ_OK;
 }
 
@@ -490,7 +530,7 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
         if (c->debug_poison) {                                                        // tests: whatever is read later must have been written by this decode
             cudaMemsetAsync(b->d_coef.p, 0xA5, b->coef_units * 128, s);
             cudaMemsetAsync(b->d_dc.p, 0xA5, b->coef_units * 2, s);
-            cudaMemsetAsync(b->d_out.p, 0xA5, b->out_bytes, s);
+            cudaMemsetAsync(b->d_out.p, 0xA5, b->inter_bytes ? b->inter_off + b->inter_bytes : b->out_bytes, s);   // (the resize sources included)
             cudaMemsetAsync(b->d_clean.p, 0xA5, b->clean_words * 4, s);
         }
         cudaMemsetAsync(flags, 0, kMaxRounds * 4, s);
@@ -549,6 +589,11 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
         b->launches++;
     }
     cudaEventRecord(b->ev[4], s);
+    if (b->n_rtiles) {                                                                // fixed-size output: only when some image is resized
+        k_resize_bilinear<<<b->n_rtiles, kTileThreads, 0, s>>>(b->dmeta<ResizeDev>(b->o_rsz), b->dmeta<uint32_t>(b->o_rtile), (int)b->n_rsz, (uint8_t *)b->d_out.p);
+        b->launches++;
+        cudaEventRecord(b->ev[6], s);                                                 // (no event otherwise: the whole-image path records what it did before)
+    }
     cudaMemcpyAsync(b->h_state(), st, (size_t)n * sizeof(HuffImgState), cudaMemcpyDeviceToHost, s);
     cudaMemcpyAsync(b->h_flags(), flags, kMaxRounds * 4, cudaMemcpyDeviceToHost, s);
     return b->dev->check(cudaGetLastError());
@@ -592,6 +637,8 @@ inline int batch_sync(bj_batch *b) {
         cudaEventElapsedTime(&b->ms_sync, b->ev[1], b->ev[2]);        // (only the last group of rounds if extra ones ran)
         cudaEventElapsedTime(&b->ms_write, b->ev[2], b->ev[3]);
         cudaEventElapsedTime(&b->ms_idct, b->ev[3], b->ev[4]);
+        b->ms_resize = 0.f;
+        if (b->n_rtiles) cudaEventElapsedTime(&b->ms_resize, b->ev[4], b->ev[6]);
         b->synced = true;
     }
     return rc;

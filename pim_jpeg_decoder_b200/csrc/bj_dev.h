@@ -6,6 +6,8 @@ namespace bj {
 
 constexpr int kTileThreads = 192;     // K2/K3 CTA size = data units per tile (192 = lcm-friendly for bpm 1,2,3,4,6)
 constexpr int kQPitch = 68;           // words between per-component dequant tables in smem (bank skew, 16 B aligned)
+constexpr int kResizeTileW = 64;      // k_resize_bilinear: output columns per tile, two per lane of a warp
+constexpr int kResizeTileH = 48;      // ... and output rows per tile, eight per warp of the kTileThreads-wide CTA
 
 // Per image: geometry + where its data lives.  Data units ("du") are 64 coefficients = 128 B, zig-zag order,
 // stored in decode order (MCU after MCU; inside an MCU: Y units row-major, then Cb, then Cr) - the order of
@@ -39,6 +41,19 @@ __host__ __device__ inline uint32_t idct_tiles_per_row(const ImgDev &im) {
     return ((uint32_t)im.mx_hi - im.mx_lo + tile_mcus - 1) / tile_mcus;
 }
 __host__ __device__ inline uint32_t idct_tile_count(const ImgDev &im) { return ((uint32_t)im.my_hi - im.my_lo) * idct_tiles_per_row(im); }
+
+// Fixed-size output: one record per image of a batch that is resized (k_resize_bilinear, kernels_resize.cuh).  The
+// source is the image's scaled crop, which the IDCT + colour kernel wrote as RGB8 (top-down, sw * 3 bytes per row) into
+// the intermediate region of the batch output buffer; the output record is laid out as an image of w x h pixels whose
+// crop window is all of it and whose MCU window starts at 0, so that tile_copy_out writes it unchanged and the output
+// tile (0, 0) is the one that writes a BMP header.
+struct ResizeDev {
+    ImgDev out;                   // the final output: width x height = cw x ch = w x h, the format's layout
+    uint64_t src_off;             // byte offset of the source's pixel (0, 0) in the batch output buffer
+    uint32_t sw, sh;              // source size: the scaled crop's cw x ch
+    uint32_t tiles_x;             // output tiles per row (kResizeTileW columns each)
+    uint32_t pad_;
+};
 
 // One set of quantisation tables as the K2 kernel stages it: per component (quantiser << 16) in ZIG-ZAG (file) order.
 struct QTab {

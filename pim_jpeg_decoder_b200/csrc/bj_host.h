@@ -123,11 +123,12 @@ public:
 inline PinnedRanges &pinned_ranges() { static PinnedRanges r; return r; }
 
 constexpr int kSlots = 3;             // sub-batches in flight inside bj_decode_batch
+constexpr size_t kDefaultMaxImagePixels = (size_t)1 << 28;   // option "max_image_pixels"
 
 enum { POOL_COMPAT_MD = 0, POOL_COMPAT_MCUS, POOL_COEF, POOL_OUT, POOL_IMGS, POOL_TILES, POOL_COUNT };
 
 // counters of one bj_decode_batch / job (bj_get_stat: "decode_batch_<name>", "total_<name>")
-enum { ST_SUB = 0, ST_LAUNCH, ST_H2D, ST_D2H, ST_HOST_MS, ST_WAIT_MS, ST_D2H_COPIES, ST_MS_UNSTUFF, ST_MS_SYNC, ST_MS_WRITE, ST_MS_IDCT, ST_DIRECT, ST_COUNT };
+enum { ST_SUB = 0, ST_LAUNCH, ST_H2D, ST_D2H, ST_HOST_MS, ST_WAIT_MS, ST_D2H_COPIES, ST_MS_UNSTUFF, ST_MS_SYNC, ST_MS_WRITE, ST_MS_IDCT, ST_DIRECT, ST_MS_RESIZE, ST_COUNT };
 
 }  // namespace bj
 
@@ -160,7 +161,7 @@ struct bj_ctx {
                                          // (bj_host_alloc / bj_host_register), 1 = the caller says it is, -1 = always stage
     int ref_m = 100;                     // BJ_OUT_REF_MCUS: MAX_MCU_PER_DPU of the host that reads the buffer (Makefile:2 of the reference)
     int debug_poison = 0;                // fill coefficient / DC / output buffers with 0xA5 before every decode (tests: every byte must be written)
-    size_t max_image_pixels = (size_t)1 << 28;   // larger images are refused (BJ_ERR_UNSUPPORTED), like the reference's "Too high resolution"
+    size_t max_image_pixels = bj::kDefaultMaxImagePixels;   // larger images are refused (BJ_ERR_UNSUPPORTED), like the reference's "Too high resolution"
     size_t sub_batch_out_bytes = (size_t)1 << 30; // decoded bytes per sub-batch of bj_decode_batch
     int sync_rounds = 0;                 // 0 = default (3 launches of the fix-up kernel before the first check)
     std::vector<bj::Device *> devs;      // never empty; staged and stage-level entries run on devs[0]
@@ -238,6 +239,25 @@ inline void set_crop(const bj_roi &r, int scale_log2, ImgDev *im) {
     im->my_lo = (uint16_t)(y_lo / mh); im->my_hi = (uint16_t)((y_hi + mh - 1) / mh);
 }
 
+// The output layout of a w x h image in the RGB8 or BMP format whose first byte is at out_base: the fields of the
+// image record the copy-out reads (tile_copy_out).  Shared by the IDCT + colour stage's records and the resize records.
+inline void set_layout(int format, uint32_t w, uint32_t h, uint64_t out_base, ImgDev *im) {
+    im->row_bytes = w * 3;
+    if (format == BJ_OUT_BMP) {
+        im->row_pad = w % 4;
+        im->out_pitch = w * 3 + im->row_pad;
+        im->out_row0 = out_base + 26 + (uint64_t)(h - 1) * im->out_pitch;
+        im->row_dir = -1;
+        im->bgr = 1;
+    } else {
+        im->row_pad = 0;
+        im->out_pitch = w * 3;
+        im->out_row0 = out_base;
+        im->row_dir = 1;
+        im->bgr = 0;
+    }
+}
+
 // out_base: byte offset of this image's output inside the batch output buffer.  roi, scale: a request roi_rect accepted
 // (nullptr, 1: the whole image; BJ_OUT_REF_MCUS always takes the whole image at full size).
 inline void fill_imgdev(const bj_image_desc &d, const Geometry &g, int format, uint32_t du_base, uint64_t out_base, ImgDev *im,
@@ -252,23 +272,35 @@ inline void fill_imgdev(const bj_image_desc &d, const Geometry &g, int format, u
     bj_roi r{};
     roi_rect(d, roi, scale, &r);
     set_crop(r, scale_log2_of(scale), im);
-    im->row_bytes = r.w * 3;
     if (format == BJ_OUT_REF_MCUS) {
+        im->row_bytes = r.w * 3;
         im->row_pad = 0; im->out_pitch = 0; im->row_dir = 1; im->bgr = 0;
         im->out_row0 = out_base;                       // byte offset of the image's first chunk
-    } else if (format == BJ_OUT_BMP) {
-        im->row_pad = r.w % 4;
-        im->out_pitch = r.w * 3 + im->row_pad;
-        im->out_row0 = out_base + 26 + (uint64_t)(r.h - 1) * im->out_pitch;
-        im->row_dir = -1;
-        im->bgr = 1;
-    } else {
-        im->row_pad = 0;
-        im->out_pitch = r.w * 3;
-        im->out_row0 = out_base;
-        im->row_dir = 1;
-        im->bgr = 0;
-    }
+    } else
+        set_layout(format, r.w, r.h, out_base, im);
+}
+
+// Fixed-size output: 0 when `size` asks for none (nullptr or {0,0}), 1 when it asks for a w x h output, -1 when it is
+// refused: only one of w, h is 0, or either is above 65535 (the BMP header holds 16-bit sizes).
+inline int resize_kind(const bj_size *size) {
+    if (!size || (size->w == 0 && size->h == 0)) return 0;
+    return (size->w == 0 || size->h == 0 || size->w > 65535u || size->h > 65535u) ? -1 : 1;
+}
+
+// The resize record of an image whose IDCT-stage record `src` (an RGB8 output of its scaled crop at src_off) is resized
+// to `size` (resize_kind 1) in `format` at out_base.
+inline void fill_resize(const bj_size &size, int format, uint64_t out_base, const ImgDev &src, ResizeDev *rz) {
+    memset(rz, 0, sizeof(*rz));
+    ImgDev &o = rz->out;
+    o.width = size.w; o.height = size.h; o.valid = 1;
+    o.cw = size.w; o.ch = size.h;                      // (cx = cy = 0, mx_lo = my_lo = 0: the tile at (0, 0) writes a BMP header)
+    set_layout(format, size.w, size.h, out_base, &o);
+    rz->src_off = src.out_row0;
+    rz->sw = src.cw; rz->sh = src.ch;
+    rz->tiles_x = (size.w + kResizeTileW - 1) / kResizeTileW;
+}
+inline uint32_t resize_tile_count(const bj_size &size) {
+    return ((size.w + kResizeTileW - 1) / kResizeTileW) * ((size.h + kResizeTileH - 1) / kResizeTileH);
 }
 
 // The image's quantiser set as the K2 kernel stages it.
@@ -307,15 +339,20 @@ inline uint32_t ref_mcus_chunks(const bj_image_desc &d, int M) {
     const uint32_t pw = (d.mcu_w_real + 1) / 2 * 2, ph = (d.mcu_h_real + 1) / 2 * 2;
     return (pw * ph + (uint32_t)M - 1) / (uint32_t)M;
 }
-// roi, scale: as for fill_imgdev (BJ_OUT_REF_MCUS ignores them)
-inline size_t output_bytes(const bj_image_desc &d, int format, int M, const bj_roi *roi = nullptr, uint32_t scale = 1) {
-    bj_roi r{};
-    roi_rect(d, roi, scale, &r);
-    const size_t w = r.w, h = r.h;
+// Bytes of a w x h image in the RGB8 or BMP format (0 for any other)
+inline size_t layout_bytes(int format, size_t w, size_t h) {
     if (format == BJ_OUT_RGB8) return w * h * 3;
     if (format == BJ_OUT_BMP) return 26 + h * (w * 3 + w % 4);
-    if (format == BJ_OUT_REF_MCUS) return (size_t)ref_mcus_chunks(d, M) * 64 * (size_t)M * 3 * sizeof(int16_t);
     return 0;
+}
+// roi, scale: as for fill_imgdev (BJ_OUT_REF_MCUS ignores them); size: a target size (resize_kind 1) or nullptr
+inline size_t output_bytes(const bj_image_desc &d, int format, int M, const bj_roi *roi = nullptr, uint32_t scale = 1,
+                           const bj_size *size = nullptr) {
+    if (format == BJ_OUT_REF_MCUS) return (size_t)ref_mcus_chunks(d, M) * 64 * (size_t)M * 3 * sizeof(int16_t);
+    if (size) return layout_bytes(format, size->w, size->h);
+    bj_roi r{};
+    roi_rect(d, roi, scale, &r);
+    return layout_bytes(format, r.w, r.h);
 }
 
 inline void append_tiles(const Geometry &g, uint32_t img, uint32_t du_base, std::vector<TileDev> *tiles) {

@@ -6,7 +6,8 @@
     pim.copy / pim.exec / pim.copy     (:276-308)          Decoder.exec_mcus(metadata, mcus)      [compat layout]
     read_JPEG                          (jpeg_scanner:345)  parse_header(bytes)
     decode_Huffman_data + exec + write_BMP gather          Decoder.decode(files, fmt) / Batch     [fast layout]
-    (a crop of each image: rois=, see roi_output_size; at 1/2, 1/4 or 1/8 size: scales=, see scaled_output_size)
+    (a crop of each image: rois=, see roi_output_size; at 1/2, 1/4 or 1/8 size: scales=, see scaled_output_size;
+    resized to a fixed size: sizes=, see resized_output_size and resize_plan)
     main(argv): sort by size, decode, write <name>.bmp     decode_files(paths)
 """
 import ctypes as C
@@ -49,6 +50,23 @@ def _scale_table(scales, n):
     return a, a.ctypes.data_as(C.c_void_p)
 
 
+def _size_table(sizes, n):
+    """sizes: None (no resize), one (w, h) for every image, or an (n, 2) array of them - each two whole numbers in
+    1..65535, or (0, 0) for no resize.  -> (keepalive uint32 (n, 2) array or None, pointer for the C ABI)"""
+    if sizes is None:
+        return None, None
+    v = np.asarray(sizes)
+    if v.dtype.kind not in "iuf":
+        raise TypeError(f"sizes must be numbers, not {v.dtype}")
+    v = np.broadcast_to(v, (n, 2)) if v.shape == (2,) else v.reshape(n, 2)
+    # a pair that is not two whole numbers in 1..65535 (nor (0, 0)) would wrap or truncate to some other size in the
+    # uint32 cast: it goes to the library as (1, 0), which refuses that image (BJ_ERR_ARG)
+    whole = (v == np.floor(v)) if v.dtype.kind == "f" else np.ones(v.shape, dtype=bool)
+    ok = ((v >= 1) & (v <= 65535) & whole).all(axis=1) | (v == 0).all(axis=1)
+    a = np.ascontiguousarray(np.where(ok[:, None], v, np.array([1, 0])).astype(np.uint32))
+    return a, a.ctypes.data_as(C.c_void_p)
+
+
 def roi_output_size(desc, roi, fmt=L.BJ_OUT_RGB8):
     """Output bytes of the image `desc` (ImageDesc) cropped to `roi` ((x, y, w, h), a Roi, or None for the whole image);
     0 if the ROI does not fit the image, and for BJ_OUT_REF_MCUS."""
@@ -64,6 +82,33 @@ def scaled_output_size(desc, roi, scale, fmt=L.BJ_OUT_RGB8):
     if roi is not None and not isinstance(roi, L.Roi):
         roi = L.Roi(*(int(v) for v in roi))
     return L.lib().bj_scaled_output_size(C.byref(desc), C.byref(roi) if roi is not None else None, int(scale), fmt)
+
+
+def resized_output_size(desc, roi, scale, size, fmt=L.BJ_OUT_RGB8):
+    """Output bytes of the image `desc` at 1/scale, cropped to `roi` (a rectangle of the scaled image, as for
+    scaled_output_size) and resized to `size` ((w, h), a Size, or None / (0, 0) for no resize); 0 for anything the
+    library refuses, and for BJ_OUT_REF_MCUS."""
+    if roi is not None and not isinstance(roi, L.Roi):
+        roi = L.Roi(*(int(v) for v in roi))
+    if size is not None and not isinstance(size, L.Size):
+        size = L.Size(*(int(v) for v in size))
+    return L.lib().bj_resized_output_size(C.byref(desc), C.byref(roi) if roi is not None else None, int(scale),
+                                          C.byref(size) if size is not None else None, fmt)
+
+
+def resize_plan(width, height, box, size):
+    """The request that turns the box (x, y, w, h) of a width x height image (None: all of it) into a (tw, th) output:
+    returns (scale, roi) for the scales= and rois= arguments.  The scale s is the largest of 8, 4, 2, 1 with
+    w >= s * tw and h >= s * th, so the bilinear stage reduces by less than 2x unless the box is more than 16 times the
+    target; the ROI is the box rounded outward onto the image scaled by 1/s (x // s, ceil((x + w) / s) - x // s, the
+    same for y), which always fits the scaled image."""
+    tw, th = (int(v) for v in size)
+    x, y, w, h = (0, 0, int(width), int(height)) if box is None else (int(v) for v in box)
+    if tw < 1 or th < 1 or w < 1 or h < 1 or x < 0 or y < 0 or x + w > width or y + h > height:
+        raise ValueError(f"resize_plan: box {box} of a {width}x{height} image to {size}")
+    s = next((s for s in (8, 4, 2) if w >= s * tw and h >= s * th), 1)
+    xs, ys = x // s, y // s
+    return s, (xs, ys, -(-(x + w) // s) - xs, -(-(y + h) // s) - ys)
 
 
 class PinnedBuffer:
@@ -101,16 +146,18 @@ def _file_arrays(files):
 class Batch:
     """A device-resident batch (bj_batch): upload -> decode -> download, each asynchronous on the context's stream.
     rois: None, or one (x, y, w, h) crop per image (see roi_output_size); scales: None, or a scale denominator for every
-    image or one per image (see scaled_output_size; a ROI is then a rectangle of the scaled image)."""
+    image or one per image (see scaled_output_size; a ROI is then a rectangle of the scaled image); sizes: None, or a
+    (w, h) target size for every image or one per image (see resized_output_size)."""
 
-    def __init__(self, dec, files, fmt=L.BJ_OUT_RGB8, rois=None, scales=None):
+    def __init__(self, dec, files, fmt=L.BJ_OUT_RGB8, rois=None, scales=None, sizes=None):
         self.dec = dec
         self.n = len(files)
         self._keep, ptrs, lens = _file_arrays(files)
         _, rp = _roi_table(rois, self.n)
         _, sp = _scale_table(scales, self.n)
+        _, zp = _size_table(sizes, self.n)
         self.h = C.c_void_p()
-        L.check(L.lib().bj_batch_create_scaled(dec.ctx, ptrs, lens, rp, sp, self.n, fmt, C.byref(self.h)), "bj_batch_create_scaled", dec.ctx)
+        L.check(L.lib().bj_batch_create_resized(dec.ctx, ptrs, lens, rp, sp, zp, self.n, fmt, C.byref(self.h)), "bj_batch_create_resized", dec.ctx)
         self.offsets, self.sizes, self.parse_status = [], [], []
         for i in range(self.n):
             off, nb = C.c_size_t(), C.c_size_t()
@@ -255,27 +302,29 @@ class Decoder:
         return out
 
     # ---- full path, one call (host buffers in, host buffers out)
-    def decode(self, files, fmt=L.BJ_OUT_RGB8, outs=None, rois=None, scales=None):
+    def decode(self, files, fmt=L.BJ_OUT_RGB8, outs=None, rois=None, scales=None, sizes=None):
         """Returns (list of uint8 arrays or None for rejected files, list of per-image status).  rois: None, or one
         (x, y, w, h) crop per image (see roi_output_size); scales: None, or a scale denominator (1, 2, 4, 8) for every
-        image or one per image (see scaled_output_size).  An image whose scale or ROI is refused gets BJ_ERR_ARG."""
+        image or one per image (see scaled_output_size); sizes: None, or a (w, h) target size for every image or one
+        per image (see resized_output_size).  An image whose scale, ROI or size is refused gets BJ_ERR_ARG."""
         n = len(files)
         keep, ptrs, lens = _file_arrays(files)
         ra, rp = _roi_table(rois, n)
         sa, sp = _scale_table(scales, n)
+        za, zp = _size_table(sizes, n)
         if outs is None:
             outs = []
             for i, f in enumerate(files):
                 st, d = parse_header(f)
                 size = 0
-                if st == L.BJ_OK and ra is None and sa is None:
-                    size = L.lib().bj_output_size(C.byref(d), fmt)          # (BJ_OUT_REF_MCUS included: it has no crop or scale)
+                if st == L.BJ_OK and ra is None and sa is None and za is None:
+                    size = L.lib().bj_output_size(C.byref(d), fmt)          # (BJ_OUT_REF_MCUS included: it has no crop, scale or size)
                 elif st == L.BJ_OK:
-                    size = scaled_output_size(d, None if ra is None else ra[i], 1 if sa is None else sa[i], fmt)
+                    size = resized_output_size(d, None if ra is None else ra[i], 1 if sa is None else sa[i], None if za is None else za[i], fmt)
                 outs.append(np.zeros(size, dtype=np.uint8) if size else None)
         optrs = (C.c_void_p * max(n, 1))(*[o.__array_interface__["data"][0] if o is not None else None for o in outs])
         status = (C.c_int * max(n, 1))()
-        L.check(L.lib().bj_decode_batch_scaled(self.ctx, ptrs, lens, rp, sp, n, fmt, optrs, status), "bj_decode_batch_scaled", self.ctx)
+        L.check(L.lib().bj_decode_batch_resized(self.ctx, ptrs, lens, rp, sp, zp, n, fmt, optrs, status), "bj_decode_batch_resized", self.ctx)
         st = list(status)[:n]
         return [o if s in (L.BJ_OK, L.BJ_ERR_CORRUPT_SCAN) else None for o, s in zip(outs, st)], st
 
@@ -297,11 +346,12 @@ class Decoder:
             outs = [o.view(np.int16) for o in outs]
         return outs, list(status)[:n]
 
-    def decode_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None, scales=None):
+    def decode_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None, scales=None, sizes=None):
         """bj_decode_batch for a batch-pipeline caller: the n files sit in ONE host buffer `src` (uint8 array, ideally
         a PinnedBuffer) at byte offsets `src_off` with lengths `src_len`; image i is written to `dst[dst_off[i]:]`
         (bj_output_size bytes, or bj_scaled_output_size with `rois`: an (n, 4) uint32 array of (x, y, w, h) crops, and
-        `scales`: a scale denominator for every image or one per image).  The pointer tables are built with vector
+        `scales`: a scale denominator for every image or one per image; bj_resized_output_size with `sizes`: one (w, h)
+        for every image or an (n, 2) array - with one size for all, dst can be one [n, h, w, 3] array).  The pointer tables are built with vector
         arithmetic, so the host-side cost per call does not grow with a Python loop over images.  Returns the
         per-image status as an int32 array."""
         n = len(src_off)
@@ -310,13 +360,14 @@ class Decoder:
         op = (np.asarray(dst_off, dtype=np.uint64) + np.uint64(dst.__array_interface__["data"][0]))
         ra, rp = _roi_table(rois, n)
         sa, sp = _scale_table(scales, n)
+        za, zp = _size_table(sizes, n)
         status = np.zeros(max(n, 1), dtype=np.int32)
-        L.check(L.lib().bj_decode_batch_scaled(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, sp, n, fmt,
-                                               op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p)), "bj_decode_batch_scaled", self.ctx)
+        L.check(L.lib().bj_decode_batch_resized(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, sp, zp, n, fmt,
+                                                op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p)), "bj_decode_batch_resized", self.ctx)
         return status[:n]
 
 
-    def submit_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None, scales=None):
+    def submit_packed(self, src, src_off, src_len, dst, dst_off, fmt=L.BJ_OUT_RGB8, rois=None, scales=None, sizes=None):
         """decode_packed without waiting (bj_submit): returns a Job; job.wait() gives the status array."""
         n = len(src_off)
         ip = (np.asarray(src_off, dtype=np.uint64) + np.uint64(src.__array_interface__["data"][0]))
@@ -324,11 +375,12 @@ class Decoder:
         op = (np.asarray(dst_off, dtype=np.uint64) + np.uint64(dst.__array_interface__["data"][0]))
         ra, rp = _roi_table(rois, n)
         sa, sp = _scale_table(scales, n)
+        za, zp = _size_table(sizes, n)
         status = np.zeros(max(n, 1), dtype=np.int32)
         h = C.c_void_p()
-        L.check(L.lib().bj_submit_scaled(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, sp, n, fmt,
-                                         op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p), C.byref(h)), "bj_submit_scaled", self.ctx)
-        return Job(self, h, (ip, il, op, ra, sa, src, dst), status, n)
+        L.check(L.lib().bj_submit_resized(self.ctx, ip.ctypes.data_as(C.c_void_p), il.ctypes.data_as(C.c_void_p), rp, sp, zp, n, fmt,
+                                          op.ctypes.data_as(C.c_void_p), status.ctypes.data_as(C.c_void_p), C.byref(h)), "bj_submit_resized", self.ctx)
+        return Job(self, h, (ip, il, op, ra, sa, za, src, dst), status, n)
 
 
 def lpt_shards(costs, world_size):
