@@ -26,7 +26,8 @@ typedef enum {
     BJ_ERR_CUDA = -2,         /* CUDA runtime/driver error (no device, launch failure ...) - see bj_last_error */
     BJ_ERR_NOMEM = -3,
     BJ_ERR_INVALID_JPEG = -4, /* the reference's read_JPEG would set header->valid = false */
-    BJ_ERR_UNSUPPORTED = -5,  /* valid for the reference's parser but not decodable by its baseline path (SOF2) */
+    BJ_ERR_UNSUPPORTED = -5,  /* valid for the reference's parser but not decodable by its baseline path (SOF2 unless the
+                                 option "progressive" is set; see there for what is refused even then) */
     BJ_ERR_CORRUPT_SCAN = -6  /* entropy-coded data inconsistent (the reference's decode_Huffman_data returns false) */
 } bj_status;
 
@@ -332,16 +333,38 @@ int bj_stage_entropy(bj_ctx *ctx, const uint8_t *file, size_t len, int16_t *coef
  *                      for the one-call path: offsets restart at 0 in every sub-batch) belong to ONE allocation,
  *                      so runs of images are copied out in one transfer, padding bytes included */
 int bj_set_option(bj_ctx *ctx, const char *name, long value);
+/* Option "progressive" (0 default, 1): progressive JPEG (SOF2: 8-bit, Huffman, 1-3 components, the sampling factors
+ * baseline files may have) in bj_decode_batch, _roi, _scaled, _resized, every bj_submit* and every bj_batch_create*,
+ * mixed freely with baseline files.  0: every SOF2 file is BJ_ERR_UNSUPPORTED, as the reference would have it.
+ *   Twin rule: a progressive file's output - RGB8 or BMP, with any ROI, scale and size - is byte for byte the output of
+ *   its baseline twin: the file with the same frame and quantised coefficients in one interleaved baseline scan and no
+ *   restart markers (libjpeg quantises the same way in both modes: Pillow's progressive=True / False at one quality and
+ *   subsampling are twins).  Only pixels inside the image depend on it: the MCU padding that non-interleaved scans do not
+ *   code is not defined.
+ *   Every scan is walked on the host (its restart segments are found there); a file whose walk fails is
+ *   BJ_ERR_INVALID_JPEG: no EOI, a marker that may not follow a scan, a scan header against T.81 G.1.1.1 (an AC scan of
+ *   several components, Ss > Se, Se > 63, Ss = 0 with Se != 0, Ah != 0 with Al != Ah - 1), an AC scan before its
+ *   component's first DC scan, a refinement whose Ah is not the band's last Al (none: no first pass), a second first pass
+ *   of a band, a table that was never defined.  Per image BJ_ERR_UNSUPPORTED: BJ_OUT_REF_MCUS (the reference has no such
+ *   buffers to mirror), more than 64 scans, a DQT behind the first scan that changes a table a component uses.  Damaged
+ *   entropy-coded data (a code not in its table, a run past Se, data past the segment's end, a restart marker count that
+ *   does not match the interval) is BJ_ERR_CORRUPT_SCAN: the damaged restart segment of that scan stops there, everything
+ *   else is decoded, and the output is fully written and deterministic.
+ *   Unchanged whatever the option: bj_parse_header (a multi-scan file is invalid at the end of its first scan, as for
+ *   read_JPEG), bj_peek_header (BJ_ERR_UNSUPPORTED with the frame filled in: enough to size the output),
+ *   bj_decode_batch_desc, bj_stage_entropy and bj_exec_mcus (one scan, or the reference's own buffers). */
 /* Counters of the last call: "exec_ms" (kernel time of bj_exec_mcus - the reference's "DPU execution" profile line,
  * src/decoder_host.cpp:291-294), "decode_batch_sub_batches", "decode_batch_launches", "decode_batch_h2d_bytes",
  * "decode_batch_d2h_bytes", "decode_batch_d2h_copies", "decode_batch_host_ms" (header parse + layout [+ staging copy]),
  * "decode_batch_wait_ms" (caller blocked on the GPU), "host_threads", "devices", and the kernel time per stage summed
  * over the sub-batches - the reference's per-stage "Profiles" lines (src/decoder_host.cpp:379-394) -
  * "decode_batch_ms_unstuff", "decode_batch_ms_sync", "decode_batch_ms_write", "decode_batch_ms_idct",
- * "decode_batch_ms_resize" (the fixed-size output's resize kernel; 0 when no image of a sub-batch is resized);
+ * "decode_batch_ms_resize" (the fixed-size output's resize kernel; 0 when no image of a sub-batch is resized),
+ * "decode_batch_ms_progressive" (the progressive entropy stage: DC clear and one launch per scan level; 0 when no image
+ * of a sub-batch is progressive; "decode_batch_host_ms" includes the progressive files' scan walk);
  * "decode_batch_direct_uploads" (sub-batches whose files went up straight from the caller's page-locked memory).
  * "total_<counter>" (total_sub_batches, total_launches, total_h2d_bytes, total_d2h_bytes, total_host_ms, total_wait_ms,
- * total_d2h_copies, total_ms_unstuff, total_ms_sync, total_ms_write, total_ms_idct, total_ms_resize, total_direct_uploads): the same
+ * total_d2h_copies, total_ms_unstuff, total_ms_sync, total_ms_write, total_ms_idct, total_ms_resize, total_ms_progressive, total_direct_uploads): the same
  * summed over every bj_decode_batch / bj_submit job since the context was created.
  * For a context of several GPUs: byte and launch counts are sums, times the maximum over the devices.
  * Environment: B200JPEG_TRACE=1 prints one line per sub-batch of bj_decode_batch (host prepare, kernels, copy-out). */

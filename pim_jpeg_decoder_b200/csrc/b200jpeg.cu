@@ -184,6 +184,7 @@ extern "C" int bj_set_option(bj_ctx *c, const char *name, long value) {
     if (!strcmp(name, "host_threads")) { if (value < 1 || value > 256) return BJ_ERR_ARG; for (Device *dev : c->devs) dev->host_pool.resize((int)value); return BJ_OK; }
     // the synchronisation pass starts every sub-sequence from its own first bit; the option stays for bench.py --sync-preroll
     if (!strcmp(name, "sync_preroll_bits")) return value == 0 ? BJ_OK : BJ_ERR_ARG;
+    if (!strcmp(name, "progressive")) { if (value != 0 && value != 1) return BJ_ERR_ARG; c->progressive = (int)value; return BJ_OK; }
     if (!strcmp(name, "sync_rounds")) { if (value < 0 || value > kMaxRounds) return BJ_ERR_ARG; c->sync_rounds = (int)value; return BJ_OK; }
     return BJ_ERR_ARG;
 }
@@ -195,7 +196,7 @@ extern "C" int bj_get_stat(const bj_ctx *c, const char *name, double *value) {
     // host_ms: parse + layout + pack, wait_ms: host blocked on the GPU; ms_*: kernel time per stage, summed over the
     // sub-batches (CUDA events) - the reference's per-stage "Profiles" lines (src/decoder_host.cpp:379-394)
     static const char *const names[ST_COUNT] = {"sub_batches", "launches", "h2d_bytes", "d2h_bytes", "host_ms", "wait_ms", "d2h_copies",
-                                                "ms_unstuff", "ms_sync", "ms_write", "ms_idct", "direct_uploads", "ms_resize"};
+                                                "ms_unstuff", "ms_sync", "ms_write", "ms_idct", "direct_uploads", "ms_resize", "ms_progressive"};
     const struct { const char *prefix; const double *counters; } sets[] = {{"decode_batch_", c->stats}, {"total_", c->totals}};
     for (const auto &set : sets) {
         const size_t len = strlen(set.prefix);
@@ -436,6 +437,7 @@ extern "C" int bj_stage_entropy(bj_ctx *c, const uint8_t *file, size_t len, int1
     int rc = bj_batch_create(c, files, lens, 1, BJ_OUT_RGB8, &b);
     if (rc != BJ_OK) return rc;
     if (b->parse_status[0] != BJ_OK) { rc = b->parse_status[0]; bj_batch_destroy(b); return rc; }
+    if (b->prog[0]) { bj_batch_destroy(b); return BJ_ERR_UNSUPPORTED; }   // (one scan only: the baseline stage's output)
     if ((size_t)b->ndu[0] * 128 > capacity_bytes) { bj_batch_destroy(b); return BJ_ERR_ARG; }
     Device *dev = b->dev;
     cudaStream_t s = dev->streams[0];
@@ -530,7 +532,7 @@ static int decode_worker(Device *dev, RangeSource *src, const CallInput &in, int
         st[ST_WAIT_MS] += wall_ms() - t0;
         if (status) for (int i = 0; i < count[slot]; i++) status[first[slot] + i] = r == BJ_OK ? batch_image_status(b, i) : r;
         st[ST_LAUNCH] += b->launches; st[ST_H2D] += (double)(b->files_bytes + b->meta_bytes); st[ST_D2H] += (double)b->d2h_bytes; st[ST_D2H_COPIES] += b->d2h_copies;
-        if (r == BJ_OK) { st[ST_MS_UNSTUFF] += b->ms_unstuff; st[ST_MS_SYNC] += b->ms_sync; st[ST_MS_WRITE] += b->ms_write; st[ST_MS_IDCT] += b->ms_idct; st[ST_MS_RESIZE] += b->ms_resize; }
+        if (r == BJ_OK) { st[ST_MS_UNSTUFF] += b->ms_unstuff; st[ST_MS_SYNC] += b->ms_sync; st[ST_MS_WRITE] += b->ms_write; st[ST_MS_IDCT] += b->ms_idct; st[ST_MS_RESIZE] += b->ms_resize; st[ST_MS_PROG] += b->ms_prog; }
         busy[slot] = false;
         return r;
     };
@@ -596,7 +598,7 @@ static int decode_batch_now(bj_ctx *c, const CallInput &in, int n, int format, u
     for (auto &t : th) t.join();
     // the devices work side by side: counts add up, a time is the longest device's
     for (int i = 0; i < ST_COUNT; i++) {
-        const bool is_time = i == ST_HOST_MS || i == ST_WAIT_MS || (i >= ST_MS_UNSTUFF && i <= ST_MS_IDCT) || i == ST_MS_RESIZE;
+        const bool is_time = i == ST_HOST_MS || i == ST_WAIT_MS || (i >= ST_MS_UNSTUFF && i <= ST_MS_IDCT) || i == ST_MS_RESIZE || i == ST_MS_PROG;
         double v = st[i];
         for (size_t d = 1; d < nd; d++) v = is_time ? std::max(v, st[d * ST_COUNT + i]) : v + st[d * ST_COUNT + i];
         c->stats[i] = v; c->totals[i] += v;

@@ -14,6 +14,7 @@
 #include "bj_host.h"
 #include "kernels_huff.cuh"
 #include "kernels_idct.cuh"
+#include "kernels_prog.cuh"
 #include "kernels_resize.cuh"
 #include "parse.h"
 
@@ -67,6 +68,15 @@ struct bj_batch {
     std::vector<bj::ImgDev> idev;
     std::vector<bj::ResizeDev> rsz;      // fixed-size output: one record per resized image ...
     std::vector<uint32_t> rtile0;        // ... and the prefix of their output tile counts (k_resize_bilinear's map)
+    // progressive images (option "progressive"): the scans parse_progressive found per image, and the device records
+    std::vector<uint8_t> prog;
+    std::vector<std::vector<bj::ProgScan>> pscans;
+    std::vector<bj::ProgImgDev> pimg;
+    std::vector<bj::ProgScanDev> pscan;
+    std::vector<bj::ProgSeg> pseg;
+    std::vector<bj::ProgHuff> ptabs;
+    std::vector<uint32_t> plscan, plitem0;   // the scans ordered by level, and per scan the prefix of its level's segment counts
+    std::vector<uint32_t> plev_first, plev_items;   // per level: first entry in plscan, work items
 
     // host staging (pinned): file bytes; descriptor blob; results
     bj::PinBuf h_files, h_meta, h_res;
@@ -74,6 +84,7 @@ struct bj_batch {
     const uint8_t *direct_src = nullptr;   // set: the files are uploaded straight from the caller's (pinned) memory, files_bytes from here
     // offsets inside the descriptor blob (host -> device)
     size_t o_himg = 0, o_idev = 0, o_qtab = 0, o_lutdc = 0, o_lutac = 0, o_lutacs = 0, o_rsz = 0, o_rtile = 0;
+    size_t o_pimg = 0, o_pscan = 0, o_pseg = 0, o_ptab = 0, o_plscan = 0, o_plitem = 0;
     // offsets inside the map buffer (written on the device by k_expand_maps)
     size_t m_tiles = 0, m_blk = 0, m_wblk = 0, m_utile = 0, m_dcc = 0, maps_bytes = 0;
     uint32_t idct_smem = 0;             // dynamic shared memory of k_idct_color: sized for the widest pixel tile of this batch
@@ -91,14 +102,14 @@ struct bj_batch {
 
     // device
     bj::DevBuf d_files, d_meta, d_maps, d_look, d_clean, d_seg, d_subseg, d_stin, d_stout, d_tot, d_pre, d_slice, d_quarter, d_blkagg, d_state, d_flags, d_coef, d_dc, d_dcagg, d_out;
-    cudaEvent_t ev[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // start, un-stuffed, synchronised, written, pixels, copied out, resized
+    cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // start, un-stuffed, synchronised, written, pixels, copied out, resized, progressive scans decoded
     cudaEvent_t ev_done = nullptr;       // one-call path: recorded behind the copy-out, created for a sleeping wait
     cudaStream_t last_stream = nullptr;
     bool uploaded = false, decoded = false, synced = false;
     bool multi_blk = false;              // some image's sub-sequences span more than one CTA of the synchronisation pass
     bool redone = false;                 // batch_sync had to run extra fix-up rounds: everything after them was computed again
     uint32_t launches = 0, sync_rounds = 0;
-    float ms_entropy = 0.f, ms_idct = 0.f, ms_unstuff = 0.f, ms_sync = 0.f, ms_write = 0.f, ms_resize = 0.f;
+    float ms_entropy = 0.f, ms_idct = 0.f, ms_unstuff = 0.f, ms_sync = 0.f, ms_write = 0.f, ms_resize = 0.f, ms_prog = 0.f;
     uint64_t d2h_bytes = 0;
     uint32_t d2h_copies = 0;
 
@@ -119,6 +130,81 @@ struct bj_batch {
 namespace bj {
 
 constexpr int kMaxRounds = 64;
+
+// The device records of the batch's progressive images (b->prog, b->pscans): images, scans, segments, the pooled and
+// de-duplicated Huffman tables, and the scans ordered by level with the prefix of their segment counts.  O(images + scans).
+inline int prog_layout(bj_batch *b, const std::vector<Geometry> &geo) {
+    b->pimg.clear(); b->pscan.clear(); b->pseg.clear(); b->ptabs.clear(); b->plscan.clear(); b->plitem0.clear();
+    b->plev_first.clear(); b->plev_items.clear();
+    std::map<std::string, uint32_t> tab_index;
+    auto table = [&](const std::string &key) -> uint32_t {
+        auto it = tab_index.find(key);
+        if (it != tab_index.end()) return it->second;
+        const uint32_t idx = (uint32_t)b->ptabs.size();
+        b->ptabs.emplace_back();
+        build_prog_huff((const uint8_t *)key.data(), key.size(), &b->ptabs.back());
+        tab_index[key] = idx;
+        return idx;
+    };
+    std::vector<uint32_t> per_level;                // scans per level, then where each level starts
+    uint64_t nseg_all = 0;
+    for (int i = 0; i < b->n; i++) {
+        if (b->parse_status[i] != BJ_OK || !b->prog[i]) continue;
+        const bj_image_desc &d = b->desc[i];
+        const Geometry &g = geo[i];
+        ProgImgDev im{};
+        im.img = (uint32_t)i; im.du_base = b->du_base[i]; im.file_off = b->file_off[i];
+        im.nmx = g.nmx; im.nmcu = g.nmcu; im.bpm = (uint8_t)g.bpm; im.ny = (uint8_t)(d.hs * d.vs); im.hs = d.hs; im.vs = d.vs;
+        for (int j = 0; j < d.ncomp; j++) {         // component j's size: ceil(X * Hj / Hmax) x ceil(Y * Vj / Vmax), in blocks
+            const uint32_t h = j ? 1u : d.hs, v = j ? 1u : d.vs;
+            im.bw[j] = (uint16_t)(((d.width * h + d.hs - 1) / d.hs + 7) / 8);
+            im.bh[j] = (uint16_t)(((d.height * v + d.vs - 1) / d.vs + 7) / 8);
+        }
+        const uint32_t pi = (uint32_t)b->pimg.size();
+        b->pimg.push_back(im);
+        for (const ProgScan &ps : b->pscans[i]) {
+            ProgScanDev sc{};
+            sc.pimg = pi; sc.ri = ps.ri;
+            sc.ncomp = ps.ncomp; sc.ss = ps.ss; sc.se = ps.se; sc.ah = ps.ah; sc.al = ps.al;
+            for (int j = 0; j < ps.ncomp; j++) { sc.comp[j] = ps.comp[j]; if (ps.ss == 0 && ps.ah == 0) sc.dc_tab[j] = table(ps.dc[j]); }
+            if (ps.se) sc.ac_tab = table(ps.ac);
+            const uint32_t nb = prog_scan_blocks(sc, im);
+            sc.nseg = ps.ri ? (nb + ps.ri - 1) / ps.ri : 1u;
+            sc.seg0 = (uint32_t)b->pseg.size();
+            const size_t R = ps.rst.size();
+            sc.bad = (ps.ri && R + 1 != sc.nseg) ? 1 : 0;
+            for (uint32_t k = 0; k < sc.nseg; k++) {   // a segment whose marker is missing is empty
+                const size_t lo = k == 0 ? ps.off : (k - 1 < R ? ps.rst[k - 1] + 2 : ps.end);
+                const size_t hi = k + 1 == sc.nseg ? ps.end : (k < R ? ps.rst[k] : ps.end);
+                b->pseg.push_back(ProgSeg{(uint32_t)lo, (uint32_t)std::max(lo, hi)});
+            }
+            nseg_all += sc.nseg;
+            if (per_level.size() <= ps.level) per_level.resize(ps.level + 1, 0);
+            per_level[ps.level]++;
+            b->pscan.push_back(sc);
+        }
+    }
+    if (nseg_all > 0x7FFFFFFFull) return BJ_ERR_ARG;
+    // counting sort of the scans by level (levels start at 1)
+    const size_t nl = per_level.empty() ? 0 : per_level.size() - 1;
+    b->plev_first.assign(nl + 1, 0);
+    for (size_t L = 1; L < nl; L++) b->plev_first[L] = b->plev_first[L - 1] + per_level[L];
+    if (nl) b->plev_first[nl] = (uint32_t)b->pscan.size();
+    b->plscan.assign(b->pscan.size(), 0); b->plitem0.assign(b->pscan.size(), 0); b->plev_items.assign(nl, 0);
+    std::vector<uint32_t> fill(b->plev_first.begin(), b->plev_first.end());
+    size_t s = 0;
+    for (int i = 0; i < b->n; i++) {
+        if (b->parse_status[i] != BJ_OK || !b->prog[i]) continue;
+        for (const ProgScan &ps : b->pscans[i]) {
+            const uint32_t L = ps.level - 1u, at = fill[L]++;
+            b->plscan[at] = (uint32_t)s;
+            b->plitem0[at] = b->plev_items[L];
+            b->plev_items[L] += b->pscan[s].nseg;
+            s++;
+        }
+    }
+    return BJ_OK;
+}
 
 // (Re)fill a batch object from a list of files: parse the headers, lay out, (stage).  Host work only (plus buffer growth).
 //   out_cap   the batch takes images from the front of the list until their decoded bytes pass this (at least one):
@@ -146,6 +232,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     b->dev = dev; b->n = n; b->format = format;
     b->uploaded = b->decoded = b->synced = false;
     b->desc.resize(n); b->parse_status.assign(n, BJ_OK);
+    b->prog.assign(n, 0); b->pscans.resize(n);
     if (dev->check(cudaSetDevice(dev->ordinal)) != BJ_OK) return BJ_ERR_CUDA;
     for (auto &e : b->ev) if (!e && dev->check(cudaEventCreate(&e)) != BJ_OK) return BJ_ERR_CUDA;
 
@@ -163,8 +250,14 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
                     if (!d.qt_set[d.qt_id[j]] || !d.dc_set[d.dc_id[j]] || !d.ac_set[d.ac_id[j]]) rc = BJ_ERR_INVALID_JPEG;
                 if (rc == BJ_OK && (d.frame_type != 0xC0 || d.scan_ncomp != d.ncomp)) rc = BJ_ERR_UNSUPPORTED;
                 if (rc == BJ_OK && kinds && kinds[i] == BJ_SCAN_UNSTUFFED && d.restart_interval != 0) rc = BJ_ERR_UNSUPPORTED;
-            } else
+            } else {
                 rc = (files[i] && lens[i]) ? parse_header(files[i], lens[i], &d, /*walk_scan=*/false) : BJ_ERR_INVALID_JPEG;
+                if (rc == BJ_ERR_UNSUPPORTED && d.frame_type == 0xC2 && c->progressive) {       // every scan, walked on the host
+                    rc = parse_progressive(files[i], lens[i], &d, &b->pscans[i]);
+                    if (rc == BJ_OK && format == BJ_OUT_REF_MCUS) rc = BJ_ERR_UNSUPPORTED;       // (the reference has no such buffers to mirror)
+                    if (rc == BJ_OK) b->prog[i] = 1;
+                }
+            }
             if (rc == BJ_OK && d.scan_len >= ((size_t)1 << 31)) rc = BJ_ERR_UNSUPPORTED;   // byte counts travel in 31 bits
             if (rc == BJ_OK && (size_t)d.width * d.height > c->max_image_pixels) rc = BJ_ERR_UNSUPPORTED;   // (the full image: its whole scan is decoded)
             bj_roi r{};
@@ -193,7 +286,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
             acc += sz; m++;
         }
         n = m; b->n = n;
-        b->desc.resize(n); b->parse_status.resize(n);
+        b->desc.resize(n); b->parse_status.resize(n); b->prog.resize(n);
     }
     b->out_off.assign(n, 0); b->out_size.assign(n, 0); b->file_off.assign(n, 0);
     b->du_base.assign(n, 0); b->ndu.assign(n, 0);
@@ -280,6 +373,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     size_t fbytes = 0, clean_words = 0, out_bytes = 0, coef_units = 0;
     uint32_t seg_entries = 0, nblk = 0, n_utile = 0, n_wblk = 0, n_dcc = 0, n_tiles = 0;
     int prev = -1;                                  // last valid image: its table slots are reused when the tables match
+    int prev_lut = -1;                              // ... of the baseline images (a progressive image has no baseline tables)
     b->pixels = 0; b->scan_bytes_max = 0; b->ref_blocks_max = 0; b->nseg_max = 0; b->lut_smem = 0; b->multi_blk = false; b->scaled = false;
     b->rsz.clear(); b->rtile0.clear();
     size_t inter_bytes = 0;                         // the resize sources, offsets from the intermediate region's start
@@ -301,9 +395,9 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         memset(&idev[i], 0, sizeof(ImgDev));
         int rc = b->parse_status[i];
         const Geometry &g = geo[i];
-        if (rc == BJ_OK) {
-            if (prev >= 0 && same_tables(d, b->desc[prev])) {
-                const HuffImg &hp = himg[prev];
+        if (rc == BJ_OK && !b->prog[i]) {
+            if (prev_lut >= 0 && same_tables(d, b->desc[prev_lut])) {
+                const HuffImg &hp = himg[prev_lut];
                 hi.ndc = hp.ndc; hi.nac = hp.nac;
                 memcpy(hi.dc_lut, hp.dc_lut, sizeof(hi.dc_lut)); memcpy(hi.ac_lut, hp.ac_lut, sizeof(hi.ac_lut));
                 memcpy(hi.dc_slot, hp.dc_slot, sizeof(hi.dc_slot)); memcpy(hi.ac_slot, hp.ac_slot, sizeof(hi.ac_slot));
@@ -363,6 +457,13 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         if (rc != BJ_OK) { seg_entries += 2; hi.ndc = hi.nac = 0; continue; }
         fbytes += align_up(lens[i] + 16, 16);
         hi.valid = 1;
+        if (b->prog[i]) {                               // no baseline entropy work: first_zero stays 0, so k_zero_tail clears its units
+            seg_entries += 2;
+            hi.nseg = 1;
+            hi.ndu = g.ndu;
+            b->du_base[i] = (uint32_t)coef_units; b->ndu[i] = g.ndu;
+            coef_units += g.ndu;
+        } else {
         hi.flags = descs ? (uint8_t)((kinds && kinds[i] == BJ_SCAN_UNSTUFFED) ? (kImgClean | kImgExact) : kImgExact) : (uint8_t)0;
         hi.raw_off = b->file_off[i] + d.scan_off;
         hi.raw_len = (uint32_t)d.scan_len;                                   // upper bound: up to the end of the file
@@ -393,6 +494,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         clean_words += hi.raw_len / 4 + 4;
         b->du_base[i] = (uint32_t)coef_units; b->ndu[i] = g.ndu;
         coef_units += g.ndu;
+        }
         const bj_roi *roi = rois ? &rois[i] : nullptr;
         const uint32_t scale = scales ? scales[i] : 1u;
         const bj_size *size = size_of(i);
@@ -415,6 +517,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
         if (prev >= 0 && same_qtab(d, b->desc[prev])) idev[i].qslot = idev[prev].qslot;
         else { idev[i].qslot = (uint32_t)qtabs.size(); qtabs.emplace_back(); fill_qtab(d, &qtabs.back()); }
         prev = i;
+        if (!b->prog[i]) prev_lut = i;
         out_bytes += align_up(b->out_size[i], 16);
         rgb_max = std::max<uint32_t>(rgb_max, std::min<uint32_t>(g.tile_mcus, g.nmx) * d.hs * 8u * d.vs * 8u * 3u);
         b->pixels += (uint64_t)d.width * d.height;
@@ -426,6 +529,7 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     for (int i = 0; i < n; i++) if (b->parse_status[i] == BJ_OK && size_of(i)) idev[i].out_row0 += b->inter_off;
     for (ResizeDev &rz : b->rsz) rz.src_off += b->inter_off;
     b->n_rsz = (uint32_t)b->rsz.size(); b->n_rtiles = (uint32_t)n_rtiles;
+    if (prog_layout(b, geo) != BJ_OK) return BJ_ERR_ARG;
     b->idct_smem = kSmemDu + kSmemQ + kRgbFront + std::min<uint32_t>(rgb_max, kRgbMax) + 64;
     b->files_bytes = b->direct_src ? (size_t)(span_hi - span_lo) : fbytes + 64; b->clean_words = clean_words + 96; b->coef_units = coef_units; b->out_bytes = out_bytes;   // (96 words of slack: a damaged unit is read to its end, up to 63 symbols of 27 bits past the data)
     b->n_wblk = n_wblk; b->n_slice_slots = slice_slots;
@@ -442,6 +546,12 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     b->o_lutacs = o; o = align_up(o + luts_acs.size() * 4, 256);
     b->o_rsz = o;   o = align_up(o + b->rsz.size() * sizeof(ResizeDev), 256);
     b->o_rtile = o; o = align_up(o + b->rtile0.size() * 4, 256);
+    b->o_pimg = o;  o = align_up(o + b->pimg.size() * sizeof(ProgImgDev), 256);
+    b->o_pscan = o; o = align_up(o + b->pscan.size() * sizeof(ProgScanDev), 256);
+    b->o_pseg = o;  o = align_up(o + b->pseg.size() * sizeof(ProgSeg), 256);
+    b->o_ptab = o;  o = align_up(o + b->ptabs.size() * sizeof(ProgHuff), 256);
+    b->o_plscan = o; o = align_up(o + b->plscan.size() * 4, 256);
+    b->o_plitem = o; o = align_up(o + b->plitem0.size() * 4, 256);
     b->meta_bytes = o;
     // ---- map buffer (device only: k_expand_maps)
     o = 0;
@@ -459,6 +569,14 @@ inline int batch_assign(bj_batch *b, Device *dev, const uint8_t *const *files, c
     if (!luts_ac.empty()) memcpy(b->hmeta<uint32_t>(b->o_lutac), luts_ac.data(), luts_ac.size() * 4);
     if (!luts_acs.empty()) memcpy(b->hmeta<uint32_t>(b->o_lutacs), luts_acs.data(), luts_acs.size() * 4);
     if (!b->rsz.empty()) { memcpy(b->hmeta<ResizeDev>(b->o_rsz), b->rsz.data(), b->rsz.size() * sizeof(ResizeDev)); memcpy(b->hmeta<uint32_t>(b->o_rtile), b->rtile0.data(), b->rtile0.size() * 4); }
+    if (!b->pimg.empty()) {
+        memcpy(b->hmeta<ProgImgDev>(b->o_pimg), b->pimg.data(), b->pimg.size() * sizeof(ProgImgDev));
+        memcpy(b->hmeta<ProgScanDev>(b->o_pscan), b->pscan.data(), b->pscan.size() * sizeof(ProgScanDev));
+        memcpy(b->hmeta<ProgSeg>(b->o_pseg), b->pseg.data(), b->pseg.size() * sizeof(ProgSeg));
+        memcpy(b->hmeta<ProgHuff>(b->o_ptab), b->ptabs.data(), b->ptabs.size() * sizeof(ProgHuff));
+        memcpy(b->hmeta<uint32_t>(b->o_plscan), b->plscan.data(), b->plscan.size() * 4);
+        memcpy(b->hmeta<uint32_t>(b->o_plitem), b->plitem0.data(), b->plitem0.size() * 4);
+    }
     // ---- stage the file bytes (only when they cannot go up from where they are; per image, independent: worker pool)
     if (!b->direct_src) {
         uint8_t *hf = reinterpret_cast<uint8_t *>(b->h_files.p);
@@ -576,6 +694,19 @@ inline int batch_launch(bj_batch *b, cudaStream_t s, int r0, int r1) {
     }
     if (!b->n_blk) cudaEventRecord(b->ev[2], s);
     cudaEventRecord(b->ev[3], s);
+    if (!b->pimg.empty()) {                                                           // progressive images: only when the batch has one
+        ProgImgDev *pimgs = b->dmeta<ProgImgDev>(b->o_pimg);
+        k_prog_zero_dc<<<(unsigned)b->pimg.size(), 256, 0, s>>>(pimgs, dcp);
+        b->launches++;
+        for (size_t L = 0; L < b->plev_items.size(); L++) {
+            const uint32_t first = b->plev_first[L], nscans = b->plev_first[L + 1] - first, items = b->plev_items[L];
+            k_prog_decode<<<(items + kProgThreads - 1) / kProgThreads, kProgThreads, 0, s>>>(pimgs, b->dmeta<ProgScanDev>(b->o_pscan), b->dmeta<ProgSeg>(b->o_pseg),
+                b->dmeta<ProgHuff>(b->o_ptab), b->dmeta<uint32_t>(b->o_plscan) + first, b->dmeta<uint32_t>(b->o_plitem) + first, nscans, items,
+                (const uint8_t *)b->d_files.p, st, (int16_t *)b->d_coef.p, dcp);
+            b->launches++;
+        }
+        cudaEventRecord(b->ev[7], s);
+    }
     if (b->n_idct_tiles && b->format == BJ_OUT_REF_MCUS) {
         const unsigned gx = std::min<unsigned>(64u, (b->ref_blocks_max * 12u + 255u) / 256u);
         k_ref_mcus_pad<<<dim3(std::max(gx, 1u), n), 256, 0, s>>>(idev, (uint8_t *)b->d_out.p);
@@ -636,7 +767,9 @@ inline int batch_sync(bj_batch *b) {
         cudaEventElapsedTime(&b->ms_unstuff, b->ev[0], b->ev[1]);
         cudaEventElapsedTime(&b->ms_sync, b->ev[1], b->ev[2]);        // (only the last group of rounds if extra ones ran)
         cudaEventElapsedTime(&b->ms_write, b->ev[2], b->ev[3]);
-        cudaEventElapsedTime(&b->ms_idct, b->ev[3], b->ev[4]);
+        cudaEventElapsedTime(&b->ms_idct, b->ev[b->pimg.empty() ? 3 : 7], b->ev[4]);
+        b->ms_prog = 0.f;
+        if (!b->pimg.empty()) cudaEventElapsedTime(&b->ms_prog, b->ev[3], b->ev[7]);
         b->ms_resize = 0.f;
         if (b->n_rtiles) cudaEventElapsedTime(&b->ms_resize, b->ev[4], b->ev[6]);
         b->synced = true;

@@ -128,7 +128,7 @@ constexpr size_t kDefaultMaxImagePixels = (size_t)1 << 28;   // option "max_imag
 enum { POOL_COMPAT_MD = 0, POOL_COMPAT_MCUS, POOL_COEF, POOL_OUT, POOL_IMGS, POOL_TILES, POOL_COUNT };
 
 // counters of one bj_decode_batch / job (bj_get_stat: "decode_batch_<name>", "total_<name>")
-enum { ST_SUB = 0, ST_LAUNCH, ST_H2D, ST_D2H, ST_HOST_MS, ST_WAIT_MS, ST_D2H_COPIES, ST_MS_UNSTUFF, ST_MS_SYNC, ST_MS_WRITE, ST_MS_IDCT, ST_DIRECT, ST_MS_RESIZE, ST_COUNT };
+enum { ST_SUB = 0, ST_LAUNCH, ST_H2D, ST_D2H, ST_HOST_MS, ST_WAIT_MS, ST_D2H_COPIES, ST_MS_UNSTUFF, ST_MS_SYNC, ST_MS_WRITE, ST_MS_IDCT, ST_DIRECT, ST_MS_RESIZE, ST_MS_PROG, ST_COUNT };
 
 }  // namespace bj
 
@@ -164,6 +164,7 @@ struct bj_ctx {
     size_t max_image_pixels = bj::kDefaultMaxImagePixels;   // larger images are refused (BJ_ERR_UNSUPPORTED), like the reference's "Too high resolution"
     size_t sub_batch_out_bytes = (size_t)1 << 30; // decoded bytes per sub-batch of bj_decode_batch
     int sync_rounds = 0;                 // 0 = default (3 launches of the fix-up kernel before the first check)
+    int progressive = 0;                 // 1: the data-loader entries decode progressive (SOF2) files too (kernels_prog.cuh)
     std::vector<bj::Device *> devs;      // never empty; staged and stage-level entries run on devs[0]
     bj::AsyncWorker *async = nullptr;    // bj_submit / bj_wait
     double stats[bj::ST_COUNT] = {};     // counters of the last bj_decode_batch / job, folded over the devices

@@ -7,6 +7,9 @@
 #pragma once
 #include <stdint.h>
 #include <string.h>
+#include <algorithm>
+#include <string>
+#include <vector>
 #include "../../include/b200jpeg.h"
 
 namespace bj {
@@ -131,30 +134,42 @@ inline void parse_scan_header(Cursor &c, bj_image_desc &d, ParseState &st) {
     if (length - 6 - 2 * ns != 0) st.valid = false;
 }
 
+inline void parse_dri(Cursor &c, bj_image_desc &d, ParseState &st) {
+    const unsigned l = c.get16();
+    d.restart_interval = c.get16();
+    if (l != 4) st.valid = false;
+}
+
 inline void skip_segment(Cursor &c) {
     const unsigned length = c.get16();
     if (length >= 2) { const size_t adv = length - 2; if (c.i + adv > c.n) { c.i = c.n; c.eof = true; } else c.i += adv; }
 }
 
 // Locate the end of the entropy-coded segment (src/jpeg_scanner.cpp:405-433): the first FF that is followed by
-// something other than 00 / RSTn / FF.  EOI ends the scan; anything else makes the file invalid.
-// Only bj_parse_header (the public, stand-alone restatement of read_JPEG) walks the scan like this; the decode path
-// leaves it to the GPU (kernels_huff.cuh: k_unstuff applies the same rule).
-inline int find_scan_end(const uint8_t *p, size_t n, size_t start, size_t *end) {
+// something other than 00 / RSTn / FF.  scan_extent: false if the file ends first; *end = that FF's position, and
+// `rst` (if given) receives the positions of the RSTn markers on the way.
+inline bool scan_extent(const uint8_t *p, size_t n, size_t start, size_t *end, std::vector<size_t> *rst = nullptr) {
     size_t i = start;
     for (;;) {
-        if (i >= n) return BJ_ERR_INVALID_JPEG;                           // "File ended prematurely"
+        if (i >= n) return false;
         const uint8_t *f = (const uint8_t *)memchr(p + i, 0xFF, n - i);
-        if (!f) return BJ_ERR_INVALID_JPEG;
+        if (!f) return false;
         i = (size_t)(f - p);
-        if (i + 1 >= n) return BJ_ERR_INVALID_JPEG;
+        if (i + 1 >= n) return false;
         const unsigned m = p[i + 1];
-        if (m == 0xD9) { *end = i; return BJ_OK; }
         if (m == 0x00) { i += 2; continue; }
-        if (m >= 0xD0 && m <= 0xD7) { i += 2; continue; }
+        if (m >= 0xD0 && m <= 0xD7) { if (rst) rst->push_back(i); i += 2; continue; }
         if (m == 0xFF) { i += 1; continue; }
-        return BJ_ERR_INVALID_JPEG;                                       // "Invalid marker during compressed data scan"
+        *end = i;
+        return true;
     }
+}
+// EOI ends the scan; anything else makes the file invalid ("File ended prematurely", "Invalid marker during
+// compressed data scan").  Only bj_parse_header (the public, stand-alone restatement of read_JPEG) walks the scan like
+// this; the baseline decode path leaves it to the GPU (kernels_huff.cuh: k_unstuff applies the same rule).
+inline int find_scan_end(const uint8_t *p, size_t n, size_t start, size_t *end) {
+    if (!scan_extent(p, n, start, end)) return BJ_ERR_INVALID_JPEG;
+    return p[*end + 1] == 0xD9 ? BJ_OK : BJ_ERR_INVALID_JPEG;
 }
 
 // walk_scan = false (the decode path): only the headers are read (a few hundred bytes); scan_len is then an UPPER
@@ -176,7 +191,7 @@ inline int parse_header(const uint8_t *file, size_t len, bj_image_desc *out, boo
         else if (cur == 0xDB) parse_dqt(c, d, st);
         else if (cur == 0xC4) parse_dht(c, d, st);
         else if (cur == 0xDA) { parse_scan_header(c, d, st); sos = true; break; }
-        else if (cur == 0xDD) { const unsigned l = c.get16(); d.restart_interval = c.get16(); if (l != 4) st.valid = false; }
+        else if (cur == 0xDD) parse_dri(c, d, st);
         else if ((cur >= 0xE0 && cur <= 0xEF) || cur == 0xFE || (cur >= 0xF0 && cur <= 0xFD) || cur == 0xDC || cur == 0xDE || cur == 0xDF) skip_segment(c);
         else if (cur == 0x01) {}
         else if (cur == 0xFF) { cur = c.get(); continue; }
@@ -196,6 +211,111 @@ inline int parse_header(const uint8_t *file, size_t len, bj_image_desc *out, boo
     }
     if (d.frame_type != 0xC0) return BJ_ERR_UNSUPPORTED;                  // SOF2: parsed, never decodable (SURVEY 2)
     if (d.scan_ncomp != d.ncomp) return BJ_ERR_UNSUPPORTED;               // non-interleaved scans: reference output is garbage
+    return BJ_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ progressive files
+// The multi-scan walk of an SOF2 file (context option "progressive"): marker by marker to EOI, through every scan.  The
+// header segments go through the same readers as above; this is the one place where the host reads entropy-coded
+// bytes - scan_extent's memchr for FF - to find where each scan and each of its restart segments lies.
+constexpr int kProgMaxScans = 64;
+
+struct ProgScan {
+    uint8_t ncomp;               // components in the scan (1 for an AC scan)
+    uint8_t comp[3];             // their indices (frame id - 1), in scan order
+    uint8_t ss, se, ah, al;
+    uint8_t level;               // 1 + the highest level of an earlier scan that touches a coefficient of this one
+    uint32_t ri;                 // restart interval: MCUs of an interleaved scan, blocks of a single-component one; 0 none
+    std::string dc[3], ac;       // the Huffman tables the scan uses (17 offsets + symbols, as parse_dht keeps them)
+    size_t off, end;             // entropy-coded bytes [off, end): end = the FF of the marker that ends the scan
+    std::vector<size_t> rst;     // positions of the RSTn markers inside
+};
+
+inline std::string huff_key(const uint8_t off[17], const uint8_t *sym) {
+    std::string k((const char *)off, 17);
+    k.append((const char *)sym, off[16] > 162 ? 162 : off[16]);
+    return k;
+}
+
+// Returns BJ_OK with *out filled as bj_peek_header fills it (first scan's header fields) and `scans` the scan list, or
+// BJ_ERR_INVALID_JPEG for a structural error (no EOI, a marker that may not follow a scan, the T.81 G.1.1.1 rules, an AC
+// scan before its component's first DC scan, a refinement of a band with no first pass (or whose Ah is not the band's
+// last Al), a first pass of a band that already had one, a table never defined), or BJ_ERR_UNSUPPORTED for more than
+// kProgMaxScans scans or a DQT behind the first scan that changes a table a frame component uses.
+inline int parse_progressive(const uint8_t *file, size_t len, bj_image_desc *out, std::vector<ProgScan> *scans) {
+    bj_image_desc &d = *out;
+    memset(&d, 0, sizeof(d));
+    d.hs = d.vs = 1;
+    for (int i = 0; i < 3; i++) d.comp_h[i] = d.comp_v[i] = 1;
+    scans->clear();
+    Cursor c{file, len, 0, false};
+    ParseState st;
+    unsigned last = c.get(), cur = c.get();
+    if (last != 0xFF || cur != 0xD8) return BJ_ERR_INVALID_JPEG;
+    last = c.get();  cur = c.get();
+    int8_t bits[3][64];          // per component and coefficient: Al of the last scan that coded it, -1 none yet
+    uint8_t level[3][64];        // ... and that scan's level
+    memset(bits, -1, sizeof(bits));
+    memset(level, 0, sizeof(level));
+    for (;;) {
+        if (!st.valid || c.eof || last != 0xFF) return BJ_ERR_INVALID_JPEG;
+        const bool after_scan = !scans->empty();
+        if (cur == 0xD9) break;
+        if (cur == 0xC2 && !after_scan) { d.frame_type = 0xC2; parse_frame(c, d, st); }
+        else if (cur == 0xDB) {
+            uint16_t qt[4][64];
+            uint8_t set[4];
+            memcpy(qt, d.qt_zz, sizeof(qt)); memcpy(set, d.qt_set, sizeof(set));
+            parse_dqt(c, d, st);
+            for (int j = 0; st.valid && after_scan && j < d.ncomp; j++) {
+                const int t = d.qt_id[j] & 3;
+                if (set[t] && memcmp(qt[t], d.qt_zz[t], sizeof(qt[t]))) return BJ_ERR_UNSUPPORTED;
+            }
+        }
+        else if (cur == 0xC4) parse_dht(c, d, st);
+        else if (cur == 0xDD) parse_dri(c, d, st);
+        else if (cur == 0xDA) {
+            if (d.frame_type != 0xC2) return BJ_ERR_INVALID_JPEG;
+            const size_t h0 = c.i;
+            parse_scan_header(c, d, st);
+            if (!st.valid || c.eof) return BJ_ERR_INVALID_JPEG;
+            if ((int)scans->size() == kProgMaxScans) return BJ_ERR_UNSUPPORTED;
+            ProgScan s;
+            // the header parse_scan_header accepted: length, Ns, Ns x (id, tables), Ss, Se, Ah/Al
+            const uint8_t *h = file + h0;
+            s.ncomp = h[2];
+            for (unsigned i = 0; i < s.ncomp; i++) s.comp[i] = (uint8_t)(((h[3 + 2 * i] + (st.zero_based ? 1u : 0u)) & 0xFF) - 1u);
+            s.ss = h[3 + 2 * s.ncomp]; s.se = h[4 + 2 * s.ncomp]; s.ah = h[5 + 2 * s.ncomp] >> 4; s.al = h[5 + 2 * s.ncomp] & 15;
+            if (s.al > 13) return BJ_ERR_INVALID_JPEG;                    // (8-bit data: coefficients have at most 11 + 3 bits)
+            s.ri = d.restart_interval;
+            int lv = 0;
+            for (unsigned i = 0; i < s.ncomp; i++) {
+                const int j = s.comp[i];
+                if (s.ss > 0 && bits[j][0] < 0) return BJ_ERR_INVALID_JPEG;          // AC before the component's first DC scan
+                for (int k = s.ss; k <= s.se; k++) {
+                    if (s.ah == 0 ? bits[j][k] >= 0 : bits[j][k] != (int)s.ah) return BJ_ERR_INVALID_JPEG;
+                    lv = std::max<int>(lv, level[j][k]);
+                }
+                s.dc[i] = huff_key(d.dc_offsets[d.dc_id[j]], d.dc_symbols[d.dc_id[j]]);
+                if (s.se > 0) s.ac = huff_key(d.ac_offsets[d.ac_id[j]], d.ac_symbols[d.ac_id[j]]);
+            }
+            s.level = (uint8_t)(lv + 1);
+            for (unsigned i = 0; i < s.ncomp; i++)
+                for (int k = s.ss; k <= s.se; k++) { bits[s.comp[i]][k] = (int8_t)s.al; level[s.comp[i]][k] = s.level; }
+            if (scans->empty()) { d.scan_off = c.i; d.scan_len = len - c.i; }
+            s.off = c.i;
+            if (!scan_extent(file, len, c.i, &s.end, &s.rst)) return BJ_ERR_INVALID_JPEG;   // no EOI
+            c.i = s.end;
+            const unsigned m = file[s.end + 1];                            // what may follow a scan
+            if (!(m == 0xD9 || m == 0xDA || m == 0xC4 || m == 0xDB || m == 0xDD || m == 0xFE || (m >= 0xE0 && m <= 0xEF))) return BJ_ERR_INVALID_JPEG;
+            scans->push_back(std::move(s));
+        }
+        else if ((cur >= 0xE0 && cur <= 0xEF) || cur == 0xFE) skip_segment(c);
+        else if (cur == 0xFF) { cur = c.get(); continue; }
+        else return BJ_ERR_INVALID_JPEG;                                   // another frame, SOI, DNL, ... inside the file
+        last = c.get();  cur = c.get();
+    }
+    if (scans->empty() || d.ncomp == 0) return BJ_ERR_INVALID_JPEG;
     return BJ_OK;
 }
 

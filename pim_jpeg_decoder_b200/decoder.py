@@ -26,6 +26,19 @@ def parse_header(data):
     return st, d
 
 
+def _sizing_header(data):
+    """The descriptor that sizes a file's output: bj_parse_header's, or for a progressive (SOF2) file - which
+    bj_parse_header calls invalid at the end of its first scan, and which the decode entries take with the context option
+    "progressive" - bj_peek_header's (the size functions read only the frame)."""
+    st, d = parse_header(data)
+    if st != L.BJ_OK:
+        p = L.ImageDesc()
+        buf = np.frombuffer(data, dtype=np.uint8)
+        if L.lib().bj_peek_header(buf.ctypes.data_as(C.c_void_p), len(data), C.byref(p)) == L.BJ_ERR_UNSUPPORTED and p.frame_type == 0xC2:
+            return L.BJ_OK, p
+    return st, d
+
+
 def _roi_table(rois, n):
     """rois: None (whole images) or n rows of (x, y, w, h) - an (n, 4) array or anything numpy makes one of; a row of
     zeros is the whole image.  -> (keepalive uint32 array or None, pointer for the C ABI)"""
@@ -315,7 +328,7 @@ class Decoder:
         if outs is None:
             outs = []
             for i, f in enumerate(files):
-                st, d = parse_header(f)
+                st, d = _sizing_header(f)
                 size = 0
                 if st == L.BJ_OK and ra is None and sa is None and za is None:
                     size = L.lib().bj_output_size(C.byref(d), fmt)          # (BJ_OUT_REF_MCUS included: it has no crop, scale or size)
